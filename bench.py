@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — gradient updates/sec of the SAC/TD3 learner iteration (batch 256, MuJoCo shapes).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b2rl|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b2rl|reference] [--workload NAME] [--dump-outputs DIR]
 
 A "step" is ONE learner iteration in the reference's cadence (orchestrator.py:337-352): replay sample
 -> update_qnets -> (every 3rd iteration) 2 x update_actor on the same batch -> update_targ_nets.
@@ -145,6 +145,40 @@ def time_kernel(fn, iters=200, warm=20, per_graph=20):
     return e0.elapsed_time(e1) / (reps * per_graph) * 1e-3
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def timed_outputs(eng) -> dict:
+    """What a caller of LearnerEngine.iteration holds after its last call: the logged losses, the batch that step
+    sampled, and the online and target parameters, as host arrays (float32; the batch indices as float64, which holds
+    them exactly). Inputs are seeded, so two builds given the same arguments can be compared array for array."""
+    ag = eng.agent
+    out = {k.replace("/", "."): v for k, v in eng.logs().items()}
+    batch = eng.last_batch()
+    for k in ("observations", "actions", "rewards", "next_observations", "dones"):
+        out[f"batch.{k}"] = batch[k].float()
+    out["batch.index"] = batch["index"].double()
+    groups = {"actor": ag.actor_params, "qnet": ag.qnet_params, "qnet_target": ag.qnet_target}
+    if ag.td3:
+        groups["actor_target"] = ag.actor_target
+    else:
+        out["log_alpha"] = ag.log_alpha
+    for g, params in groups.items():
+        out.update({f"{g}.{n}": p for n, p in params.items()})
+    return {k: v.detach().cpu().numpy() for k, v in out.items()}
+
+
+def write_outputs(directory, arrays: dict) -> None:
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES} byte limit")
+    d = Path(directory)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(d / f"{name}.npy", a)
+
+
 def run_b2rl(args, rank, world, device):
     import ctypes as C
     from sac_td3_cudagraphs_pytorch_b200 import _lib as L
@@ -173,6 +207,7 @@ def run_b2rl(args, rank, world, device):
             launches += eng.launches(i)
         e1.record()
         barrier()
+        outputs = timed_outputs(eng) if args.dump_outputs and rank == 0 else None  # before the untimed steps below
         # nvidia-smi samples every 100 ms and the K timed steps may last less than that: keep the SAME load running
         # (untimed) until the sampler has seen it a few times, so that `clocks` describes this load and not idle
         t_load, extra = time.perf_counter(), W + K
@@ -189,6 +224,8 @@ def run_b2rl(args, rank, world, device):
         elapsed = float(t)
     value = world * K / elapsed
     finite = bool(torch.isfinite(ag.out).all())
+    if outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
 
     # ---- end to end through the public API (LearnerEngine.step_async / wait): per step 4 new transitions written by the
     #      host into pinned memory -> read from there by the replay-write kernel (the H2D copy) -> sample -> update(s)
@@ -198,7 +235,6 @@ def run_b2rl(args, rank, world, device):
     #      step, one step late; "sync": it reads step t's losses before preparing step t + 1.
     n_env = 4
     src_rows = torch.randn(n_env, fmt.row_stride)           # "what the envs just produced" (pageable host memory)
-    Ke = max(300, min(K, 3000))  # (>= 300 steps: ~20 ms of wall clock even at the driver's --steps 20)
     step_no = [W + K]
 
     def e2e_loop(n, pipelined):
@@ -220,14 +256,14 @@ def run_b2rl(args, rank, world, device):
     def timed(pipelined):
         barrier()
         t0 = time.perf_counter()
-        e2e_loop(Ke, pipelined)
+        e2e_loop(K, pipelined)
         barrier()
         el = time.perf_counter() - t0
         if world > 1:
             t = torch.tensor([el], device=device, dtype=torch.float64)
             torch.distributed.all_reduce(t, op=torch.distributed.ReduceOp.MAX)
             el = float(t)
-        return world * Ke / el
+        return world * K / el
 
     e2e_loop(12, True)                                       # captures the step-graph variants (both slots)
     e2e_sync = timed(False)
@@ -253,11 +289,11 @@ def run_b2rl(args, rank, world, device):
     policy_loop(12)
     barrier()
     t0 = time.perf_counter()
-    policy_loop(Ke)
+    policy_loop(K)
     barrier()
-    e2e_policy = world * Ke / (time.perf_counter() - t0)
+    e2e_policy = world * K / (time.perf_counter() - t0)
     e2e = {"value": e2e_pipe, "unit": "updates/s", "h2d_bytes_per_step": n_env * fmt.row_stride * 4,
-           "d2h_bytes_per_step": 32, "steps": Ke, "mode": "one step in flight while the host prepares the next; "
+           "d2h_bytes_per_step": 32, "steps": K, "mode": "one step in flight while the host prepares the next; "
            "every step's losses are read, one step late", "sync_value": e2e_sync,
            "with_policy_value": e2e_policy, "with_policy": "the same plus Agent.predict on 4 observations inside the step graph "
            "(pinned obs in, pinned actions out, actions read before the next step is launched)"}
@@ -631,7 +667,11 @@ def main():
     ap.add_argument("--also", default="sac_hopper,sac_humanoid", help="extra workloads measured after the main one (N=1)")
     ap.add_argument("--no-legs", action="store_true", help="skip the config-4 (population) and config-5 (data-parallel) legs")
     ap.add_argument("--no-torch-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the main workload's last timed step computed "
+                    "(losses, sampled batch, online and target parameters) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b2rl":
+        ap.error("--dump-outputs needs --impl b2rl")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -651,7 +691,7 @@ def main():
     if rank == 0 and world == 1 and args.also:
         for w in [x for x in args.also.split(",") if x and x != args.workload]:
             a2 = argparse.Namespace(**vars(args))
-            a2.workload, a2.steps = w, min(args.steps, 1500)
+            a2.workload, a2.dump_outputs = w, None
             r2 = run_b2rl(a2, 0, 1, device)
             extra[w] = {"updates_per_s": r2["value"], "ms_per_step": r2["elapsed"] / a2.steps * 1e3,
                         "e2e_updates_per_s": r2["e2e"]["value"], "critic_fused_frac_of_ffma_peak": r2["roofline"]["frac"],

@@ -37,3 +37,31 @@ def test_torch_cudagraph_baseline_runs():
         del bench.WORKLOADS["_toy"]
     assert r["value"] > 0 and r["replay_rows"] == 4096 and not r["tf32"]
     assert r["kernels_per_graph"]["q"] is None or r["kernels_per_graph"]["q"] > 50  # ~130-230 torch kernels per update graph
+
+
+@pytest.mark.parametrize("algo", ["td3", "sac"])
+def test_dumped_outputs_repeat_for_the_same_steps(algo, tmp_path):
+    """--dump-outputs: the same seeded run gives the same arrays bit for bit; one step more gives other ones."""
+    import numpy as np
+
+    import bench
+    bench.WORKLOADS["_toy"] = (algo, 11, 3, 1.0, 4096)
+    dumps = []
+    try:
+        for run, steps in enumerate((7, 7, 8)):
+            eng = bench.build_learner("_toy", "cuda:0", seed=1000)[2]
+            for i in range(steps):
+                eng.iteration(i)
+            torch.cuda.synchronize()
+            bench.write_outputs(tmp_path / str(run), bench.timed_outputs(eng))
+            dumps.append({p.stem: np.load(p) for p in (tmp_path / str(run)).glob("*.npy")})
+    finally:
+        del bench.WORKLOADS["_toy"]
+    a, b, c = dumps
+    assert {"loss.qf_loss", "loss.actor_loss", "batch.observations", "batch.index", "actor.fc_stack.fc_block_1.fc.weight",
+            "qnet_target.fc_stack.fc_block_1.fc.weight"} <= a.keys()
+    assert ("actor_target.fc_stack.fc_block_1.fc.weight" in a) == (algo == "td3") and ("log_alpha" in a) == (algo == "sac")
+    assert a.keys() == b.keys() == c.keys()
+    assert all(v.dtype in (np.float32, np.float64) for v in a.values())
+    assert all(np.array_equal(a[k], b[k]) for k in a)
+    assert not np.array_equal(a["qnet.fc_stack.fc_block_1.fc.weight"], c["qnet.fc_stack.fc_block_1.fc.weight"])
