@@ -233,9 +233,20 @@ int b2rl_replay_extend(float* storage, int64_t capacity, int64_t cursor, b2rl_ro
 /* Graph-capturable variant of b2rl_replay_extend (orchestrator.py:100-113): the write cursor and the fill count
  * live on the device (counters[B2RL_CTR_CURSOR], counters[B2RL_CTR_SIZE]) and advance there, so one captured
  * graph can hold "copy the new transitions in -> write them -> sample -> update" and be replayed without host
- * patches. The last CTA to finish advances the counters (self-resetting ticket in counters[B2RL_CTR_XTICKET]). */
+ * patches. The last CTA to finish advances the counters (self-resetting ticket in counters[B2RL_CTR_XTICKET]).
+ * new_rows may be device memory or pinned host memory (device-addressable: the kernel then is the host->device copy).
+ * Same kernel and results as b2rl_replay_extend_dev_stack with n_agents = 1. */
 int b2rl_replay_extend_dev(float* storage, int64_t capacity, b2rl_rowfmt_t fmt, const float* new_rows, int32_t n,
                            uint64_t* counters, void* stream);
+
+/* b2rl_replay_extend_dev for n_agents stacked learners (a population: every member appends n transitions per step).
+ *   storage   [n_agents][..][row_stride], agent g's slice of `capacity` rows at storage + g * storage_agent_stride
+ *             (>= capacity * row_stride floats, a multiple of 4; any value when n_agents == 1)
+ *   new_rows  [n_agents][n][row_stride], contiguous, device or pinned host memory
+ *   counters  uint64[n_agents][8]: agent g's cursor, fill count and ticket are counters[g*8 + B2RL_CTR_CURSOR / _SIZE /
+ *             _XTICKET]; each agent's cursor and size advance on their own (the last CTA of agent g's grid row) */
+int b2rl_replay_extend_dev_stack(float* storage, int64_t storage_agent_stride, int64_t capacity, b2rl_rowfmt_t fmt,
+                                 const float* new_rows, int32_t n, int32_t n_agents, uint64_t* counters, void* stream);
 
 /* ---- stacked agents on the wide path ------------------------------------------------------------------------------------
  * Every entry point of the wide (layer-by-layer, tensor-core) path below takes a trailing `const b2rl_stack_t* stack`.
@@ -478,7 +489,10 @@ int b2rl_bump_counter(uint64_t* counters, int32_t which, int32_t n_agents, void*
  *   Philox keyed on (`draw`, a->agent_base = the learner's global id), `draw` < 2^31 advanced by the caller per call;
  *   draw = UINT64_MAX with a->counters set: keyed on counters[B2RL_CTR_Q] | 2^31, for use inside a captured step graph,
  *   a key space disjoint from the host-counted draws). `obs` and `actions_out` may be pinned host memory
- *   (device-addressable): the kernel then is the host<->device copy. */
+ *   (device-addressable): the kernel then is the host<->device copy.
+ * Stacked agents (a->n_agents > 1; 0 or 1 = one learner): agent g reads its actor at a->arena + g * a->arena_agent_stride,
+ *   its counters at a->counters + g * 8 (draw = UINT64_MAX), keys its noise on the global id a->agent_base + g, and
+ *   obs / a->eps / actions_out are [n_agents][n][..], contiguous. Each agent's actions equal those of a single call for it. */
 int b2rl_actor_predict(const b2rl_update_args_t* a, const float* obs, int32_t n, int32_t mode,
                        float explore_std, uint64_t draw, float* actions_out, void* stream);
 

@@ -104,6 +104,8 @@ SYMBOLS = {
                                             C.c_int32, C.c_int32, C.c_int32, C.c_void_p]),
     "b2rl_replay_extend": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, RowFmt, C.c_void_p, C.c_int32, C.c_void_p]),
     "b2rl_replay_extend_dev": (C.c_int, [C.c_void_p, C.c_int64, RowFmt, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]),
+    "b2rl_replay_extend_dev_stack": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, RowFmt, C.c_void_p, C.c_int32, C.c_int32,
+                                               C.c_void_p, C.c_void_p]),
     "b2rl_critic_update_sac": (C.c_int, [C.POINTER(UpdateArgs), C.c_void_p]),
     "b2rl_critic_update_td3": (C.c_int, [C.POINTER(UpdateArgs), C.c_void_p]),
     "b2rl_actor_update_sac": (C.c_int, [C.POINTER(UpdateArgs), C.c_void_p]),

@@ -377,15 +377,10 @@ predict_kernel(const __grid_constant__ b2rl_update_args_t A, const float* __rest
   const int nvalid = min(RT, n - b0);
   float4* X = reinterpret_cast<float4*>(smem_raw + sizeof(PredictSmem));
   const bool td3 = A.hp.td3 != 0;
-  const float* P = A.arena;
-  // draw = ~0: key the exploration noise on the critic step counter (a captured step graph cannot take a new
-  // host value per replay; the counter advances once per learner iteration). Bit 31 of the 32-bit step field separates
-  // these draws from the host-counted ones (draw = 1, 2, ... < 2^31), and the GLOBAL agent id is part of the key, so learners
-  // that share a seed (data-parallel ranks, population members) explore independently.
-  const uint64_t step = (draw == ~0ull && A.counters) ? (A.counters[B2RL_CTR_Q] | 0x80000000ull) : draw;
-  const uint32_t agent = (uint32_t)A.agent_base;
-  if (w == 0) stage_net(P, &A.actor, &M.ns, &M.n, G.c * CW);
-  else stage_tile(batch_row(obs, O, b0, nvalid), nvalid, 0, O, X, O, t - 32, NT - 32);
+  // stacked agents (grid y = local agent g; one learner: g = 0): g's actor, counters, observations, noise and actions
+  const int g = blockIdx.y;
+  if (w == 0) stage_net(A.arena + (size_t)g * A.arena_agent_stride, &A.actor, &M.ns, &M.n, G.c * CW);
+  else stage_tile(batch_row(obs + (size_t)g * n * O, O, b0, nvalid), nvalid, 0, O, X, O, t - 32, NT - 32);
   const Net& act = M.n;
   cp_async_wait_all();
   __syncthreads();
@@ -394,11 +389,17 @@ predict_kernel(const __grid_constant__ b2rl_update_args_t A, const float* __rest
   if (rank != 0) return;
   rowdot(act.p[F_W3], act.p[F_B3], act.out_dim, S.h[1], S.u);
   __syncthreads();
+  // draw = ~0: key the exploration noise on the critic step counter (a captured step graph cannot take a new
+  // host value per replay; the counter advances once per learner iteration). Bit 31 of the 32-bit step field separates
+  // these draws from the host-counted ones (draw = 1, 2, ... < 2^31), and the GLOBAL agent id is part of the key, so learners
+  // that share a seed (data-parallel ranks, population members) explore independently.
+  const uint64_t step = (draw == ~0ull && A.counters) ? (A.counters[(size_t)g * 8 + B2RL_CTR_Q] | 0x80000000ull) : draw;
+  const uint32_t agent = (uint32_t)(A.agent_base + g);
   for (int r = w; r < nvalid; r += NW) {
     if (l < AD) {
       const float lo = __ldg(A.min_ac + l), hi = __ldg(A.max_ac + l);
       const float scale = (hi - lo) * 0.5f, bias = (hi + lo) * 0.5f;
-      const int64_t e = (int64_t)(b0 + r) * AD + l;
+      const int64_t e = ((int64_t)g * n + b0 + r) * AD + l;  // [n_agents][n][AD]
       const float u0 = uref(S.u, r, l);
       float a;
       if (td3) {  // agents/nets.py:149-159
@@ -457,9 +458,10 @@ cudaError_t launch_predict(const b2rl_update_args_t& a, const float* obs, int n,
                            uint64_t draw, float* actions, cudaStream_t st) {
   const size_t smem = predict_smem_bytes(a.fmt.ob_dim);
   if (smem > (size_t)MAX_DYN_SMEM) return cudaErrorInvalidValue;
+  const dim3 grid(2 * row_blocks(n), a.n_agents > 1 ? a.n_agents : 1);  // n_agents 0 or 1: one learner, as before
   if (a.fmt.ob_dim > W1S_ROWS)
-    return launch_cluster(predict_kernel<true>, dim3(2 * row_blocks(n)), 2, smem, st, a, obs, n, mode, explore_std, draw, actions);
-  return launch_cluster(predict_kernel<false>, dim3(2 * row_blocks(n)), 2, smem, st, a, obs, n, mode, explore_std, draw, actions);
+    return launch_cluster(predict_kernel<true>, grid, 2, smem, st, a, obs, n, mode, explore_std, draw, actions);
+  return launch_cluster(predict_kernel<false>, grid, 2, smem, st, a, obs, n, mode, explore_std, draw, actions);
 }
 
 }  // namespace b2rl

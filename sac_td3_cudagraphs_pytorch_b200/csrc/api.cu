@@ -21,7 +21,7 @@ cudaError_t launch_gather(const float*, int64_t, int64_t, b2rl_rowfmt_t, int, in
                           uint64_t, uint64_t*, int, int, int, cudaStream_t);
 cudaError_t launch_extend(float*, int64_t, int64_t, b2rl_rowfmt_t, const float*, int, cudaStream_t);
 cudaError_t launch_publish(const float*, int, float*, uint64_t*, uint64_t*, cudaStream_t);
-cudaError_t launch_extend_dev(float*, int64_t, b2rl_rowfmt_t, const float*, int, uint64_t*, cudaStream_t);
+cudaError_t launch_extend_dev(float*, int64_t, int64_t, b2rl_rowfmt_t, const float*, int, int, uint64_t*, cudaStream_t);
 int max_in_dim_critic();
 int max_in_dim_actor();
 cudaError_t init_critic();
@@ -224,14 +224,25 @@ int b2rl_replay_extend(float* storage, int64_t capacity, int64_t cursor, b2rl_ro
   return check_launch(b2rl::launch_extend(storage, capacity, cursor, fmt, new_rows, n, (cudaStream_t)stream), "replay_extend");
 }
 
-int b2rl_replay_extend_dev(float* storage, int64_t capacity, b2rl_rowfmt_t fmt, const float* new_rows, int32_t n,
-                           uint64_t* counters, void* stream) {
+int b2rl_replay_extend_dev_stack(float* storage, int64_t storage_agent_stride, int64_t capacity, b2rl_rowfmt_t fmt,
+                                 const float* new_rows, int32_t n, int32_t n_agents, uint64_t* counters, void* stream) {
   if (int rc = check_fmt(fmt)) return rc;
   if (!storage || !new_rows || !counters || !aligned16(storage) || !aligned16(new_rows))
     return fail(B2RL_E_INVALID, "storage / new_rows / counters must be non-null, rows 16-byte aligned");
   if (capacity < 1 || n < 1 || n > capacity) return fail(B2RL_E_INVALID, "bad capacity / n");
-  return check_launch(b2rl::launch_extend_dev(storage, capacity, fmt, new_rows, n, counters, (cudaStream_t)stream),
+  if (n_agents < 1 || n_agents > 65535) return fail(B2RL_E_INVALID, "n_agents %d out of range", n_agents);
+  if (storage_agent_stride & 3) return fail(B2RL_E_INVALID, "storage_agent_stride must be a multiple of 4 floats");
+  if (n_agents > 1 && storage_agent_stride < capacity * fmt.row_stride)
+    return fail(B2RL_E_INVALID, "storage_agent_stride %lld is smaller than one agent's storage (capacity x row_stride)",
+                (long long)storage_agent_stride);
+  return check_launch(b2rl::launch_extend_dev(storage, storage_agent_stride, capacity, fmt, new_rows, n, n_agents, counters,
+                                              (cudaStream_t)stream),
                       "replay_extend_dev");
+}
+
+int b2rl_replay_extend_dev(float* storage, int64_t capacity, b2rl_rowfmt_t fmt, const float* new_rows, int32_t n,
+                           uint64_t* counters, void* stream) {
+  return b2rl_replay_extend_dev_stack(storage, 0, capacity, fmt, new_rows, n, 1, counters, stream);
 }
 
 int b2rl_tc_split_lo(const float* W, float* W_lo, int32_t n, const b2rl_stack_t* stack, void* stream) {
@@ -519,6 +530,10 @@ int b2rl_actor_predict(const b2rl_update_args_t* a, const float* obs, int32_t n,
   if (int rc = check_net(a->actor, "actor", false)) return rc;
   if (!a->arena || !a->min_ac || !a->max_ac) return fail(B2RL_E_INVALID, "predict: null device pointer");
   if (mode != 0 && mode != 1) return fail(B2RL_E_INVALID, "predict: mode must be 0 or 1");
+  if (a->n_agents < 0 || a->n_agents > 65535) return fail(B2RL_E_INVALID, "predict: n_agents %d out of range", a->n_agents);
+  if (a->n_agents > 1 && (a->agent_base < 0 || (int64_t)a->agent_base + a->n_agents > (1 << 30) || a->arena_agent_stride < 1 ||
+                          (a->arena_agent_stride & 3)))
+    return fail(B2RL_E_INVALID, "predict: stacked agents need ids below 2^30 and an arena agent stride that is a positive multiple of 4 floats");
   return check_launch(b2rl::launch_predict(*a, obs, n, mode, explore_std, draw, actions_out, (cudaStream_t)stream), "actor_predict");
 }
 

@@ -101,11 +101,17 @@ extend_kernel(float* __restrict__ storage, int64_t capacity, int64_t cursor, int
   }
 }
 
-// graph-capturable write: cursor and size live in the device counters; the last CTA to finish advances them
-__global__ void __launch_bounds__(256)
-extend_dev_kernel(float* __restrict__ storage, int64_t capacity, int row_stride, const float* __restrict__ new_rows, int n,
-                  uint64_t* __restrict__ counters) {
+// graph-capturable write: cursor and size live in the device counters; the last CTA to finish advances them.
+// Stacked agents: grid y = agent g, with its own storage slice, source rows [g][n][row_stride] and counters[g*8 + ..];
+// the last CTA of agent g's grid row advances g's cursor and size and resets g's ticket.
+__global__ void __launch_bounds__(256, 8)  // 8 resident CTAs per SM (launch_extend_dev's grid): <= 32 registers
+extend_dev_kernel(float* __restrict__ storage, int64_t storage_agent_stride, int64_t capacity, int row_stride,
+                  const float* __restrict__ new_rows, int n, uint64_t* __restrict__ counters) {
   pdl_enter();
+  const int g = blockIdx.y;
+  storage += (size_t)g * storage_agent_stride;
+  new_rows += (size_t)g * n * row_stride;
+  counters += (size_t)g * 8;
   const int chunks = row_stride >> 2;
   const int64_t total = (int64_t)n * chunks;
   const int64_t cursor = (int64_t)counters[B2RL_CTR_CURSOR];
@@ -127,13 +133,14 @@ extend_dev_kernel(float* __restrict__ storage, int64_t capacity, int row_stride,
   }
 }
 
-cudaError_t launch_extend_dev(float* storage, int64_t capacity, b2rl_rowfmt_t fmt, const float* new_rows, int n,
-                              uint64_t* counters, cudaStream_t st) {
+cudaError_t launch_extend_dev(float* storage, int64_t storage_agent_stride, int64_t capacity, b2rl_rowfmt_t fmt,
+                              const float* new_rows, int n, int n_agents, uint64_t* counters, cudaStream_t st) {
   const int64_t total = (int64_t)n * (fmt.row_stride >> 2);
   int ctas = (int)((total + 255) / 256);
   if (ctas > 148 * 8) ctas = 148 * 8;
   if (ctas < 1) ctas = 1;
-  return launch_k(extend_dev_kernel, dim3(ctas), dim3(256), 1, 0, st, storage, capacity, (int)fmt.row_stride, new_rows, n, counters);
+  return launch_k(extend_dev_kernel, dim3(ctas, n_agents), dim3(256), 1, 0, st, storage, storage_agent_stride, capacity,
+                  (int)fmt.row_stride, new_rows, n, counters);
 }
 
 // last node of a captured step: log block -> pinned host memory, then the sequence number the host polls

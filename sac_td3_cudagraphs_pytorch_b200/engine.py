@@ -22,6 +22,7 @@ import torch
 from . import _lib as L
 from .agents.agent import Agent
 from .replay import Batch, ReplayBuffer
+from .staging import StepStaging
 
 
 class LearnerEngine:
@@ -57,27 +58,13 @@ class LearnerEngine:
         self._size_on_device = -1
         self._cursor_on_device = -1
         self.launches_per_variant: dict[tuple, int] = {}
-        # end-to-end step (step()): pinned staging for the transitions coming in and the log block going out
-        self._h_new: dict[int, torch.Tensor] = {}
-        # two slots each (step parity): one step may be in flight while the host prepares the next (step_async / wait)
-        self._host_outs = [torch.zeros(8, dtype=torch.float32).pin_memory() for _ in range(2)]
-        self.host_out = self._host_outs[0]
-        self._host_outs_np = [t.numpy() for t in self._host_outs]
-        self._waited = 0
-        # the behaviour policy inside the step graph (step_async(..., n_obs=)): observations in, actions out, both pinned
-        self._h_obs: dict[tuple, torch.Tensor] = {}
-        self._h_act: dict[tuple, torch.Tensor] = {}
-        self._d_act: dict[int, torch.Tensor] = {}
-        self._host_act_seq = torch.zeros(1, dtype=torch.int64).pin_memory()
-        self._host_act_seq_np = self._host_act_seq.numpy()
-        self._act_seq_dev = torch.zeros(1, dtype=torch.int64, device=dev)
-        self._act_seq, self._act_last = 0, None
+        # end-to-end step (step_async / wait): pinned staging for the transitions and observations coming in, the log
+        # block and the actions going out, two slots each (step parity) so one step may be in flight while the host
+        # prepares the next
+        self._stage = StepStaging(dev, (), agent.fmt.row_stride, agent.ob_dim, agent.ac_dim)
+        self.host_out = self._stage.host_outs[0]
         self._keep: list = []
         self._side_stream = torch.cuda.Stream(device=dev)
-        self._host_seq = torch.zeros(1, dtype=torch.int64).pin_memory()
-        self._host_seq_np = self._host_seq.numpy()  # (a view: polled without going through torch)
-        self._seq_dev = torch.zeros(1, dtype=torch.int64, device=dev)
-        self._seq = 0
 
     # -- what one iteration enqueues --------------------------------------------------------------
     def _enqueue(self, do_actor: bool, do_polyak: bool, args_q=None, before_last_adam=None) -> int:
@@ -124,49 +111,18 @@ class LearnerEngine:
         (replay.pack_rows(td, fmt, out=...)) and call step(i, n) / step_async(i, n). There are two slots (the parity
         of the step's sequence number; default: the next step's), so the buffer of step t may be filled while step
         t - 1 is still running — but only after wait() of step t - 2, which read from the same slot."""
-        slot = (self._seq & 1) if slot is None else int(slot) & 1
-        if (n, slot) not in self._h_new:
-            self._h_new[(n, slot)] = torch.zeros(n, self.agent.fmt.row_stride, dtype=torch.float32).pin_memory()
-        return self._h_new[(n, slot)]
+        return self._stage.rows(n, slot)
 
     def host_obs(self, n: int, slot: Optional[int] = None) -> torch.Tensor:
         """Pinned staging buffer [n, ob_dim] for the observations the policy acts on in the next step
         (step_async(..., n_obs=n)); two slots, like host_rows."""
-        slot = (self._seq & 1) if slot is None else int(slot) & 1
-        if (n, slot) not in self._h_obs:
-            ag = self.agent
-            self._h_obs[(n, slot)] = torch.zeros(n, ag.ob_dim, dtype=torch.float32).pin_memory()
-            blocks = (n * ag.ac_dim + 7) // 8  # b2rl_publish_logs copies blocks of 8 floats
-            self._h_act[(n, slot)] = torch.zeros(blocks * 8, dtype=torch.float32).pin_memory()
-            if n not in self._d_act:
-                self._d_act[n] = torch.zeros(blocks * 8, dtype=torch.float32, device=ag.device)
-        return self._h_obs[(n, slot)]
+        return self._stage.obs(n, slot)
 
     def wait_actions(self) -> "np.ndarray":
         """Actions of the last step launched with n_obs > 0 ([n_obs, A], a view of pinned host memory written by the
         device; valid until the step two launches later): polls the sequence number the step's policy part publishes
         — it runs FIRST in the graph, so the environments can step while the update of the same replay runs."""
-        n, slot, want = self._act_last
-        self._poll(self._host_act_seq_np, want, "the policy's actions")
-        ag = self.agent
-        return self._h_act[(n, slot)].numpy()[: n * ag.ac_dim].reshape(n, ag.ac_dim)
-
-    def _poll(self, seq, want: int, what: str, timeout_s: float = 30.0) -> None:
-        """Spin on a pinned sequence number the device publishes. Every 4096 empty polls the stream is queried: a step
-        that has FINISHED without publishing (a faulted replay: the publish kernel never ran) or a deadline miss raises
-        instead of hanging the host."""
-        spins, t0 = 0, None
-        while seq[0] < want:
-            spins += 1
-            if spins & 0xFFF:
-                continue
-            import time
-            t0 = t0 or time.monotonic()
-            done = torch.cuda.current_stream(self.agent.device).query()  # raises on a sticky CUDA error
-            if done and seq[0] < want:
-                raise L.B2rlError(f"the stream drained but {what} was never published (sequence {int(seq[0])} < {want})")
-            if time.monotonic() - t0 > timeout_s:
-                raise L.B2rlError(f"timed out after {timeout_s:.0f} s waiting for {what} (sequence {int(seq[0])} < {want})")
+        return self._stage.actions()
 
     def step_async(self, i: int, n_new: int = 0, n_obs: int = 0, explore: bool = True) -> int:
         """orchestrator.py:100-113 + :337-352 as ONE CUDA graph replay and no stream synchronisation: the replay
@@ -180,9 +136,7 @@ class LearnerEngine:
         the reference loop — and publishes the actions to pinned host memory: wait_actions()."""
         ag, rb = self.agent, self.rb
         assert self.use_graphs, "step() is the graph path"
-        if self._seq - self._waited >= 2:
-            self.wait(self._seq - 1)
-        slot = self._seq & 1
+        slot = self._stage.begin()
         do_actor = (i % (ag.hps.actor_update_delay + 1) == 0)
         key = (do_actor, self._polyak_due(), int(n_new), slot, int(n_obs), bool(explore))
         self._sync_size()
@@ -197,30 +151,23 @@ class LearnerEngine:
         ag.qnet_updates_so_far += 1
         if do_actor:
             ag.actor_updates_so_far += int(ag.hps.actor_update_delay)
-        self._seq += 1
-        if n_obs:
-            self._act_seq += 1
-            self._act_last = (int(n_obs), slot, self._act_seq)
-        return self._seq
+        return self._stage.launched(n_obs, slot)
 
     def wait(self, ticket: int, as_numpy: bool = False):
         """Poll the sequence number the step's last kernel publishes; returns that step's pinned log block
         (_lib.OUT_* indices; a torch tensor, or its numpy view), valid until the step two tickets later is launched."""
-        self._poll(self._host_seq_np, ticket, "the step's log block")  # written after the log block (system-scope fence)
-        self._waited = max(self._waited, int(ticket))
-        return (self._host_outs_np if as_numpy else self._host_outs)[(ticket - 1) & 1]
+        return self._stage.wait(ticket, as_numpy)
 
     def step(self, i: int, n_new: int = 0, n_obs: int = 0, explore: bool = True) -> torch.Tensor:
         """step_async + wait: the loop of a trainer that reads the losses of every step before the next one."""
         return self.wait(self.step_async(i, n_new, n_obs, explore))
 
     def _capture_step(self, key) -> torch.cuda.CUDAGraph:
-        ag, rb = self.agent, self.rb
+        ag, rb, stage = self.agent, self.rb, self._stage
         do_actor, do_polyak, n_new, slot, n_obs, explore = key
-        if n_new:
-            self.host_rows(n_new, slot)
+        new_rows = stage.rows(n_new, slot) if n_new else None
         if n_obs:
-            self.host_obs(n_obs, slot)
+            obs = stage.obs(n_obs, slot)
             pa = L.UpdateArgs()
             pa.hp, pa.fmt, pa.actor = ag._hyper, ag.fmt, ag.layout.actor.c_struct()
             pa.arena, pa.region_stride, pa.agent_base = ag.arena.flat.data_ptr(), ag.layout.region, ag.agent_id
@@ -232,23 +179,21 @@ class LearnerEngine:
             n = 0
             if n_obs:  # the policy first: the environments get their actions while the update runs
                 std = float(ag.hps.actor_noise_std) if ag.td3 else 0.0
-                L.check(ag._lib.b2rl_actor_predict(C.byref(pa), self._h_obs[(n_obs, slot)].data_ptr(), n_obs, int(explore), std,
-                                                   C.c_uint64(2 ** 64 - 1), self._d_act[n_obs].data_ptr(), ag._stream()),
+                L.check(ag._lib.b2rl_actor_predict(C.byref(pa), obs.data_ptr(), n_obs, int(explore), std,
+                                                   C.c_uint64(2 ** 64 - 1), stage.device_actions(n_obs).data_ptr(), ag._stream()),
                         "actor_predict")
-                L.check(ag._lib.b2rl_publish_logs(self._d_act[n_obs].data_ptr(), self._d_act[n_obs].numel() // 8,
-                                                  self._h_act[(n_obs, slot)].data_ptr(), self._act_seq_dev.data_ptr(),
-                                                  self._host_act_seq.data_ptr(), ag._stream()), "publish actions")
+                stage.publish_actions(ag._lib, n_obs, slot, ag._stream())
                 n += 2
             args_q = None
             if n_new and self.fused_sample and not self.fused_opt:
                 # the replay write rides in the critic step too (b2rl_update_args_t.new_rows): the kernel reads the pinned
                 # rows itself (UVA), no separate write launch
                 args_q = ag.update_args(self.rows, eps_out=self.noise_q, storage=rb.storage, idx_out=self.idx,
-                                        new_rows=self._h_new[(n_new, slot)], n_new=n_new)
+                                        new_rows=new_rows, n_new=n_new)
                 self._keep.append(args_q)
             elif n_new:  # pinned host memory is device-addressable (UVA): the write kernel is the host->device copy
                 L.check(ag._lib.b2rl_replay_extend_dev(rb.storage.data_ptr(), rb.capacity, rb.fmt,
-                                                       self._h_new[(n_new, slot)].data_ptr(), n_new, ag.counters.data_ptr(),
+                                                       new_rows.data_ptr(), n_new, ag.counters.data_ptr(),
                                                        ag._stream()), "replay_extend_dev")
                 n += 1
             # The log block is final before the iteration's last Adam launch (unless SAC's temperature step follows):
@@ -256,8 +201,7 @@ class LearnerEngine:
             joined = []
 
             def publish():
-                L.check(ag._lib.b2rl_publish_logs(ag.out.data_ptr(), 1, self._host_outs[slot].data_ptr(),
-                                                  self._seq_dev.data_ptr(), self._host_seq.data_ptr(), ag._stream()), "publish_logs")
+                stage.publish_logs(ag._lib, ag.out, slot, ag._stream())
 
             def fork_publish():
                 main, ev = torch.cuda.current_stream(ag.device), torch.cuda.Event()

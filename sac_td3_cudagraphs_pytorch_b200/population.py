@@ -7,6 +7,12 @@ live in one arena `[N, 5, region]` and every kernel of the update takes the agen
 Nothing is shared and nothing is reduced between agents; sharding a population over GPUs is a partition
 of the agent ids (`shard`) with no collective, and because every random draw is keyed on the GLOBAL agent
 id the results do not depend on the partition (tests/test_gpu_population.py).
+
+Training against environments (the reference loop, orchestrator.py:317-352: predict -> env step -> rb.extend -> update)
+runs N seeds at once: `predict` (the stacked behaviour policy) and `extend` (every agent appends n transitions to its own
+slice) are the eager collection path before learning starts; `step_async` / `wait` / `wait_actions` run policy, replay
+write, iteration and the log block as ONE graph replay per step, like LearnerEngine.step_async for one learner
+(tests/test_gpu_population_step.py).
 """
 from __future__ import annotations
 
@@ -22,6 +28,7 @@ from .agents.agent import HID_DIMS
 from .agents.nets import Actor, Critic, TanhGaussActor
 from .arena import Arena, make_layout, set_shadow_pairs
 from .replay import pack_rows, row_format
+from .staging import StepStaging
 
 
 def shard(n_total: int, world: int, rank: int) -> range:
@@ -109,7 +116,8 @@ class Population:
         self.idx = torch.zeros(N, self.B, dtype=torch.int64, device=dev)
         self.capacity = int(rb_capacity)
         self.storage = torch.zeros(N, self.capacity, self.fmt.row_stride, dtype=torch.float32, device=dev)
-        self.size = 0
+        self.size = 0  # host mirror of every agent's replay fill count and write cursor (counters[:, SIZE / CURSOR])
+        self.cursor = 0
         self.iterations = 0
         self.graphs: dict = {}
         self.launches_per_variant: dict = {}
@@ -127,6 +135,8 @@ class Population:
             own = _Owner(self)
             self.wide_q = WideCritic(own, self.B, wide)
             self.wide_pi = WideActor(own, self.B, wide)
+        self._stage = StepStaging(dev, (N,), self.fmt.row_stride, self.ob_dim, self.ac_dim)
+        self._predict_draw = 0
 
     # ------------------------------------------------------------------ replay
     def fill_replay(self, td: Mapping[str, torch.Tensor], agent: Optional[int] = None) -> None:
@@ -139,7 +149,63 @@ class Population:
         else:
             self.storage[agent, :n] = rows
         self.size = max(self.size, n)
+        self.cursor = n % self.capacity
         self.counters[:, L.CTR_SIZE] = self.size
+        self.counters[:, L.CTR_CURSOR] = self.cursor
+
+    def _launch_extend(self, rows_ptr: int, n: int) -> None:
+        L.check(self._lib.b2rl_replay_extend_dev_stack(self.storage.data_ptr(), self.storage[0].numel(), self.capacity, self.fmt,
+                                                       rows_ptr, n, self.N, self.counters.data_ptr(), self._stream()),
+                "replay_extend_dev_stack")
+
+    def _advance(self, n: int) -> None:
+        self.cursor = (self.cursor + n) % self.capacity
+        self.size = min(self.capacity, self.size + n)
+
+    def extend(self, rows: torch.Tensor) -> None:
+        """rb.extend(td) (orchestrator.py:100-113) for every agent at once: rows [N, n, row_stride] (replay.pack_rows
+        layout; device or pinned host memory, which the write kernel reads itself) are appended round robin to each
+        agent's slice at the shared cursor. Enqueued only: a pinned source must stay untouched until the stream has
+        passed this point."""
+        if not isinstance(rows, torch.Tensor) or rows.dim() != 3 or rows.shape[0] != self.N or \
+                rows.shape[2] != self.fmt.row_stride or rows.dtype != torch.float32:
+            raise L.B2rlError(f"extend: rows must be float32 [{self.N}, n, {self.fmt.row_stride}], got "
+                              f"{getattr(rows, 'dtype', type(rows))} {tuple(getattr(rows, 'shape', ()))}")
+        n = rows.shape[1]
+        if not 1 <= n <= self.capacity:
+            raise L.B2rlError(f"extend: n = {n} transitions per agent must be in [1, capacity = {self.capacity}]")
+        rows = rows.contiguous()
+        if not (rows.is_cuda or rows.is_pinned()):
+            rows = rows.to(self.device)
+        self._launch_extend(rows.data_ptr(), n)
+        self._advance(n)
+
+    # ------------------------------------------------------------------ behaviour policy
+    def _launch_predict(self, args: L.UpdateArgs, obs_ptr: int, n: int, explore: bool, draw: int, act_ptr: int) -> None:
+        std = float(self.hps.actor_noise_std) if self.td3 else 0.0
+        L.check(self._lib.b2rl_actor_predict(C.byref(args), obs_ptr, n, int(explore), std, C.c_uint64(draw), act_ptr,
+                                             self._stream()), "actor_predict")
+
+    def predict(self, obs: torch.Tensor, explore: bool, eps: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Agent.predict (agents/agent.py:172-181) for every agent: obs [N, n, ob_dim] -> actions [N, n, A] (device).
+        explore: SAC sample / TD3 action + exploration noise; otherwise SAC mode / TD3 action (evaluation episodes).
+        The noise is Philox keyed on a host-counted draw and the global agent id (or eps [N, n, A] when given), so each
+        call draws new noise and agent g's actions equal Agent(agent_id=base + g).predict_device."""
+        obs = torch.as_tensor(obs).to(device=self.device, dtype=torch.float32).contiguous()
+        if obs.dim() != 3 or obs.shape[0] != self.N or obs.shape[2] != self.ob_dim or obs.shape[1] < 1:
+            raise L.B2rlError(f"predict: obs must be [{self.N}, n, {self.ob_dim}], got {tuple(obs.shape)}")
+        n = obs.shape[1]
+        act = torch.empty(self.N, n, self.ac_dim, dtype=torch.float32, device=self.device)
+        args = self.args
+        if eps is not None:
+            eps = torch.as_tensor(eps).to(device=self.device, dtype=torch.float32).contiguous()
+            if tuple(eps.shape) != (self.N, n, self.ac_dim):
+                raise L.B2rlError(f"predict: eps must be [{self.N}, {n}, {self.ac_dim}], got {tuple(eps.shape)}")
+            args = L.UpdateArgs.from_buffer_copy(self.args)
+            args.eps = eps.data_ptr()
+        self._predict_draw += 1
+        self._launch_predict(args, obs.data_ptr(), n, explore, self._predict_draw, act.data_ptr())
+        return act
 
     # ------------------------------------------------------------------ enqueue
     def _stream(self) -> int:
@@ -223,13 +289,16 @@ class Population:
                 n += 1
         return n
 
-    def iteration(self, i: Optional[int] = None) -> None:
-        """One learner iteration (orchestrator.py:337-352) for every agent of the population."""
-        i = self.iterations if i is None else i
+    def _variant(self, i: int) -> tuple:
         h = self.hps
         do_actor = (i % (h.actor_update_delay + 1) == 0)
         do_polyak = self.td3 or ((self.iterations + 1) % h.crit_targ_update_freq == 0)
-        key = (do_actor, do_polyak)
+        return do_actor, do_polyak
+
+    def iteration(self, i: Optional[int] = None) -> None:
+        """One learner iteration (orchestrator.py:337-352) for every agent of the population."""
+        i = self.iterations if i is None else i
+        key = self._variant(i)
         if not self.use_graphs:
             self.launches_per_variant[key] = self._enqueue(*key)
         else:
@@ -242,6 +311,78 @@ class Population:
                 self.graphs[key] = g
             g.replay()
         self.iterations += 1
+
+    # ------------------------------------------------------------------ the environment-facing step
+    def host_rows(self, n: int, slot: Optional[int] = None) -> torch.Tensor:
+        """Pinned staging buffer [N, n, row_stride] for the transitions of the next step (n per agent); two slots, as
+        LearnerEngine.host_rows: the buffer of step t may be filled while step t - 1 runs, after wait() of step t - 2."""
+        return self._stage.rows(n, slot)
+
+    def host_obs(self, n: int, slot: Optional[int] = None) -> torch.Tensor:
+        """Pinned staging buffer [N, n, ob_dim] for the observations the policy acts on in the next step; two slots."""
+        return self._stage.obs(n, slot)
+
+    def wait_actions(self) -> "np.ndarray":
+        """Actions [N, n_obs, A] of the last step launched with n_obs > 0 (a view of pinned host memory; valid until the
+        step two launches later). The policy runs first in the step graph: the environments can step while the
+        update runs."""
+        return self._stage.actions()
+
+    def wait(self, ticket: int, as_numpy: bool = False):
+        """The log block [N, 8] (_lib.OUT_* columns) of the step with this ticket, from pinned host memory; valid until
+        the step two tickets later is launched."""
+        return self._stage.wait(ticket, as_numpy)
+
+    def step(self, i: Optional[int] = None, n_new: int = 0, n_obs: int = 0, explore: bool = True) -> torch.Tensor:
+        """step_async + wait."""
+        return self.wait(self.step_async(i, n_new, n_obs, explore))
+
+    def step_async(self, i: Optional[int] = None, n_new: int = 0, n_obs: int = 0, explore: bool = True) -> int:
+        """One step of the reference loop for every agent as ONE graph replay, without a stream synchronisation:
+        the behaviour policy on the n_obs observations per agent in host_obs(n_obs) (parameters before this step's
+        update; actions published to pinned memory: wait_actions()), the replay write of the n_new transitions per agent
+        in host_rows(n_new), the iteration (sample over each agent's grown replay, updates, Adam / Polyak) and the log
+        block (wait()). Returns a ticket; at most two steps are in flight. Needs graphs."""
+        if not self.use_graphs:
+            raise L.B2rlError("step_async is the graph path: build the Population with use_graphs=True")
+        n_new, n_obs = int(n_new), int(n_obs)
+        if not 0 <= n_new <= self.capacity or n_obs < 0:
+            raise L.B2rlError(f"step_async: need 0 <= n_new <= capacity ({self.capacity}) and n_obs >= 0")
+        if self.size + n_new < 1:
+            raise L.B2rlError("step_async: the replay is empty (fill_replay / extend first, or pass n_new > 0)")
+        slot = self._stage.begin()
+        i = self.iterations if i is None else i
+        key = self._variant(i) + (n_new, slot, n_obs, bool(explore))
+        g = self.graphs.get(key)
+        if g is None:
+            g = self._capture_step(key)
+        g.replay()
+        if n_new:
+            self._advance(n_new)
+        self.iterations += 1
+        return self._stage.launched(n_obs, slot)
+
+    def _capture_step(self, key) -> torch.cuda.CUDAGraph:
+        do_actor, do_polyak, n_new, slot, n_obs, explore = key
+        stage = self._stage
+        new_rows = stage.rows(n_new, slot) if n_new else None
+        obs = stage.obs(n_obs, slot) if n_obs else None
+        g = torch.cuda.CUDAGraph()
+        torch.cuda.synchronize(self.device)
+        with torch.cuda.graph(g):
+            n = 0
+            if n_obs:  # noise keyed on each agent's critic step counter (draw = UINT64_MAX), as in LearnerEngine's step
+                self._launch_predict(self.args, obs.data_ptr(), n_obs, explore, 2 ** 64 - 1, stage.device_actions(n_obs).data_ptr())
+                stage.publish_actions(self._lib, n_obs, slot, self._stream())
+                n += 2
+            if n_new:  # pinned host memory is device-addressable: the write kernel is the host->device copy
+                self._launch_extend(new_rows.data_ptr(), n_new)
+                n += 1
+            m = self._enqueue(do_actor, do_polyak)  # (-1: the wide path does not count its launches)
+            stage.publish_logs(self._lib, self.out, slot, self._stream())
+        self.launches_per_variant[key] = -1 if m < 0 else n + m + 1
+        self.graphs[key] = g
+        return g
 
     # ------------------------------------------------------------------ inspection
     def agent_arena(self, g: int) -> torch.Tensor:
