@@ -122,6 +122,19 @@ def test_wide_population_matches_the_fp32_row_path(algo):
         for k in (L.OUT_QF_LOSS, L.OUT_ACTOR_LOSS):
             a, b = float(wide.out[g, k]), float(row.out[g, k])
             assert abs(a - b) <= 2e-5 * max(abs(b), 1e-3), (g, k, a, b)
+        if algo == "sac":
+            # The temperature step draws its own noise (stream 3, keyed on the actor counter after the actor step advanced
+            # it), so it checks that key on the wide path. Its loss alpha * (mean(-logpi) - targ_ent) is a difference of
+            # O(A) terms, judged against alpha * A (helpers.alpha_loss_scale). A draw keyed on another counter moves
+            # mean(-logpi) by ~sqrt(A / 2B) ~ 0.08, i.e. ~3e-2 of that scale. Measured on a B200: <= 5e-7 of alpha * A, and
+            # log alpha equal after the two Adam steps.
+            a, b = float(wide.out[g, L.OUT_ALPHA_LOSS]), float(row.out[g, L.OUT_ALPHA_LOSS])
+            sc = float(row.out[g, L.OUT_ALPHA]) * 3
+            la_w, la_r = float(wide.alpha_state[g, 0]), float(row.alpha_state[g, 0])
+            print(f"agent {ids[g]}: alpha loss wide {a:.7f} row {b:.7f} (|d| / alpha A = {abs(a - b) / sc:.2e}), "
+                  f"log alpha |d| {abs(la_w - la_r):.2e}")
+            assert abs(a - b) <= 1e-4 * sc, (g, a, b)
+            assert abs(la_w - la_r) <= 1e-6, (g, la_w, la_r)
         for c in lay.critic:  # (the reference's tensors: the w2n shadow has no gradient of its own on the wide path)
             gw = wide.arena.flat[g, L.REGION_G, c.begin:c.core_end]
             gr = row.arena.flat[g, L.REGION_G, c.begin:c.core_end]

@@ -295,25 +295,6 @@ def test_full_size_properties(algo, ob, ac, bound):
     assert a.shape == (4, ac) and np.all(np.abs(a) <= bound + 1e-6)
 
 
-def test_predict_matches_torch_forward():
-    for name in ("sac_hopper", "td3_hopper", "sac_humanoid"):
-        inp = case_inputs(name)
-        ag = make_agent(inp)
-        obs = inp["storage"]["observations"][:7].cuda()
-        eps = inp["eps_q"][0][:7].cuda()
-        with torch.no_grad():
-            if ag.td3:
-                want0 = ag.actor_detach(obs)
-                want1 = want0 + eps * (ag.actor_detach.action_scale * ag.actor_detach.exploration_noise)
-            else:
-                r = ag.actor_detach.get_action(obs, eps)
-                want0, want1 = r["mode"], r["sample"]
-        got0 = ag.predict_device(obs, explore=False)
-        got1 = ag.predict_device(obs, explore=True, eps=eps)
-        assert torch.allclose(got0, want0, rtol=1e-5, atol=2e-6), name
-        assert torch.allclose(got1, want1, rtol=1e-5, atol=2e-6), name
-
-
 def test_errors_are_loud():
     from sac_td3_cudagraphs_pytorch_b200 import _lib as L, sac_hps
     from sac_td3_cudagraphs_pytorch_b200.agents.agent import Agent
