@@ -163,7 +163,7 @@ typedef struct b2rl_seg {
   int32_t do_polyak;   /* target <- lerp(target, p, polyak)   agents/agent.py:328-331 */
   int32_t counter;     /* B2RL_CTR_* holding this optimizer's step count (read, not bumped) */
   float grad_scale;    /* multiplies g first (1/world for data parallel; 1 otherwise) */
-  int32_t clip;        /* 1: scale g by min(1, clip_norm/(norm+1e-6)), norm from b2rl_grad_norm */
+  int32_t clip;        /* 1: scale g by min(1, clip_norm/(norm+1e-6)), norm = sqrt(b2rl_grad_sumsq) * grad_scale */
 } b2rl_seg_t;
 
 typedef struct b2rl_adam_args {
@@ -450,7 +450,9 @@ int b2rl_actor_update_td3(const b2rl_update_args_t* a, void* stream);
  * a->hp.td3. opt->seg[0] must be an Adam segment (clip = 0, grad_scale = 1) over exactly the trained nets
  * ([critic[0].begin, critic[1].end) / [actor.begin, actor.end)) with the matching counter; further segments must
  * be Polyak-only spans (e.g. TD3's actor target in an iteration without actor update). Gradient clipping and
- * data-parallel training need the gradients complete before the step: use the three-launch form there. */
+ * data-parallel training need the gradients complete before the step: use the three-launch form there. The
+ * 3xTF32 mirror is not written here: opt->lo must be NULL (B2RL_E_INVALID otherwise, before any launch), and a
+ * learner that keeps a mirror uses the three-launch form. */
 int b2rl_critic_update_opt(const b2rl_update_args_t* a, const b2rl_adam_args_t* opt, void* stream);
 int b2rl_actor_update_opt(const b2rl_update_args_t* a, const b2rl_adam_args_t* opt, void* stream);
 

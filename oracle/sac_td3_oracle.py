@@ -239,7 +239,11 @@ class _Adam:
     ``capturable=False`` follows torch/optim/adam.py:528-550 (bias corrections in host
     float64, ``addcdiv_(m, denom, value=-step_size)``); ``capturable=True`` follows
     :478-527 (fp32 device scalars, ``denom = sqrt(v)/(bc2_sqrt*(-ss)) + eps/(-ss)``;
-    ``p += m/denom``). Checked against torch.optim.Adam in tests/test_oracle_adam.py.
+    ``p += m/denom``). In the capturable branch the step count is a float32 tensor, so the
+    bias corrections are fp32 whatever the dtype of the parameters: a float64 oracle is
+    float64 in its optimizer only with ``capturable=False``. Checked against
+    torch.optim.Adam in tests/test_gpu_optimizer.py (``test_oracle_adam_matches_torch``:
+    both branches, the capturable one on the GPU).
     """
 
     def __init__(self, params, lr, capturable=False, b1=0.9, b2=0.999, eps=1e-8):

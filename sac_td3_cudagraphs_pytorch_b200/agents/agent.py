@@ -261,8 +261,11 @@ class Agent:
     def lo_mirror(self) -> torch.Tensor:
         """[1][2][region]: the "lo parts" p - tf32(p) of the online and target regions, at the parameters' own offsets —
         the second operand of the 3xTF32 tensor-core products (wide.py). Created on first use; from then on every
-        Adam / Polyak launch of this agent keeps it current (b2rl_adam_args_t.lo). Host-side writes to the parameters
-        (load_params, load_from_disk do it themselves; module.load_state_dict does not) need refresh_lo()."""
+        Adam / Polyak launch of this agent keeps it current (b2rl_adam_args_t.lo); steps that asked for the fused
+        optimizer take the three-launch form from then on (fuses_opt). Host-side writes to the parameters
+        (load_params, load_from_disk do it themselves; module.load_state_dict does not) need refresh_lo().
+        Create the mirror before capturing any graph of this agent: a graph captured without it keeps launching with
+        lo = NULL (and, if it was captured with the fused optimizer, keeps the fused form), so the mirror goes stale."""
         if self._lo is None:
             self._lo = torch.zeros(1, 2, self.layout.region, dtype=torch.float32, device=self.device)
             self.refresh_lo()
@@ -297,11 +300,17 @@ class Agent:
         return segs
 
     # ------------------------------------------------------------------ enqueue-only steps (graph-safe)
+    def fuses_opt(self, fused_opt: bool = True) -> bool:
+        """Whether a step asked for the fused optimizer (b2rl_*_update_opt) gets it: not while a lo mirror exists,
+        which only the stand-alone Adam / Polyak launch keeps current."""
+        return bool(fused_opt) and self._lo is None
+
     def enqueue_critic_step(self, args: L.UpdateArgs, extra_segs: list = (), polyak: bool = False,
                             fused_opt: bool = True, before_adam=None) -> None:
         """update_qnets incl. optimizer.step(): fused kernel + weight gradients with Adam (and Polyak) applied in the
-        same launch (fused_opt), or the three-launch form (fused kernel, weight gradients, Adam/Polyak)."""
-        if fused_opt:
+        same launch (fused_opt), or the three-launch form (fused kernel, weight gradients, Adam/Polyak). The fused form
+        does not write the 3xTF32 mirror, so an agent that has one (lo_mirror()) takes the three-launch form."""
+        if self.fuses_opt(fused_opt):
             opt = self._adam_args(self.critic_segs(polyak) + list(extra_segs))
             L.check(self._lib.b2rl_critic_update_opt(C.byref(args), C.byref(opt), self._stream()), "critic_update_opt")
             return
@@ -313,7 +322,7 @@ class Agent:
 
     def enqueue_actor_step(self, args: L.UpdateArgs, polyak: bool = False, fused_opt: bool = True, before_adam=None) -> None:
         st = self._stream()
-        if fused_opt and not self.hps.clip_norm > 0:  # (clipping needs the whole gradient's norm before the step)
+        if self.fuses_opt(fused_opt) and not self.hps.clip_norm > 0:  # (clipping needs the whole gradient's norm first)
             opt = self._adam_args(self.actor_segs(polyak))
             L.check(self._lib.b2rl_actor_update_opt(C.byref(args), C.byref(opt), st), "actor_update_opt")
             if self.autotune:

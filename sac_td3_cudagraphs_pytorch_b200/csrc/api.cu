@@ -421,6 +421,8 @@ int b2rl_publish_logs(const float* out, int32_t n_agents, float* host_out, uint6
 static int check_opt(const b2rl_update_args_t* a, const b2rl_adam_args_t* o, int64_t begin, int64_t end, int counter) {
   if (!o) return B2RL_OK;
   if (o->n_seg < 1 || o->n_seg > B2RL_MAX_SEG) return fail(B2RL_E_INVALID, "opt: n_seg %d out of range", o->n_seg);
+  if (o->lo)  // (the weight-gradient kernel does not write the 3xTF32 mirror: it would go stale)
+    return fail(B2RL_E_INVALID, "opt: the fused optimizer does not keep a lo mirror current; use the three-launch form");
   const b2rl_seg_t& s0 = o->seg[0];
   if (!s0.do_adam || s0.clip || s0.grad_scale != 1.0f || s0.begin != begin || s0.end != end || s0.counter != counter)
     return fail(B2RL_E_INVALID, "opt: seg[0] must be an unclipped, unscaled Adam segment over the trained nets");

@@ -82,15 +82,16 @@ class LearnerEngine:
         delay = int(ag.hps.actor_update_delay) if do_actor else 0
         # TD3's target actor is averaged once per iteration, after the last actor update if there is one
         extra = ag.polyak_segs(critics=False, actor=True) if (ag.td3 and do_polyak and delay == 0) else []
-        hook = None if self.fused_opt else before_last_adam
-        ag.enqueue_critic_step(args_q, extra_segs=extra, polyak=do_polyak, fused_opt=self.fused_opt,
+        fused = ag.fuses_opt(self.fused_opt)  # (not with a lo mirror: only the stand-alone Adam launch writes it)
+        hook = None if fused else before_last_adam
+        ag.enqueue_critic_step(args_q, extra_segs=extra, polyak=do_polyak, fused_opt=fused,
                                before_adam=hook if delay == 0 else None)
-        n += 2 if self.fused_opt else 3
+        n += 2 if fused else 3
         for j in range(delay):
             ag.enqueue_actor_step(self.args_pi[j], polyak=ag.td3 and do_polyak and j == delay - 1,
-                                  fused_opt=self.fused_opt,
+                                  fused_opt=fused,
                                   before_adam=hook if (j == delay - 1 and not ag.autotune) else None)
-            n += (5 if ag.hps.clip_norm > 0 else (2 if self.fused_opt else 3)) + (1 if ag.autotune else 0)
+            n += (5 if ag.hps.clip_norm > 0 else (2 if fused else 3)) + (1 if ag.autotune else 0)
         return n
 
     def _polyak_due(self) -> bool:
@@ -185,7 +186,7 @@ class LearnerEngine:
                 stage.publish_actions(ag._lib, n_obs, slot, ag._stream())
                 n += 2
             args_q = None
-            if n_new and self.fused_sample and not self.fused_opt:
+            if n_new and self.fused_sample and not ag.fuses_opt(self.fused_opt):
                 # the replay write rides in the critic step too (b2rl_update_args_t.new_rows): the kernel reads the pinned
                 # rows itself (UVA), no separate write launch
                 args_q = ag.update_args(self.rows, eps_out=self.noise_q, storage=rb.storage, idx_out=self.idx,
