@@ -98,6 +98,26 @@ typedef struct b2rl_hyper {
   uint64_t seed;               /* Philox key when noise/indices are drawn on the device */
 } b2rl_hyper_t;
 
+/* ---- per-agent hyperparameters -------------------------------------------------------------
+ * One 64-byte row per local agent of a launch, in device memory (row g = agent g, a local index like
+ * arena_agent_stride). A captured graph freezes every by-value argument, so values that may differ between
+ * stacked agents (a sweep) or change during training (population-based training) are read from this table
+ * instead: rewriting a row with a stream-ordered copy changes what the next replay computes, with no recapture.
+ * Where a struct or entry point takes `agent_hp`, NULL means its scalars as before; a table replaces exactly the
+ * scalars listed here and only where the scalar path reads them (the flags — targ_smoothing, seg.do_adam /
+ * do_polyak / clip, predict's mode — still decide whether a value is used). */
+typedef struct b2rl_agent_hp {
+  float lr[3];           /* Adam learning rate by the optimizer's counter: [B2RL_CTR_Q] critics (hps.qnets_lr),
+                            [B2RL_CTR_PI] actor (hps.actor_lr), [B2RL_CTR_ALPHA] temperature (hps.log_alpha_lr);
+                            replaces b2rl_seg_t.lr and the log_alpha_lr arguments */
+  float gamma, polyak;   /* agents/agent.py:228, :328-331 */
+  float td3_std, td3_c;  /* target smoothing (agents/agent.py:197-200) */
+  float targ_ent;        /* SAC target entropy (-A in the reference, agents/agent.py:134) */
+  float clip_norm;       /* used when seg.clip; +inf = this agent does not clip (min(1, inf / (norm + 1e-6)) is exactly 1) */
+  float explore_std;     /* TD3 behaviour noise (hps.actor_noise_std, nets.py:155-159) */
+  float reserved[6];
+} b2rl_agent_hp_t;
+
 /* Everything a fused update needs. Pointers are `dev`. Population stacking: agent g uses
  * base + g*<x>_agent_stride for every per-agent buffer (n_agents == 1 for a single learner). */
 typedef struct b2rl_update_args {
@@ -147,6 +167,10 @@ typedef struct b2rl_update_args {
   int64_t capacity;
   int32_t n_new;
   int32_t reserved2;
+  /* dev [n_agents] or NULL: per-agent gamma, td3_std / td3_c, targ_ent, explore_std (b2rl_actor_predict) and the
+   * temperature's learning rate (b2rl_alpha_update) in place of hp.* and the scalar arguments. Refused by the
+   * fused-optimizer entry points (b2rl_*_update_opt). */
+  const b2rl_agent_hp_t* agent_hp;
 } b2rl_update_args_t;
 
 #define B2RL_OUT_QF_LOSS 0
@@ -193,6 +217,9 @@ typedef struct b2rl_adam_args {
   int64_t shadow_src[3], shadow_dst[3];
   int32_t n_shadow;            /* 0..3 */
   int32_t reserved2;
+  /* dev [n_agents] or NULL: agent g steps with lr[seg.counter] (seg.lr is ignored), polyak and clip_norm of its row.
+   * b2rl_grad_sumsq and seg.clip are needed when ANY agent clips; an agent that does not gets clip_norm = +inf. */
+  const b2rl_agent_hp_t* agent_hp;
 } b2rl_adam_args_t;
 
 /* ---- entry points ---------------------------------------------------------------------- */
@@ -268,6 +295,8 @@ typedef struct b2rl_stack {
   int64_t alpha_stride;    /* floats between agents' log_alpha state blocks */
   int64_t counters_stride; /* uint64 between agents' counter blocks (8) */
   int64_t out_stride;      /* floats between agents' log blocks (8) */
+  const b2rl_agent_hp_t* agent_hp; /* dev [n_agents] or NULL: per-agent gamma (critic heads), td3_std / td3_c (policy head
+                                      with smoothing), targ_ent (b2rl_wide_alpha_grad) in place of the scalars */
 } b2rl_stack_t;
 
 /* Large-batch hidden layer on the tensor cores (tcgen05.mma kind::tf32, operands staged by TMA, accumulator in
@@ -400,6 +429,8 @@ int b2rl_wide_actor_head_bwd(const float* dqda0, const float* dqda1, const float
 int b2rl_wide_actor_scalars(const float* part_s, const float* part_du, int32_t P, int32_t M, int32_t out_dim, int32_t td3,
                             const float* log_alpha, float* G, int64_t off_b3, float* out, const b2rl_stack_t* stack, void* stream);
 int b2rl_wide_alpha_grad(const float* logp2, int32_t M, float targ_ent, float* alpha_state, const b2rl_stack_t* stack, void* stream);
+/* (b2rl_wide_q_head / b2rl_tc_linear_q read gamma, b2rl_wide_policy_head td3_std / td3_c when smoothing, and
+ * b2rl_wide_alpha_grad targ_ent from stack->agent_hp when it is set.) */
 
 /* Weight gradient of one layer on the tensor cores (tc_wgrad.cu): C[m][n] = sum_b A[b][m] * Bm[b][n] for m < MA, with A
  * [Bn][lda] (a_cols >= MA columns exist; 16-byte aligned rows) and Bm [Bn][256]; Ct, if not NULL, receives the transpose
@@ -452,14 +483,16 @@ int b2rl_actor_update_td3(const b2rl_update_args_t* a, void* stream);
  * be Polyak-only spans (e.g. TD3's actor target in an iteration without actor update). Gradient clipping and
  * data-parallel training need the gradients complete before the step: use the three-launch form there. The
  * 3xTF32 mirror is not written here: opt->lo must be NULL (B2RL_E_INVALID otherwise, before any launch), and a
- * learner that keeps a mirror uses the three-launch form. */
+ * learner that keeps a mirror uses the three-launch form. The same holds for per-agent hyperparameters: a->agent_hp
+ * and opt->agent_hp must be NULL. */
 int b2rl_critic_update_opt(const b2rl_update_args_t* a, const b2rl_adam_args_t* opt, void* stream);
 int b2rl_actor_update_opt(const b2rl_update_args_t* a, const b2rl_adam_args_t* opt, void* stream);
 
 /* Replaces the autotune tail of update_actor (agents/agent.py:295-303): second no-grad
  * get_action with the UPDATED actor and fresh noise (a->eps2), alpha_loss, its gradient, and the
  * scalar Adam step on log_alpha (lr = log_alpha_lr; 0 = gradient only, see b2rl_alpha_adam). Writes
- * out[ALPHA_LOSS], out[ALPHA]; bumps counters[ALPHA]. One launch. */
+ * out[ALPHA_LOSS], out[ALPHA]; bumps counters[ALPHA]. One launch. With a->agent_hp, agent g's target entropy is
+ * its row's targ_ent, and a positive log_alpha_lr means "step with the row's lr[B2RL_CTR_ALPHA]". */
 int b2rl_alpha_update(const b2rl_update_args_t* a, float log_alpha_lr, void* stream);
 
 /* Data-parallel variant of the temperature step: b2rl_alpha_update with log_alpha_lr == 0 only
@@ -468,6 +501,9 @@ int b2rl_alpha_update(const b2rl_update_args_t* a, float log_alpha_lr, void* str
  * g = grad_scale * state[1] (grad_scale = 1/world) and bumps counters[ALPHA]. */
 int b2rl_alpha_adam(float* log_alpha, uint64_t* counters, int32_t n_agents, float log_alpha_lr,
                     float grad_scale, float* out, void* stream);
+/* b2rl_alpha_adam with per-agent learning rates: agent g steps with hp[g].lr[B2RL_CTR_ALPHA] (hp: dev [n_agents]). */
+int b2rl_alpha_adam_hp(float* log_alpha, uint64_t* counters, int32_t n_agents, const b2rl_agent_hp_t* hp,
+                       float grad_scale, float* out, void* stream);
 
 /* Sum of squares of the gradient span [begin,end) of region 4, per agent, into sumsq[agent]
  * (first half of clip_grad_norm_, agents/agent.py:284-285). Deterministic two-stage reduction. */
@@ -494,7 +530,8 @@ int b2rl_bump_counter(uint64_t* counters, int32_t which, int32_t n_agents, void*
  *   (device-addressable): the kernel then is the host<->device copy.
  * Stacked agents (a->n_agents > 1; 0 or 1 = one learner): agent g reads its actor at a->arena + g * a->arena_agent_stride,
  *   its counters at a->counters + g * 8 (draw = UINT64_MAX), keys its noise on the global id a->agent_base + g, and
- *   obs / a->eps / actions_out are [n_agents][n][..], contiguous. Each agent's actions equal those of a single call for it. */
+ *   obs / a->eps / actions_out are [n_agents][n][..], contiguous. Each agent's actions equal those of a single call for it.
+ *   a->agent_hp: agent g's TD3 noise std in mode 1 is its row's explore_std (explore_std is then ignored). */
 int b2rl_actor_predict(const b2rl_update_args_t* a, const float* obs, int32_t n, int32_t mode,
                        float explore_std, uint64_t draw, float* actions_out, void* stream);
 

@@ -33,6 +33,13 @@ class Hyper(C.Structure):
                 ("seed", C.c_uint64)]
 
 
+class AgentHp(C.Structure):
+    """b2rl_agent_hp_t: one 64-byte row of per-agent hyperparameters (lr indexed by CTR_Q / CTR_PI / CTR_ALPHA)."""
+    _fields_ = [("lr", C.c_float * 3), ("gamma", C.c_float), ("polyak", C.c_float), ("td3_std", C.c_float),
+                ("td3_c", C.c_float), ("targ_ent", C.c_float), ("clip_norm", C.c_float), ("explore_std", C.c_float),
+                ("reserved", C.c_float * 6)]
+
+
 class UpdateArgs(C.Structure):
     _fields_ = [("hp", Hyper), ("fmt", RowFmt), ("actor", Net), ("critic", Net * 2),
                 ("batch", C.c_int32), ("n_agents", C.c_int32), ("agent_base", C.c_int32), ("reserved", C.c_int32),
@@ -44,7 +51,7 @@ class UpdateArgs(C.Structure):
                 ("out", C.c_void_p), ("dbg_targ_q", C.c_void_p), ("dbg_q", C.c_void_p),
                 ("storage", C.c_void_p), ("storage_agent_stride", C.c_int64), ("storage_size", C.c_int64),
                 ("idx_out", C.c_void_p), ("new_rows", C.c_void_p), ("capacity", C.c_int64), ("n_new", C.c_int32),
-                ("reserved2", C.c_int32)]
+                ("reserved2", C.c_int32), ("agent_hp", C.c_void_p)]
 
 
 class Seg(C.Structure):
@@ -58,7 +65,8 @@ class AdamArgs(C.Structure):
                 ("beta1", C.c_float), ("beta2", C.c_float), ("eps", C.c_float), ("reserved", C.c_int32),
                 ("region_stride", C.c_int64), ("arena_agent_stride", C.c_int64),
                 ("arena", C.c_void_p), ("counters", C.c_void_p), ("grad_sumsq", C.c_void_p), ("lo", C.c_void_p), ("lo_agent_stride", C.c_int64),
-                ("shadow_src", C.c_int64 * 3), ("shadow_dst", C.c_int64 * 3), ("n_shadow", C.c_int32), ("reserved2", C.c_int32)]
+                ("shadow_src", C.c_int64 * 3), ("shadow_dst", C.c_int64 * 3), ("n_shadow", C.c_int32), ("reserved2", C.c_int32),
+                ("agent_hp", C.c_void_p)]
 
 
 class WidePolicy(C.Structure):
@@ -88,7 +96,7 @@ class ColsumJob(C.Structure):
 class Stack(C.Structure):
     """b2rl_stack_t: agents stacked along the row dimension of the wide path (NULL = one learner)."""
     _fields_ = [("n_agents", C.c_int32), ("agent_base", C.c_int32), ("param_stride", C.c_int64), ("lo_stride", C.c_int64),
-                ("alpha_stride", C.c_int64), ("counters_stride", C.c_int64), ("out_stride", C.c_int64)]
+                ("alpha_stride", C.c_int64), ("counters_stride", C.c_int64), ("out_stride", C.c_int64), ("agent_hp", C.c_void_p)]
 
 
 _STK = C.POINTER(Stack)
@@ -146,6 +154,7 @@ SYMBOLS = {
     "b2rl_actor_update_opt": (C.c_int, [C.POINTER(UpdateArgs), C.POINTER(AdamArgs), C.c_void_p]),
     "b2rl_alpha_update": (C.c_int, [C.POINTER(UpdateArgs), C.c_float, C.c_void_p]),
     "b2rl_alpha_adam": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_float, C.c_float, C.c_void_p, C.c_void_p]),
+    "b2rl_alpha_adam_hp": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_float, C.c_void_p, C.c_void_p]),
     "b2rl_grad_sumsq": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int32,
                                   C.c_void_p, C.c_void_p, C.c_void_p]),
     "b2rl_adam_polyak_multi": (C.c_int, [C.POINTER(AdamArgs), C.c_void_p]),

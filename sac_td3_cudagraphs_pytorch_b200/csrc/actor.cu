@@ -230,7 +230,7 @@ struct AlphaSmem {
   // followed by the observation tile float4[RQ * O]
 };
 __host__ __device__ inline size_t alpha_smem_bytes(int ob_dim) {
-  return sizeof(AlphaSmem) + (size_t)RQ * ob_dim * sizeof(float4);
+  return sizeof(AlphaSmem) + (size_t)RQ * ob_dim * sizeof(float4) + 4 * sizeof(float);  // + {targ_ent, lr} behind the tile
 }
 
 __device__ __forceinline__ void adam_scalar(float* st /*{p,g,m,v}*/, float g, float lr, float t, float b1, float b2,
@@ -260,6 +260,7 @@ __global__ void __launch_bounds__(NT, 1) alpha_kernel(const __grid_constant__ b2
   const int O = A.fmt.ob_dim, AD = A.fmt.ac_dim, rs = A.fmt.row_stride, B = A.batch;
   const int nvalid = min(RT, B - b0);
   float4* X = reinterpret_cast<float4*>(smem_raw + sizeof(AlphaSmem));
+  float* hpv = reinterpret_cast<float*>(X + RQ * O);  // this agent's {targ_ent, lr} (common.cuh agent_hp)
   const uint32_t gid = (uint32_t)(A.agent_base + agent);
   const float* P = A.arena + (size_t)agent * A.arena_agent_stride;
   const float* rows = A.rows + (size_t)agent * A.rows_agent_stride;
@@ -268,8 +269,15 @@ __global__ void __launch_bounds__(NT, 1) alpha_kernel(const __grid_constant__ b2
   float* wsb = A.workspace + (size_t)agent * A.workspace_agent_stride;
   float* part = ws_carve(wsb, B, 0).part;
 
-  if (w == 0) stage_net(P, &A.actor, &M.ns, &M.n, G.c * CW);
-  else stage_tile(batch_row(rows, rs, b0, nvalid), nvalid, 0, O, X, O, t - 32, NT - 32);
+  if (w == 0) {
+    stage_net(P, &A.actor, &M.ns, &M.n, G.c * CW);
+    if (l == 0) {
+      hpv[0] = agent_hp(A.agent_hp, agent, HP_TARG_ENT, A.hp.targ_ent);
+      hpv[1] = agent_hp(A.agent_hp, agent, HP_LR + B2RL_CTR_ALPHA, lr);  // (lr > 0 decides whether to step at all)
+    }
+  } else {
+    stage_tile(batch_row(rows, rs, b0, nvalid), nvalid, 0, O, X, O, t - 32, NT - 32);
+  }
   const Net& act = M.n;
   cp_async_wait_all();
   __syncthreads();
@@ -293,7 +301,7 @@ __global__ void __launch_bounds__(NT, 1) alpha_kernel(const __grid_constant__ b2
   }
   __syncthreads();
   if (t == 0) {
-    const float te = A.hp.targ_ent;
+    const float te = hpv[0];
     float s = 0.f;
     for (int r = 0; r < nvalid; ++r) s += (-M.logpi[r] - te);  // sum_r (-logpi_r - targ_ent), agent.py:300
     part[(size_t)rb * PART_LEN + PART_SCAL + 2] = s;
@@ -314,7 +322,7 @@ __global__ void __launch_bounds__(NT, 1) alpha_kernel(const __grid_constant__ b2
       const float loss = alpha * (s / (float)B);
       if (lr > 0.f) {
         const uint64_t tstep = ctr[B2RL_CTR_ALPHA] + 1;
-        adam_scalar(st, loss, lr, (float)tstep, 0.9f, 0.999f, 1e-8f);
+        adam_scalar(st, loss, hpv[1], (float)tstep, 0.9f, 0.999f, 1e-8f);
         ctr[B2RL_CTR_ALPHA] = tstep;
       } else {
         st[1] = loss;  // data parallel: local gradient only; b2rl_alpha_adam finishes after the all-reduce
@@ -327,15 +335,16 @@ __global__ void __launch_bounds__(NT, 1) alpha_kernel(const __grid_constant__ b2
   }
 }
 
-__global__ void alpha_adam_kernel(float* log_alpha, uint64_t* counters, int n_agents, float lr, float grad_scale,
-                                  float* out) {
+// hp: per-agent learning rates (b2rl_alpha_adam_hp) or NULL (b2rl_alpha_adam: lr for every agent)
+__global__ void alpha_adam_kernel(float* log_alpha, uint64_t* counters, int n_agents, float lr, const b2rl_agent_hp_t* hp,
+                                  float grad_scale, float* out) {
   pdl_enter();
   const int a = blockIdx.x * blockDim.x + threadIdx.x;
   if (a >= n_agents) return;
   float* st = log_alpha + (size_t)a * 5;
   uint64_t* ctr = counters + (size_t)a * 8;
   const uint64_t tstep = ctr[B2RL_CTR_ALPHA] + 1;
-  adam_scalar(st, st[1] * grad_scale, lr, (float)tstep, 0.9f, 0.999f, 1e-8f);
+  adam_scalar(st, st[1] * grad_scale, agent_hp(hp, a, HP_LR + B2RL_CTR_ALPHA, lr), (float)tstep, 0.9f, 0.999f, 1e-8f);
   ctr[B2RL_CTR_ALPHA] = tstep;
   if (out) {
     out[(size_t)a * 8 + B2RL_OUT_ALPHA_LOSS] = st[1];
@@ -343,9 +352,10 @@ __global__ void alpha_adam_kernel(float* log_alpha, uint64_t* counters, int n_ag
   }
 }
 
-cudaError_t launch_alpha_adam(float* log_alpha, uint64_t* counters, int n_agents, float lr, float grad_scale,
-                              float* out, cudaStream_t st) {
-  return launch_k(alpha_adam_kernel, dim3((n_agents + 127) / 128), dim3(128), 1, 0, st, log_alpha, counters, n_agents, lr, grad_scale, out);
+cudaError_t launch_alpha_adam(float* log_alpha, uint64_t* counters, int n_agents, float lr, const b2rl_agent_hp_t* hp,
+                              float grad_scale, float* out, cudaStream_t st) {
+  return launch_k(alpha_adam_kernel, dim3((n_agents + 127) / 128), dim3(128), 1, 0, st, log_alpha, counters, n_agents, lr, hp,
+                  grad_scale, out);
 }
 
 // ---- inference policy ----------------------------------------------------------------------------
@@ -356,7 +366,7 @@ struct PredictSmem {
   // followed by the observation tile float4[RQ * O]
 };
 __host__ __device__ inline size_t predict_smem_bytes(int ob_dim) {
-  return sizeof(PredictSmem) + (size_t)RQ * ob_dim * sizeof(float4);
+  return sizeof(PredictSmem) + (size_t)RQ * ob_dim * sizeof(float4) + 4 * sizeof(float);  // + explore_std behind the tile
 }
 
 template <bool WIDE>
@@ -376,11 +386,16 @@ predict_kernel(const __grid_constant__ b2rl_update_args_t A, const float* __rest
   const int O = A.fmt.ob_dim, AD = A.fmt.ac_dim;
   const int nvalid = min(RT, n - b0);
   float4* X = reinterpret_cast<float4*>(smem_raw + sizeof(PredictSmem));
+  float* xstd = reinterpret_cast<float*>(X + RQ * O);  // this agent's explore_std (common.cuh agent_hp)
   const bool td3 = A.hp.td3 != 0;
   // stacked agents (grid y = local agent g; one learner: g = 0): g's actor, counters, observations, noise and actions
   const int g = blockIdx.y;
-  if (w == 0) stage_net(A.arena + (size_t)g * A.arena_agent_stride, &A.actor, &M.ns, &M.n, G.c * CW);
-  else stage_tile(batch_row(obs + (size_t)g * n * O, O, b0, nvalid), nvalid, 0, O, X, O, t - 32, NT - 32);
+  if (w == 0) {
+    stage_net(A.arena + (size_t)g * A.arena_agent_stride, &A.actor, &M.ns, &M.n, G.c * CW);
+    if (l == 0) *xstd = agent_hp(A.agent_hp, g, HP_EXPLORE, explore_std);
+  } else {
+    stage_tile(batch_row(obs + (size_t)g * n * O, O, b0, nvalid), nvalid, 0, O, X, O, t - 32, NT - 32);
+  }
   const Net& act = M.n;
   cp_async_wait_all();
   __syncthreads();
@@ -405,7 +420,7 @@ predict_kernel(const __grid_constant__ b2rl_update_args_t A, const float* __rest
       if (td3) {  // agents/nets.py:149-159
         float th;
         a = td3_action(u0, scale, bias, th);
-        if (mode == 1) a += noise_at(A.eps, e, ~A.hp.seed, b0 + r, l, step, agent, STREAM_ACTOR_EPS) * (scale * explore_std);
+        if (mode == 1) a += noise_at(A.eps, e, ~A.hp.seed, b0 + r, l, step, agent, STREAM_ACTOR_EPS) * (scale * *xstd);
       } else if (mode == 1) {  // sample
         const float z = noise_at(A.eps, e, ~A.hp.seed, b0 + r, l, step, agent, STREAM_ACTOR_EPS);  // key != learner's
         a = gauss_sample(u0, uref(S.u, r, AD + l), z, scale, bias).action;

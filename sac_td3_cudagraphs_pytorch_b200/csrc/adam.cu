@@ -28,6 +28,7 @@ __global__ void __launch_bounds__(256) adam_polyak_kernel(const __grid_constant_
   float* G = P + 4 * A.region_stride;
   const uint64_t* ctr = A.counters + (size_t)agent * 8;
   float* LO = A.lo ? A.lo + (size_t)agent * A.lo_agent_stride : nullptr;  // 3xTF32 mirror: lo parts of what is written here
+  const float polyak = agent_hp(A.agent_hp, agent, HP_POLYAK, A.polyak);
 
   __shared__ SegScalars sc[B2RL_MAX_SEG];
   if (threadIdx.x < A.n_seg) {
@@ -35,12 +36,12 @@ __global__ void __launch_bounds__(256) adam_polyak_kernel(const __grid_constant_
     SegScalars v = {0.f, 1.f, 1.f, 1.f, 0.f};
     if (s.do_adam) {
       const float t = (float)ctr[s.counter];  // step count AFTER this step's bump (>= 1)
-      v = adam_scalars(s.lr, A.beta1, A.beta2, t);
+      v = adam_scalars(agent_hp(A.agent_hp, agent, HP_LR + s.counter, s.lr), A.beta1, A.beta2, t);
       adam_finish(v, A.eps);
       v.gscale = s.grad_scale;
       if (s.clip) {  // clip_grad_norm_: g *= min(1, max_norm / (norm + 1e-6))
         const float norm = sqrtf(A.grad_sumsq[agent]) * s.grad_scale;
-        v.gscale *= fminf(1.0f, A.clip_norm / (norm + 1e-6f));
+        v.gscale *= fminf(1.0f, agent_hp(A.agent_hp, agent, HP_CLIP, A.clip_norm) / (norm + 1e-6f));
       }
     }
     sc[threadIdx.x] = v;
@@ -96,10 +97,10 @@ __global__ void __launch_bounds__(256) adam_polyak_kernel(const __grid_constant_
       }
     }
     if (dp) {
-      tg.x = polyak_elem(tg.x, p.x, A.polyak);
-      tg.y = polyak_elem(tg.y, p.y, A.polyak);
-      tg.z = polyak_elem(tg.z, p.z, A.polyak);
-      tg.w = polyak_elem(tg.w, p.w, A.polyak);
+      tg.x = polyak_elem(tg.x, p.x, polyak);
+      tg.y = polyak_elem(tg.y, p.y, polyak);
+      tg.z = polyak_elem(tg.z, p.z, polyak);
+      tg.w = polyak_elem(tg.w, p.w, polyak);
       *reinterpret_cast<float4*>(T + i) = tg;
       stage(4, tg);
       if (LO) {
@@ -165,10 +166,10 @@ __global__ void __launch_bounds__(256) adam_polyak_kernel(const __grid_constant_
       }
       if (s.do_polyak) {
         float4 tg = *reinterpret_cast<const float4*>(T + i);
-        tg.x = polyak_elem(tg.x, p.x, A.polyak);
-        tg.y = polyak_elem(tg.y, p.y, A.polyak);
-        tg.z = polyak_elem(tg.z, p.z, A.polyak);
-        tg.w = polyak_elem(tg.w, p.w, A.polyak);
+        tg.x = polyak_elem(tg.x, p.x, polyak);
+        tg.y = polyak_elem(tg.y, p.y, polyak);
+        tg.z = polyak_elem(tg.z, p.z, polyak);
+        tg.w = polyak_elem(tg.w, p.w, polyak);
         *reinterpret_cast<float4*>(T + i) = tg;
         if (LO) *reinterpret_cast<float4*>(LO + A.region_stride + i) = tf32_lo4(tg);
       }

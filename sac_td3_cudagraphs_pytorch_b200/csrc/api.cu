@@ -11,7 +11,7 @@ namespace b2rl {
 cudaError_t launch_critic_fused(const b2rl_update_args_t&, cudaStream_t);
 cudaError_t launch_actor_fused(const b2rl_update_args_t&, cudaStream_t);
 cudaError_t launch_alpha(const b2rl_update_args_t&, float, cudaStream_t);
-cudaError_t launch_alpha_adam(float*, uint64_t*, int, float, float, float*, cudaStream_t);
+cudaError_t launch_alpha_adam(float*, uint64_t*, int, float, const b2rl_agent_hp_t*, float, float*, cudaStream_t);
 cudaError_t launch_predict(const b2rl_update_args_t&, const float*, int, int, float, uint64_t, float*, cudaStream_t);
 cudaError_t launch_wgrad(const b2rl_update_args_t&, int, int, const b2rl_adam_args_t*, cudaStream_t, int skip_vec = 0);
 cudaError_t launch_adam(const b2rl_adam_args_t&, cudaStream_t);
@@ -86,6 +86,11 @@ static int check_launch(cudaError_t e, const char* what) {
   return fail(B2RL_E_LAUNCH, "%s: %s", what, cudaGetErrorString(e));
 }
 static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
+// a per-agent hyperparameter table (NULL = the scalars): float-aligned device rows
+static int check_hp(const b2rl_agent_hp_t* hp, const char* what) {
+  if (hp && (reinterpret_cast<uintptr_t>(hp) & 3u)) return fail(B2RL_E_INVALID, "%s: agent_hp must be 4-byte aligned", what);
+  return B2RL_OK;
+}
 // the stacked-agents descriptor of the wide path (NULL = one learner)
 static int check_stack(const b2rl_stack_t* s, const char* what) {
   if (!s) return B2RL_OK;
@@ -94,7 +99,7 @@ static int check_stack(const b2rl_stack_t* s, const char* what) {
   if (s->param_stride < 0 || s->lo_stride < 0 || s->alpha_stride < 0 || s->counters_stride < 0 || s->out_stride < 0 ||
       (s->param_stride & 3) || (s->lo_stride & 3))
     return fail(B2RL_E_INVALID, "%s: stack strides must be >= 0 (param / lo strides multiples of 4 floats)", what);
-  return B2RL_OK;
+  return check_hp(s->agent_hp, what);
 }
 using b2rl::make_stk;
 
@@ -133,6 +138,7 @@ static int check_update(const b2rl_update_args_t* a, bool actor_step) {
       (a->workspace_agent_stride & 3))
     return fail(B2RL_E_INVALID, "arena/workspace must be 16-byte aligned with strides that are multiples of 4 floats");
   if (!a->hp.td3 && !a->log_alpha) return fail(B2RL_E_INVALID, "SAC needs log_alpha");
+  if (int rc = check_hp(a->agent_hp, "update args")) return rc;
   if (int rc = check_net(a->actor, "actor", actor_step)) return rc;
   if (int rc = check_net(a->critic[0], "critic[0]", true)) return rc;
   if (int rc = check_net(a->critic[1], "critic[1]", true)) return rc;
@@ -423,6 +429,8 @@ static int check_opt(const b2rl_update_args_t* a, const b2rl_adam_args_t* o, int
   if (o->n_seg < 1 || o->n_seg > B2RL_MAX_SEG) return fail(B2RL_E_INVALID, "opt: n_seg %d out of range", o->n_seg);
   if (o->lo)  // (the weight-gradient kernel does not write the 3xTF32 mirror: it would go stale)
     return fail(B2RL_E_INVALID, "opt: the fused optimizer does not keep a lo mirror current; use the three-launch form");
+  if (a->agent_hp || o->agent_hp)  // (the weight-gradient kernel takes its optimizer scalars from opt alone)
+    return fail(B2RL_E_INVALID, "opt: the fused optimizer takes no per-agent hyperparameter table; use the three-launch form");
   const b2rl_seg_t& s0 = o->seg[0];
   if (!s0.do_adam || s0.clip || s0.grad_scale != 1.0f || s0.begin != begin || s0.end != end || s0.counter != counter)
     return fail(B2RL_E_INVALID, "opt: seg[0] must be an unclipped, unscaled Adam segment over the trained nets");
@@ -474,9 +482,17 @@ int b2rl_alpha_adam(float* log_alpha, uint64_t* counters, int32_t n_agents, floa
                     float* out, void* stream) {
   if (!log_alpha || !counters || n_agents < 1 || !(log_alpha_lr > 0.f))
     return fail(B2RL_E_INVALID, "alpha_adam: bad arguments");
-  return check_launch(b2rl::launch_alpha_adam(log_alpha, counters, n_agents, log_alpha_lr, grad_scale, out,
+  return check_launch(b2rl::launch_alpha_adam(log_alpha, counters, n_agents, log_alpha_lr, nullptr, grad_scale, out,
                                               (cudaStream_t)stream),
                       "alpha_adam");
+}
+
+int b2rl_alpha_adam_hp(float* log_alpha, uint64_t* counters, int32_t n_agents, const b2rl_agent_hp_t* hp, float grad_scale,
+                       float* out, void* stream) {
+  if (!log_alpha || !counters || n_agents < 1 || !hp) return fail(B2RL_E_INVALID, "alpha_adam_hp: bad arguments");
+  if (int rc = check_hp(hp, "alpha_adam_hp")) return rc;
+  return check_launch(b2rl::launch_alpha_adam(log_alpha, counters, n_agents, 0.f, hp, grad_scale, out, (cudaStream_t)stream),
+                      "alpha_adam_hp");
 }
 
 int b2rl_grad_sumsq(const float* arena, int64_t region_stride, int64_t arena_agent_stride, int64_t begin, int64_t end,
@@ -497,6 +513,7 @@ int b2rl_adam_polyak_multi(const b2rl_adam_args_t* a, void* stream) {
   if (a->lo && (!aligned16(a->lo) || (a->lo_agent_stride & 3) || a->lo_agent_stride < 2 * a->region_stride))
     return fail(B2RL_E_INVALID, "adam: the lo mirror must be 16-byte aligned, its agent stride >= 2 regions and a multiple of 4 floats");
   if (a->n_shadow < 0 || a->n_shadow > 3) return fail(B2RL_E_INVALID, "adam: n_shadow %d out of range", a->n_shadow);
+  if (int rc = check_hp(a->agent_hp, "adam")) return rc;
   for (int q = 0; q < a->n_shadow; ++q) {
     const int64_t src = a->shadow_src[q], dst = a->shadow_dst[q], n = (int64_t)B2RL_HID * B2RL_HID;
     if (src < 0 || dst < 0 || (src & 3) || (dst & 3) || src + n > a->region_stride || dst + n > a->region_stride ||
@@ -515,6 +532,8 @@ int b2rl_adam_polyak_multi(const b2rl_adam_args_t* a, void* stream) {
       return fail(B2RL_E_INVALID, "adam: segment %d [%lld,%lld) must be 4-float aligned inside a region", i,
                   (long long)s.begin, (long long)s.end);
     if (s.do_adam && (s.counter < 0 || s.counter > 3)) return fail(B2RL_E_INVALID, "adam: segment %d bad counter", i);
+    if (s.do_adam && a->agent_hp && s.counter > B2RL_CTR_ALPHA)  // (the table has a learning rate for counters 0..2)
+      return fail(B2RL_E_INVALID, "adam: segment %d: with agent_hp the counter must be Q, PI or ALPHA", i);
     if (s.do_adam && s.clip && !a->grad_sumsq) return fail(B2RL_E_INVALID, "adam: clip needs grad_sumsq");
   }
   return check_launch(b2rl::launch_adam(*a, (cudaStream_t)stream), "adam_polyak_multi");
@@ -532,6 +551,7 @@ int b2rl_actor_predict(const b2rl_update_args_t* a, const float* obs, int32_t n,
   if (int rc = check_net(a->actor, "actor", false)) return rc;
   if (!a->arena || !a->min_ac || !a->max_ac) return fail(B2RL_E_INVALID, "predict: null device pointer");
   if (mode != 0 && mode != 1) return fail(B2RL_E_INVALID, "predict: mode must be 0 or 1");
+  if (int rc = check_hp(a->agent_hp, "predict")) return rc;
   if (a->n_agents < 0 || a->n_agents > 65535) return fail(B2RL_E_INVALID, "predict: n_agents %d out of range", a->n_agents);
   if (a->n_agents > 1 && (a->agent_base < 0 || (int64_t)a->agent_base + a->n_agents > (1 << 30) || a->arena_agent_stride < 1 ||
                           (a->arena_agent_stride & 3)))

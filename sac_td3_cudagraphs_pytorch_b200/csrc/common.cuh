@@ -1,6 +1,7 @@
 // common.cuh — shared device helpers for libb2rl (sm_100a).
 #pragma once
 #include <cuda_runtime.h>
+#include <stddef.h>
 #include <stdint.h>
 
 #include "../../include/b2rl.h"
@@ -111,15 +112,31 @@ inline cudaError_t launch_cluster(void (*kernel)(KArgs...), dim3 grid, int clust
   return launch_k(kernel, grid, dim3(NT), cluster_x, smem, st, static_cast<Args&&>(args)...);
 }
 
+// ---- per-agent hyperparameters (include/b2rl.h b2rl_agent_hp_t): float index of each field in a row
+enum AgentHpField { HP_LR = 0 /* + B2RL_CTR_* */, HP_GAMMA = 3, HP_POLYAK, HP_TD3_STD, HP_TD3_C, HP_TARG_ENT, HP_CLIP, HP_EXPLORE };
+static_assert(sizeof(b2rl_agent_hp_t) == 64, "one 64-byte row per agent");
+static_assert(offsetof(b2rl_agent_hp_t, gamma) == 4 * HP_GAMMA && offsetof(b2rl_agent_hp_t, polyak) == 4 * HP_POLYAK &&
+                  offsetof(b2rl_agent_hp_t, td3_std) == 4 * HP_TD3_STD && offsetof(b2rl_agent_hp_t, td3_c) == 4 * HP_TD3_C &&
+                  offsetof(b2rl_agent_hp_t, targ_ent) == 4 * HP_TARG_ENT && offsetof(b2rl_agent_hp_t, clip_norm) == 4 * HP_CLIP &&
+                  offsetof(b2rl_agent_hp_t, explore_std) == 4 * HP_EXPLORE,
+              "AgentHpField follows b2rl_agent_hp_t");
+// Agent g's value of one hyperparameter: row g of the launch's table, or — no table — the scalar the launch was given.
+// Every kernel that reads a swept value goes through here, once per CTA and ahead of its dependent chain.
+__device__ __forceinline__ float agent_hp(const b2rl_agent_hp_t* tab, int g, int field, float scalar) {
+  return tab ? __ldg(reinterpret_cast<const float*>(tab + g) + field) : scalar;
+}
+
 // stacked agents on the wide path (include/b2rl.h b2rl_stack_t): the device-side copy, n = 1 and zero strides when NULL
 struct Stk {
   int n;
   unsigned base;
   long long ps, ls, as, cs, os;  // param / lo / alpha / counters / out strides
+  const b2rl_agent_hp_t* hp;     // per-agent hyperparameters or NULL
 };
 inline Stk make_stk(const b2rl_stack_t* s) {
-  Stk k = {1, 0u, 0, 0, 0, 0, 0};
-  if (s) k = {s->n_agents, (unsigned)s->agent_base, s->param_stride, s->lo_stride, s->alpha_stride, s->counters_stride, s->out_stride};
+  Stk k = {1, 0u, 0, 0, 0, 0, 0, nullptr};
+  if (s) k = {s->n_agents, (unsigned)s->agent_base, s->param_stride, s->lo_stride, s->alpha_stride, s->counters_stride, s->out_stride,
+              s->agent_hp};
   return k;
 }
 

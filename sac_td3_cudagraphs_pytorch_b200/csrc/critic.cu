@@ -24,11 +24,13 @@ struct CriticSmem {
   float lo[MAX_A], hi[MAX_A], eps[RT][MAX_A];
   float rd[RT][2];             // (reward, done) of the 8 rows
   float logpi[RT], qn[2][RT], y[RT], dq[RT], sq[RT];  // per-row scalars
-  // followed by two input tiles float4[RQ * (O + A)]: [next_obs | a'] and [obs | act]
+  // followed by two input tiles float4[RQ * (O + A)]: [next_obs | a'] and [obs | act], then CriticVals
 };
+// this agent's values (common.cuh agent_hp), behind the tiles so that the tiles keep their offset
+struct CriticVals { float gamma, td3_std, td3_c, pad; };
 
 __host__ __device__ inline size_t critic_smem_bytes(int in_dim) {
-  return sizeof(CriticSmem) + (size_t)2 * RQ * in_dim * sizeof(float4);
+  return sizeof(CriticSmem) + (size_t)2 * RQ * in_dim * sizeof(float4) + sizeof(CriticVals);
 }
 
 template <bool WIDE>
@@ -48,6 +50,7 @@ __global__ void __launch_bounds__(NT, 1) critic_fused_kernel(const __grid_consta
   const int ldx = O + AD, nvalid = min(RT, B - b0);
   float4* XA = reinterpret_cast<float4*>(smem_raw + sizeof(CriticSmem));  // [next_obs | a']
   float4* XB = XA + RQ * ldx;                                             // [obs | act]
+  CriticVals& V = *reinterpret_cast<CriticVals*>(XB + RQ * ldx);
   const uint32_t gid = (uint32_t)(A.agent_base + agent);  // global agent id: keys the Philox streams
   const bool td3 = A.hp.td3 != 0;
 
@@ -67,6 +70,11 @@ __global__ void __launch_bounds__(NT, 1) critic_fused_kernel(const __grid_consta
     if (l < AD) {
       M.lo[l] = __ldg(A.min_ac + l);
       M.hi[l] = __ldg(A.max_ac + l);
+    }
+    if (l == 0) {
+      V.gamma = agent_hp(A.agent_hp, agent, HP_GAMMA, A.hp.gamma);
+      V.td3_std = agent_hp(A.agent_hp, agent, HP_TD3_STD, A.hp.td3_std);
+      V.td3_c = agent_hp(A.agent_hp, agent, HP_TD3_C, A.hp.td3_c);
     }
     tile_noise<RT, MAX_A>(M.eps, A.eps, rank == 0 ? A.eps_out : nullptr, A.hp.seed, (int64_t)agent * B + b0, b0, nvalid, AD, step, gid,
                           STREAM_CRITIC_EPS, !td3 || A.hp.targ_smoothing, l);
@@ -150,8 +158,8 @@ __global__ void __launch_bounds__(NT, 1) critic_fused_kernel(const __grid_consta
         float th;
         act_v = td3_action(u0, scale, bias, th);
         if (A.hp.targ_smoothing) {
-          float n = __fmul_rn(z, A.hp.td3_std);
-          n = fminf(fmaxf(n, -A.hp.td3_c), A.hp.td3_c);
+          float n = __fmul_rn(z, V.td3_std);
+          n = fminf(fmaxf(n, -V.td3_c), V.td3_c);
           act_v = fminf(fmaxf(__fadd_rn(act_v, n), lo), hi);
         }
       } else {
@@ -193,7 +201,7 @@ __global__ void __launch_bounds__(NT, 1) critic_fused_kernel(const __grid_consta
       qp = __fsub_rn(qp, __fmul_rn(alpha, M.logpi[r]));
     }
     const float rew = M.rd[r][0], done = M.rd[r][1];
-    const float y = __fadd_rn(rew, __fmul_rn(__fmul_rn(1.0f - done, A.hp.gamma), qp));
+    const float y = __fadd_rn(rew, __fmul_rn(__fmul_rn(1.0f - done, V.gamma), qp));
     M.y[r] = y;
     if (A.dbg_targ_q && rank == 0 && r < nvalid) A.dbg_targ_q[(size_t)agent * B + b0 + r] = y;
   }

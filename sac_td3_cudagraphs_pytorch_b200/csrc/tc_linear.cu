@@ -80,7 +80,8 @@ struct __align__(1024) TcSmemT {
   // fills with the x-hat chunks the LayerNorm backward reads (and the staging tile of the chunk being worked on)
   alignas(1024) float tile[EPW][NXB][32 * 32];  // (TMA reads and writes them: the 128-byte swizzle follows absolute address bits)
   alignas(16) float cvec[4][HID];  // bias, gamma, beta, and (fused critic head) w3
-  float wpart[MODE == 2 ? 4 : 1][MODE == 2 ? 3 : 4][HID];  // (forward: only the second vector set lives here, 4 KB)
+  alignas(16) float wpart[MODE == 2 ? 4 : 1][MODE == 2 ? 3 : 4][HID];  // (forward: only the second vector set lives here, 4 KB)
+  float qgamma[2];  // fused critic head: the discount of each vector set's agent (fetched with the vectors)
   float4 xch[EPW == 8 ? 2 * 2 * TCM : 1];  // [slot][half][row]: what the two column halves of a row swap (paired epilogue warps)
 };
 
@@ -451,6 +452,10 @@ tc_linear_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
           *reinterpret_cast<float4*>(dst) = make_float4(c, c, c, c);
         }
       }
+      if (head && et == 0) {  // the TD target's discount: agent_hp's choice, fetched like the vectors
+        if (K.hp) asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(s32(&S.qgamma[set])), "l"(&K.hp[ag].gamma) : "memory");
+        else S.qgamma[set] = Q.gamma;  // (no table: the scalar, as common.cuh agent_hp would return)
+      }
       asm volatile("cp.async.commit_group;" ::: "memory");
     };
     float v[32];
@@ -604,7 +609,7 @@ tc_linear_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
               float qp = Q.bcq_mix ? __fadd_rn(__fmul_rn(0.75f, qmin), __fmul_rn(0.25f, fmaxf(q0, q1))) : qmin;
               if (!Q.td3) qp = __fsub_rn(qp, __fmul_rn(expf(Q.log_alpha[(size_t)ag * K.as]), Q.logp[grow]));
               const float* rr = Q.rows + grow * Q.row_stride + Q.rd_off;
-              const float y = __fadd_rn(rr[0], __fmul_rn(__fmul_rn(1.0f - rr[1], Q.gamma), qp));
+              const float y = __fadd_rn(rr[0], __fmul_rn(__fmul_rn(1.0f - rr[1], S.qgamma[cset]), qp));
               if (Q.targ_out) Q.targ_out[grow] = y;
               const float dlt = q - y;
               dqv = dlt * (2.0f / (float)Q.M);

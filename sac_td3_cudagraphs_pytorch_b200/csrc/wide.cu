@@ -140,7 +140,8 @@ constexpr int WP_ROWS = 64;  // rows per CTA (8 per warp): the head's weights ar
 // transcendental part (Philox, Box-Muller, 2 tanh, exp, 2 log, a division: ~450 instructions) now runs once per 32
 // (row, dimension) pairs instead of once per row with 3 lanes alive: the one-phase version issued 669 warp instructions
 // per row and was issue-bound (74 % issue-slot utilisation, 1.5 TB/s of its 6.5: profiles/r2_ncu_full_pop256_summary.csv).
-__global__ void __launch_bounds__(256) wide_policy_head_kernel(const __grid_constant__ WidePolicyArgs P, const Stk K) {
+// (min 5 CTAs per SM: without it, the per-agent smoothing values pushed ptxas from 48 to 64 registers, 4 CTAs per SM)
+__global__ void __launch_bounds__(256, 5) wide_policy_head_kernel(const __grid_constant__ WidePolicyArgs P, const Stk K) {
   extern __shared__ float w3s[];            // [out][256], then us [64][out] head outputs, then lps [64][A] log-prob terms
   float* us = w3s + P.out_dim * HID;
   float* lps = us + WP_ROWS * P.out_dim;
@@ -208,6 +209,10 @@ __global__ void __launch_bounds__(256) wide_policy_head_kernel(const __grid_cons
   __syncthreads();
   const uint32_t agent = P.agent + (uint32_t)ag;
   const uint64_t step = P.counters[ag * K.cs + P.counter_idx];
+  // this agent's target smoothing, loaded beside `step`; the actor and temperature steps run the head without smoothing
+  const bool smooth = P.td3 && P.smoothing;
+  const float td3_std = smooth ? agent_hp(K.hp, (int)ag, HP_TD3_STD, P.td3_std) : 0.f;
+  const float td3_c = smooth ? agent_hp(K.hp, (int)ag, HP_TD3_C, P.td3_c) : 0.f;
   for (int i = t; i < nrows * P.A; i += 256) {
     const int rr = i / P.A, a = i - rr * P.A;
     const int row = row0 + rr;                  // row inside the agent's batch: the Philox key
@@ -224,8 +229,8 @@ __global__ void __launch_bounds__(256) wide_policy_head_kernel(const __grid_cons
       if (P.smoothing) {
         const float z = noise_at(P.eps, e, P.seed, row, a, step, agent, P.stream_id);
         if (P.eps_out) P.eps_out[e] = z;
-        float n = __fmul_rn(z, P.td3_std);
-        n = fminf(fmaxf(n, -P.td3_c), P.td3_c);
+        float n = __fmul_rn(z, td3_std);
+        n = fminf(fmaxf(n, -td3_c), td3_c);
         act_v = fminf(fmaxf(__fadd_rn(act_v, n), lo), hi);
       }
     } else {
@@ -262,6 +267,7 @@ __global__ void __launch_bounds__(256) wide_q_head_kernel(const __grid_constant_
   const int lrow = blockIdx.x * 8 + w;
   const size_t row = ag * Q.M + lrow;
   const float* w3 = Q.w3 + ag * K.ps;
+  const float gamma = agent_hp(K.hp, (int)ag, HP_GAMMA, Q.gamma);
   float sq = 0.f, dqv = 0.f;
   if (lrow < Q.M) {
     float s = 0.f;
@@ -276,7 +282,7 @@ __global__ void __launch_bounds__(256) wide_q_head_kernel(const __grid_constant_
         float qp = Q.bcq_mix ? __fadd_rn(__fmul_rn(0.75f, qmin), __fmul_rn(0.25f, fmaxf(q0, q1))) : qmin;
         if (!Q.td3) qp = __fsub_rn(qp, __fmul_rn(expf(Q.log_alpha[ag * K.as]), Q.logp[row]));
         const float* rr = Q.rows + row * Q.row_stride + Q.rd_off;
-        const float y = __fadd_rn(rr[0], __fmul_rn(__fmul_rn(1.0f - rr[1], Q.gamma), qp));
+        const float y = __fadd_rn(rr[0], __fmul_rn(__fmul_rn(1.0f - rr[1], gamma), qp));
         if (Q.targ_out) Q.targ_out[row] = y;
         const float dlt = q - y;
         dqv = dlt * (2.0f / (float)Q.M);
@@ -634,7 +640,9 @@ wide_actor_scalars_kernel(const float* __restrict__ part_s, const float* __restr
 
 // temperature gradient (agents/agent.py:295-303): log_alpha state slot 1 <- alpha * mean(-logpi'' - targ_ent); one CTA
 __global__ void __launch_bounds__(256)
-wide_alpha_grad_kernel(const float* __restrict__ logp2, int M, float targ_ent, float* __restrict__ alpha_state, long long as) {
+wide_alpha_grad_kernel(const float* __restrict__ logp2, int M, float targ_ent_arg, float* __restrict__ alpha_state, long long as,
+                       const b2rl_agent_hp_t* __restrict__ hp) {
+  const float targ_ent = agent_hp(hp, blockIdx.x, HP_TARG_ENT, targ_ent_arg);
   logp2 += (size_t)blockIdx.x * M, alpha_state += (size_t)blockIdx.x * as;  // stacked agents: blockIdx.x = agent
   __shared__ float red[256];
   const int t = threadIdx.x;
@@ -734,7 +742,7 @@ cudaError_t launch_wide_actor_scalars(const float* part_s, const float* part_du,
   return cudaGetLastError();
 }
 cudaError_t launch_wide_alpha_grad(const float* logp2, int M, float targ_ent, float* alpha_state, const Stk& k, cudaStream_t st) {
-  wide_alpha_grad_kernel<<<k.n, 256, 0, st>>>(logp2, M, targ_ent, alpha_state, k.as);
+  wide_alpha_grad_kernel<<<k.n, 256, 0, st>>>(logp2, M, targ_ent, alpha_state, k.as, k.hp);
   return cudaGetLastError();
 }
 

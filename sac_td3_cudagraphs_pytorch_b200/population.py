@@ -13,6 +13,10 @@ runs N seeds at once: `predict` (the stacked behaviour policy) and `extend` (eve
 slice) are the eager collection path before learning starts; `step_async` / `wait` / `wait_actions` run policy, replay
 write, iteration and the log block as ONE graph replay per step, like LearnerEngine.step_async for one learner
 (tests/test_gpu_population_step.py).
+
+Members may differ in their hyperparameters (a sweep, `agent_hps`), and these may change during training
+(population-based training: `set_agent_hps`, `exploit`). The kernels read them from a per-agent table in device memory
+(include/b2rl.h b2rl_agent_hp_t), so a changed value reaches the next graph replay without a recapture.
 """
 from __future__ import annotations
 
@@ -25,6 +29,7 @@ import torch
 
 from . import _lib as L
 from .agents.agent import HID_DIMS
+from .hps import hp_get
 from .agents.nets import Actor, Critic, TanhGaussActor
 from .arena import Arena, make_layout, set_shadow_pairs
 from .replay import pack_rows, row_format
@@ -36,6 +41,86 @@ def shard(n_total: int, world: int, rank: int) -> range:
     q, r = divmod(n_total, world)
     lo = rank * q + min(rank, r)
     return range(lo, lo + q + (1 if rank < r else 0))
+
+
+# the hyperparameters that may differ between the members of one population: all of them are read by the kernels from the
+# per-agent table (alpha_init only sets the initial log alpha on the host). Everything else changes launch shapes or which
+# graph variant runs, and is the same for every member.
+SWEEPABLE = ("qnets_lr", "actor_lr", "log_alpha_lr", "gamma", "polyak", "td3_std", "td3_c", "clip_norm", "actor_noise_std",
+             "alpha_init", "targ_ent")
+_ABSENT = {"log_alpha_lr": 0.0, "alpha_init": 1.0, "td3_std": 0.0, "td3_c": 0.0, "actor_noise_std": 0.0, "clip_norm": 0.0}
+
+
+def _check_hp_value(key: str, v, wide: bool) -> float:
+    try:
+        v = float(v)
+    except (TypeError, ValueError):
+        raise L.B2rlError(f"agent_hps: {key} = {v!r} is not a number") from None
+    if not math.isfinite(v):
+        raise L.B2rlError(f"agent_hps: {key} = {v} must be finite")
+    if key.endswith("_lr") and v < 0:
+        raise L.B2rlError(f"agent_hps: {key} = {v} must be >= 0")
+    if key == "gamma" and not 0 < v <= 1:
+        raise L.B2rlError(f"agent_hps: gamma = {v} must be in (0, 1]")
+    if key == "polyak" and not 0 <= v <= 1:
+        raise L.B2rlError(f"agent_hps: polyak = {v} must be in [0, 1]")
+    if key in ("td3_std", "td3_c", "actor_noise_std", "clip_norm") and v < 0:
+        raise L.B2rlError(f"agent_hps: {key} = {v} must be >= 0")
+    if key == "alpha_init" and not v > 0:
+        raise L.B2rlError(f"agent_hps: alpha_init = {v} must be > 0")
+    if key == "clip_norm" and v > 0 and wide:
+        raise L.B2rlError(f"agent_hps: clip_norm = {v}: the tensor-core (wide) actor step has no gradient clipping")
+    return v
+
+
+def agent_hp_values(hps, n: int, ac_dim: int, agent_hps=None, wide: bool = False) -> list:
+    """The effective sweepable values of each of n agents: `hps` (targ_ent defaults to -ac_dim), overridden by agent_hps —
+    a mapping {key: n values} or a sequence of n override mappings. Raises B2rlError on a key that may not differ
+    between agents (it sets launch shapes or graph variants), a wrong length or an out-of-range value."""
+    base = {k: hp_get(hps, k, _ABSENT.get(k)) for k in SWEEPABLE}
+    if base["targ_ent"] is None:
+        base["targ_ent"] = -float(ac_dim)
+    cols: dict = {}
+    if agent_hps is None:
+        pass
+    elif isinstance(agent_hps, Mapping):
+        for k, vs in agent_hps.items():
+            if isinstance(vs, (str, bytes)) or not hasattr(vs, "__len__") or len(vs) != n:
+                raise L.B2rlError(f"agent_hps[{k!r}]: expected a sequence of {n} values (one per agent), got {vs!r}")
+            cols[k] = list(vs)
+    else:
+        rows = list(agent_hps)
+        if len(rows) != n:
+            raise L.B2rlError(f"agent_hps: expected {n} override mappings (one per agent), got {len(rows)}")
+        for g, r in enumerate(rows):
+            for k, v in dict(r).items():
+                cols.setdefault(k, [base.get(k, hp_get(hps, k))] * n)[g] = v
+    for k, vs in cols.items():
+        if k not in SWEEPABLE and any(v != hp_get(hps, k) for v in vs):
+            raise L.B2rlError(f"agent_hps: {k!r} cannot differ between the agents of a population (it changes launch shapes "
+                              f"or graph variants); every agent uses hps.{k} = {hp_get(hps, k)!r}. Per-agent keys: "
+                              f"{', '.join(SWEEPABLE)}")
+    out = []
+    for g in range(n):
+        d = {k: _check_hp_value(k, cols[k][g] if k in cols else base[k], wide) for k in SWEEPABLE}
+        out.append(d)
+    return out
+
+
+def agent_hp_table(values: list, td3: bool) -> np.ndarray:
+    """The b2rl_agent_hp_t rows [n, 16] float32 of these effective values. An agent with clip_norm <= 0 does not clip:
+    +inf there makes its clip factor min(1, inf / (norm + 1e-6)) exactly 1 when another agent's clipping launches the
+    clipped optimizer step. SAC stores no TD3 noise (td3_std / td3_c / explore_std = 0), as the scalar path passes."""
+    t = np.zeros((len(values), C.sizeof(L.AgentHp) // 4), dtype=np.float32)
+    for g, v in enumerate(values):
+        r = L.AgentHp()
+        r.lr[L.CTR_Q], r.lr[L.CTR_PI], r.lr[L.CTR_ALPHA] = v["qnets_lr"], v["actor_lr"], v["log_alpha_lr"]
+        r.gamma, r.polyak, r.targ_ent = v["gamma"], v["polyak"], v["targ_ent"]
+        r.td3_std, r.td3_c = (v["td3_std"], v["td3_c"]) if td3 else (0.0, 0.0)
+        r.explore_std = v["actor_noise_std"] if td3 else 0.0
+        r.clip_norm = v["clip_norm"] if v["clip_norm"] > 0 else math.inf
+        t[g] = np.frombuffer(bytes(r), dtype=np.float32)
+    return t
 
 
 def init_agent_params(agent_id: int, seed: int, ob_dim: int, ac_dim: int, td3: bool, layer_norm: bool,
@@ -63,8 +148,10 @@ def init_agent_params(agent_id: int, seed: int, ob_dim: int, ac_dim: int, td3: b
 class Population:
     def __init__(self, agent_ids, ob_dim: int, ac_dim: int, min_ac, max_ac, hps, device, seed: int = 0,
                  rb_capacity: int = 100_000, batch_size: Optional[int] = None, use_graphs: bool = True,
-                 wide: Optional[str] = None):
-        """wide: None = the batch-256 row-group kernels with the agent in blockIdx.y (each agent's layers stream from L2
+                 wide: Optional[str] = None, agent_hps=None):
+        """agent_hps: per-agent values of the SWEEPABLE keys, as {key: N values} or N override mappings (None: every agent
+        uses hps). Agent g then trains exactly as a one-agent Population built with its values as plain hps.
+        wide: None = the batch-256 row-group kernels with the agent in blockIdx.y (each agent's layers stream from L2
         once per 8 rows: latency-optimal for ONE agent, ~10 TFLOP/s however many are stacked); "3xtf32" / "tf32" = the
         layer-by-layer tensor-core path (wide.py) with the agents stacked along the row dimension — n_agents x batch rows
         per launch, per-agent weights fetched by rank-3 TMA maps: what a population of hundreds of agents wants."""
@@ -89,10 +176,20 @@ class Population:
         self.arena = Arena(self.layout, self.device, n_agents=self.N)
         N, dev, lay = self.N, self.device, self.layout
         self.autotune = (not self.td3) and bool(hps.autotune)
+        self._hp = agent_hp_values(hps, N, self.ac_dim, agent_hps, wide=bool(wide))
+        # what the captured graphs fix: whether the clipped actor step runs (any agent clips) and whether the temperature
+        # takes an Adam step (log_alpha_lr > 0) or leaves its gradient only (0); set_agent_hps keeps both
+        self._clip = any(v["clip_norm"] > 0 for v in self._hp)
+        self._alpha_steps = any(v["log_alpha_lr"] > 0 for v in self._hp)
+        if self.autotune and self._alpha_steps != all(v["log_alpha_lr"] > 0 for v in self._hp):
+            raise L.B2rlError("agent_hps: log_alpha_lr = 0 (temperature gradient only) cannot be mixed with positive rates")
+        if self.autotune and wide and not self._alpha_steps:
+            raise L.B2rlError("agent_hps: the tensor-core (wide) temperature step needs log_alpha_lr > 0")
+        self.agent_hp_table = torch.from_numpy(agent_hp_table(self._hp, self.td3)).to(dev)
 
         for g, aid in enumerate(self.ids):
             a, q1, q2 = init_agent_params(aid, seed, ob_dim, ac_dim, self.td3, ln, self.min_ac.cpu(), self.max_ac.cpu(),
-                                          float(hps.actor_noise_std) if self.td3 else 0.1)
+                                          self._hp[g]["actor_noise_std"] if self.td3 else 0.1)
             for net, src in ((lay.actor, a), (lay.critic[0], q1), (lay.critic[1], q2)):
                 with torch.no_grad():
                     for name, view in self.arena.named(net, L.REGION_P, g).items():
@@ -105,7 +202,7 @@ class Population:
         self.out = torch.zeros(N, 8, dtype=torch.float32, device=dev)
         self.alpha_state = torch.zeros(N, 5, dtype=torch.float32, device=dev)
         if not self.td3:
-            self.alpha_state[:, 0] = math.log(hps.alpha_init)
+            self.alpha_state[:, 0] = torch.tensor([math.log(v["alpha_init"]) for v in self._hp], dtype=torch.float32)
         self.sumsq = torch.zeros(N, dtype=torch.float32, device=dev)
         self.sumsq_scratch = torch.zeros(N * 64, dtype=torch.float32, device=dev)
         ws = self._lib.b2rl_workspace_floats(self.B)
@@ -126,7 +223,9 @@ class Population:
             targ_smoothing=int(bool(hps.targ_actor_smoothing)) if self.td3 else 0, autotune=int(self.autotune),
             gamma=float(hps.gamma), td3_std=float(hps.td3_std) if self.td3 else 0.0,
             td3_c=float(hps.td3_c) if self.td3 else 0.0, targ_ent=float(-self.ac_dim), seed=self.seed)
-        self.args = self._make_args()
+        self.args = self._make_args()  # the scalars of hps (agent_hp NULL): what a caller of the fused-optimizer entry points passes
+        self._hp_args = L.UpdateArgs.from_buffer_copy(self.args)  # every launch of the population reads its table
+        self._hp_args.agent_hp = self.agent_hp_table.data_ptr()
         self._lo: Optional[torch.Tensor] = None
         self.wide = wide
         self.wide_q = self.wide_pi = None
@@ -196,12 +295,12 @@ class Population:
             raise L.B2rlError(f"predict: obs must be [{self.N}, n, {self.ob_dim}], got {tuple(obs.shape)}")
         n = obs.shape[1]
         act = torch.empty(self.N, n, self.ac_dim, dtype=torch.float32, device=self.device)
-        args = self.args
+        args = self._hp_args
         if eps is not None:
             eps = torch.as_tensor(eps).to(device=self.device, dtype=torch.float32).contiguous()
             if tuple(eps.shape) != (self.N, n, self.ac_dim):
                 raise L.B2rlError(f"predict: eps must be [{self.N}, {n}, {self.ac_dim}], got {tuple(eps.shape)}")
-            args = L.UpdateArgs.from_buffer_copy(self.args)
+            args = L.UpdateArgs.from_buffer_copy(self._hp_args)
             args.eps = eps.data_ptr()
         self._predict_draw += 1
         self._launch_predict(args, obs.data_ptr(), n, explore, self._predict_draw, act.data_ptr())
@@ -232,7 +331,8 @@ class Population:
         for i, s in enumerate(segs):
             a.seg[i] = s
         a.n_seg, a.n_agents = len(segs), self.N
-        a.polyak, a.clip_norm = float(self.hps.polyak), float(self.hps.clip_norm)
+        a.polyak, a.clip_norm = float(self.hps.polyak), float(self.hps.clip_norm)  # (the table's values are used)
+        a.agent_hp = self.agent_hp_table.data_ptr()
         a.beta1, a.beta2, a.eps = 0.9, 0.999, 1e-8
         a.region_stride, a.arena_agent_stride = self.layout.region, self.arena.agent_stride
         a.arena, a.counters, a.grad_sumsq = self.arena.flat.data_ptr(), self.counters.data_ptr(), self.sumsq.data_ptr()
@@ -269,13 +369,13 @@ class Population:
                 self.wide_pi.update_actor(self.rows, polyak=self.td3 and do_polyak and j == delay - 1)
             return -1
         fn = lib.b2rl_critic_update_td3 if self.td3 else lib.b2rl_critic_update_sac
-        L.check(fn(C.byref(self.args), st), "critic_update")
+        L.check(fn(C.byref(self._hp_args), st), "critic_update")
         self._adam([seg(lay.critic[0].begin, lay.critic[1].end, float(h.qnets_lr), True, do_polyak, L.CTR_Q)] + extra)
         n += 4
         for j in range(delay):
             fn = lib.b2rl_actor_update_td3 if self.td3 else lib.b2rl_actor_update_sac
-            L.check(fn(C.byref(self.args), st), "actor_update")
-            clip = h.clip_norm > 0
+            L.check(fn(C.byref(self._hp_args), st), "actor_update")
+            clip = self._clip  # any agent clips; the others have clip_norm = +inf in the table
             if clip:
                 L.check(lib.b2rl_grad_sumsq(self.arena.flat.data_ptr(), lay.region, self.arena.agent_stride,
                                             lay.actor.begin, lay.actor.core_end, self.N, self.sumsq.data_ptr(),
@@ -285,7 +385,7 @@ class Population:
                             self.td3 and do_polyak and j == delay - 1, L.CTR_PI, clip)])
             n += 3
             if self.autotune:
-                L.check(lib.b2rl_alpha_update(C.byref(self.args), float(h.log_alpha_lr), st), "alpha_update")
+                L.check(lib.b2rl_alpha_update(C.byref(self._hp_args), 1.0 if self._alpha_steps else 0.0, st), "alpha_update")
                 n += 1
         return n
 
@@ -372,7 +472,7 @@ class Population:
         with torch.cuda.graph(g):
             n = 0
             if n_obs:  # noise keyed on each agent's critic step counter (draw = UINT64_MAX), as in LearnerEngine's step
-                self._launch_predict(self.args, obs.data_ptr(), n_obs, explore, 2 ** 64 - 1, stage.device_actions(n_obs).data_ptr())
+                self._launch_predict(self._hp_args, obs.data_ptr(), n_obs, explore, 2 ** 64 - 1, stage.device_actions(n_obs).data_ptr())
                 stage.publish_actions(self._lib, n_obs, slot, self._stream())
                 n += 2
             if n_new:  # pinned host memory is device-addressable: the write kernel is the host->device copy
@@ -383,6 +483,63 @@ class Population:
         self.launches_per_variant[key] = -1 if m < 0 else n + m + 1
         self.graphs[key] = g
         return g
+
+    # ------------------------------------------------------------------ per-agent hyperparameters, population-based training
+    def agent_hps(self, g: int) -> dict:
+        """The effective values of the SWEEPABLE keys of local agent g (alpha_init: its initial value)."""
+        return dict(self._hp[g])
+
+    def _agents(self, agents) -> list:
+        gs = [agents] if isinstance(agents, int) else [int(g) for g in agents]
+        for g in gs:
+            if not 0 <= g < self.N:
+                raise L.B2rlError(f"agent {g} is not a local agent index in [0, {self.N})")
+        return gs
+
+    def set_agent_hps(self, agents, **values) -> None:
+        """Change per-agent hyperparameters of the local agents `agents` (an index or a sequence) during training: the
+        explore half of population-based training. The rows are written by a stream-ordered copy on the current stream,
+        so every iteration or step launched after this call uses the new values (steps already in flight keep the old
+        ones), and no graph is captured again. alpha_init is refused (use exploit or write alpha_state); so is a value
+        that would need another graph: clipping when no agent clipped at construction, or moving log_alpha_lr between 0
+        (gradient only) and positive."""
+        gs = self._agents(agents)
+        bad = [k for k in values if k not in SWEEPABLE or k == "alpha_init"]
+        if bad:
+            raise L.B2rlError(f"set_agent_hps: {bad[0]!r} cannot be changed per agent during training; keys: "
+                              f"{', '.join(k for k in SWEEPABLE if k != 'alpha_init')}")
+        new = [dict(self._hp[g], **{k: _check_hp_value(k, v, bool(self.wide)) for k, v in values.items()}) for g in gs]
+        for v in new:
+            if v["clip_norm"] > 0 and not self._clip:
+                raise L.B2rlError("set_agent_hps: clip_norm > 0 needs the clipped actor step, which this population's graphs "
+                                  "do not contain (no agent clipped at construction)")
+            if self.autotune and (v["log_alpha_lr"] > 0) != self._alpha_steps:
+                raise L.B2rlError("set_agent_hps: log_alpha_lr cannot move between 0 (gradient only) and positive rates")
+        rows = torch.from_numpy(agent_hp_table(new, self.td3)).pin_memory()
+        for i, g in enumerate(gs):
+            self.agent_hp_table[g].copy_(rows[i], non_blocking=True)
+            self._hp[g] = new[i]
+
+    def exploit(self, dst: int, src: int) -> None:
+        """The exploit half of population-based training: local agent dst takes over local agent src's learner state —
+        parameters, targets and Adam moments (the whole arena row, shadows included), the temperature state, the optimizer
+        step counters (CTR_Q / CTR_PI / CTR_ALPHA), the 3xTF32 mirror row if there is one and the hyperparameter row — by
+        stream-ordered device copies on the current stream. dst keeps its replay slice, its replay counters and its global
+        id (its own random streams). Between steps only, not inside a graph capture; follow with set_agent_hps(dst, ...)
+        to perturb."""
+        dst, src = self._agents([dst, src])
+        if dst == src:
+            raise L.B2rlError("exploit: dst and src are the same agent")
+        if torch.cuda.is_current_stream_capturing():
+            raise L.B2rlError("exploit: not legal inside a graph capture")
+        with torch.no_grad():
+            self.arena.flat[dst].copy_(self.arena.flat[src])
+            self.alpha_state[dst].copy_(self.alpha_state[src])
+            self.counters[dst, L.CTR_Q:L.CTR_ALPHA + 1].copy_(self.counters[src, L.CTR_Q:L.CTR_ALPHA + 1])
+            if self._lo is not None:
+                self._lo[dst].copy_(self._lo[src])
+            self.agent_hp_table[dst].copy_(self.agent_hp_table[src])
+        self._hp[dst] = dict(self._hp[src])
 
     # ------------------------------------------------------------------ inspection
     def agent_arena(self, g: int) -> torch.Tensor:

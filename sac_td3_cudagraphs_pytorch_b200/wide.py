@@ -52,9 +52,8 @@ class _Owner:
         """The ``b2rl_stack_t*`` argument (None for a single learner)."""
         if not self.stacked:
             return None
-        s = L.Stack(self.n, self.base, self.arena.agent_stride, lo_stride, self.alpha_state.stride(0), self.counters.stride(0),
-                    self.out.stride(0))
-        return s
+        return L.Stack(self.n, self.base, self.arena.agent_stride, lo_stride, self.alpha_state.stride(0), self.counters.stride(0),
+                       self.out.stride(0), self.owner.agent_hp_table.data_ptr())
 
     def workspace(self, M: int) -> torch.Tensor:
         """H1 H2 DZ1 DZ2 [2][n*M][256] + DZ3 [2][n*M][MAX_OUT], shared by the critic and the actor step."""
@@ -271,7 +270,8 @@ class WideActor:
     def __init__(self, agent, batch: int, precision: str = "3xtf32"):
         assert precision in ("3xtf32", "tf32")
         own = self.ag = agent if isinstance(agent, _Owner) else _Owner(agent)
-        assert not own.hps.clip_norm > 0, "the wide actor step has no gradient clipping: use the row-group path"
+        assert not (own.owner._clip if own.stacked else own.hps.clip_norm > 0), \
+            "the wide actor step has no gradient clipping: use the row-group path"
         self.x3 = precision == "3xtf32"
         self.M = int(batch)
         M, dev, n = self.M, own.device, own.n
@@ -409,8 +409,12 @@ class WideActor:
             return out
         if ag.autotune:
             self.alpha_grad(rows, eps_alpha)
-            L.check(lib.b2rl_alpha_adam(la, ag.counters.data_ptr(), ag.n, float(ag.hps.log_alpha_lr), 1.0, ag.out.data_ptr(), st),
-                    "alpha_adam")
+            if ag.stacked:  # the population's per-agent rates
+                L.check(lib.b2rl_alpha_adam_hp(la, ag.counters.data_ptr(), ag.n, ag.owner.agent_hp_table.data_ptr(), 1.0,
+                                               ag.out.data_ptr(), st), "alpha_adam_hp")
+            else:
+                L.check(lib.b2rl_alpha_adam(la, ag.counters.data_ptr(), ag.n, float(ag.hps.log_alpha_lr), 1.0, ag.out.data_ptr(), st),
+                        "alpha_adam")
             out["loss/alpha_loss"] = ag.out[..., L.OUT_ALPHA_LOSS]
         out["vitals/alpha"] = ag.out[..., L.OUT_ALPHA]
         return out
