@@ -84,6 +84,37 @@ class ArenaAdam:
         self._agent.arena.sync_shadows((L.REGION_M, L.REGION_V))
 
 
+def checkpoint_path(path, sfx: Optional[str], timesteps_so_far: int) -> Path:
+    """File name of a checkpoint in directory `path` (agents/agent.py:337-341)."""
+    fname = f"ckpt_{sfx}" if sfx is not None else f".ckpt_{timesteps_so_far}ts"
+    return Path(path) / f"{fname}.pth"
+
+
+def checkpoint_dict(hps, timesteps_so_far: int, actor, qnet1, qnet2, actor_optimizer: ArenaAdam, q_optimizer: ArenaAdam,
+                    actor_target: Mapping[str, torch.Tensor], qnet_target: Mapping[str, torch.Tensor],
+                    log_alpha: Optional[torch.Tensor] = None, alpha_optimizer: Optional[ArenaAdam] = None) -> dict:
+    """The dict Agent.save writes and Agent.load_from_disk reads: the reference's layout (agents/agent.py:343-352) plus
+    targets and temperature. actor / qnet1 / qnet2 are nets.py modules (their state_dicts), targets map the reference's
+    names to tensors ([2, ...] for the critics), log_alpha / alpha_optimizer are SAC's (the optimizer with autotune)."""
+    clone = lambda sd: {k: v.detach().clone().contiguous() for k, v in sd.items()}
+    ckpt = {
+        "hps": dict(hps) if isinstance(hps, Mapping) else hps,
+        "timesteps_so_far": timesteps_so_far,
+        "actor": clone(actor.state_dict()),
+        "qnet1": clone(qnet1.state_dict()),
+        "qnet2": clone(qnet2.state_dict()),
+        "actor_optimizer": actor_optimizer.state_dict(),
+        "q_optimizer": q_optimizer.state_dict(),
+        "actor_target": clone(actor_target),
+        "qnet_target": clone(qnet_target),
+    }
+    if log_alpha is not None:
+        ckpt["log_alpha"] = log_alpha.detach().clone()
+    if alpha_optimizer is not None:
+        ckpt["alpha_optimizer"] = alpha_optimizer.state_dict()
+    return ckpt
+
+
 class Agent:
 
     def __init__(self, net_shapes: dict[str, tuple[int, ...]], min_ac: np.ndarray, max_ac: np.ndarray,
@@ -165,12 +196,15 @@ class Agent:
         self._predict_draw = 0
         self._lo: Optional[torch.Tensor] = None  # 3xTF32 mirror of the online / target regions (wide path), see lo_mirror()
         self.autotune = False
+        # agent.py:134 fixes the target entropy at -A; a config may set it (a population member exported with its own value)
+        targ_ent = hp_get(hps, "targ_ent")
+        targ_ent = -self.ac_dim if targ_ent is None else float(targ_ent)
         if not self.td3:
             self._alpha_state[0] = math.log(hps.alpha_init)
             self.log_alpha = self._alpha_state[0:1].view(())  # 0-dim view, agent.py:128
             self.autotune = bool(hps.autotune)
             if self.autotune:
-                self.targ_ent = -self.ac_dim  # agent.py:134
+                self.targ_ent = targ_ent
                 self.alpha_optimizer = ArenaAdam(self, {"log_alpha": self.log_alpha},
                                                  {"log_alpha": self._alpha_state[2:3].view(())},
                                                  {"log_alpha": self._alpha_state[3:4].view(())},
@@ -181,7 +215,7 @@ class Agent:
             targ_smoothing=int(bool(hps.targ_actor_smoothing)) if self.td3 else 0,
             autotune=int(self.autotune), gamma=float(hps.gamma),
             td3_std=float(hps.td3_std) if self.td3 else 0.0, td3_c=float(hps.td3_c) if self.td3 else 0.0,
-            targ_ent=float(-self.ac_dim), seed=self.seed)
+            targ_ent=float(targ_ent), seed=self.seed)
         self.info = [log_module_info(m) for m in (self.actor, self.qnet1, self.qnet2)]
 
     # ------------------------------------------------------------------ plumbing
@@ -431,24 +465,11 @@ class Agent:
         """Same dict layout as the reference. Deviation (documented in DESIGN.md): ``qnet1``/``qnet2``
         hold the LIVE critics (the reference saves their stale initial weights, SURVEY.md App. C.10) and
         ``log_alpha`` / targets are included so that training can resume."""
-        fname = f"ckpt_{sfx}" if sfx is not None else f".ckpt_{self.timesteps_so_far}ts"
-        path = Path(path) / f"{fname}.pth"
-        clone = lambda sd: {k: v.detach().clone().contiguous() for k, v in sd.items()}
-        ckpt = {
-            "hps": dict(self.hps) if isinstance(self.hps, Mapping) else self.hps,
-            "timesteps_so_far": self.timesteps_so_far,
-            "actor": clone(self.actor.state_dict()),
-            "qnet1": clone(self.qnet1.state_dict()),
-            "qnet2": clone(self.qnet2.state_dict()),
-            "actor_optimizer": self.actor_optimizer.state_dict(),
-            "q_optimizer": self.q_optimizer.state_dict(),
-            "actor_target": clone(self.actor_target),
-            "qnet_target": clone(self.qnet_target),
-        }
-        if not self.td3:
-            ckpt["log_alpha"] = self.log_alpha.detach().clone()
-            if self.autotune:
-                ckpt["alpha_optimizer"] = self.alpha_optimizer.state_dict()
+        path = checkpoint_path(path, sfx, self.timesteps_so_far)
+        ckpt = checkpoint_dict(self.hps, self.timesteps_so_far, self.actor, self.qnet1, self.qnet2, self.actor_optimizer,
+                               self.q_optimizer, self.actor_target, self.qnet_target,
+                               log_alpha=None if self.td3 else self.log_alpha,
+                               alpha_optimizer=self.alpha_optimizer if self.autotune else None)
         torch.save(ckpt, path)
         return path
 

@@ -17,18 +17,25 @@ write, iteration and the log block as ONE graph replay per step, like LearnerEng
 Members may differ in their hyperparameters (a sweep, `agent_hps`), and these may change during training
 (population-based training: `set_agent_hps`, `exploit`). The kernels read them from a per-agent table in device memory
 (include/b2rl.h b2rl_agent_hp_t), so a changed value reaches the next graph replay without a recapture.
+
+A population's learner state is saved with `save` and read back in place with `load`, also by a population that holds
+a different partition of the same global ids (re-sharding); `save_agent` exports one member as an Agent checkpoint
+(tests/test_gpu_population_checkpoint.py).
 """
 from __future__ import annotations
 
 import ctypes as C
 import math
+import os
+from pathlib import Path
+from types import SimpleNamespace
 from typing import Mapping, Optional
 
 import numpy as np
 import torch
 
 from . import _lib as L
-from .agents.agent import HID_DIMS
+from .agents.agent import HID_DIMS, ArenaAdam, checkpoint_dict, checkpoint_path
 from .hps import hp_get
 from .agents.nets import Actor, Critic, TanhGaussActor
 from .arena import Arena, make_layout, set_shadow_pairs
@@ -121,6 +128,24 @@ def agent_hp_table(values: list, td3: bool) -> np.ndarray:
         r.clip_norm = v["clip_norm"] if v["clip_norm"] > 0 else math.inf
         t[g] = np.frombuffer(bytes(r), dtype=np.float32)
     return t
+
+
+CKPT_FORMAT, CKPT_VERSION = "b2rl-population", 1
+
+
+def _copy_rows(dst: torch.Tensor, src: torch.Tensor, chunk_bytes: int = 1 << 28) -> None:
+    """dst.copy_(src) between host and device in slices along dim 0: a strided side (a slice of the arena or of the replay)
+    then needs at most one slice of contiguous scratch, not a copy of the whole array."""
+    n = src.shape[0]
+    step = max(1, chunk_bytes // max(1, src[0].numel() * src.element_size())) if n else 1
+    for a in range(0, n, step):
+        dst[a:a + step].copy_(src[a:a + step])
+
+
+def _to_host(src: torch.Tensor) -> torch.Tensor:
+    out = torch.empty(src.shape, dtype=src.dtype)
+    _copy_rows(out, src)
+    return out
 
 
 def init_agent_params(agent_id: int, seed: int, ob_dim: int, ac_dim: int, td3: bool, layer_norm: bool,
@@ -496,6 +521,15 @@ class Population:
                 raise L.B2rlError(f"agent {g} is not a local agent index in [0, {self.N})")
         return gs
 
+    def _check_graph_variant(self, values: list, what: str) -> None:
+        """Refuse per-agent values that would need a graph variant this population's graphs do not contain."""
+        for v in values:
+            if v["clip_norm"] > 0 and not self._clip:
+                raise L.B2rlError(f"{what}: clip_norm > 0 needs the clipped actor step, which this population's graphs "
+                                  "do not contain (no agent clipped at construction)")
+            if self.autotune and (v["log_alpha_lr"] > 0) != self._alpha_steps:
+                raise L.B2rlError(f"{what}: log_alpha_lr cannot move between 0 (gradient only) and positive rates")
+
     def set_agent_hps(self, agents, **values) -> None:
         """Change per-agent hyperparameters of the local agents `agents` (an index or a sequence) during training: the
         explore half of population-based training. The rows are written by a stream-ordered copy on the current stream,
@@ -509,12 +543,7 @@ class Population:
             raise L.B2rlError(f"set_agent_hps: {bad[0]!r} cannot be changed per agent during training; keys: "
                               f"{', '.join(k for k in SWEEPABLE if k != 'alpha_init')}")
         new = [dict(self._hp[g], **{k: _check_hp_value(k, v, bool(self.wide)) for k, v in values.items()}) for g in gs]
-        for v in new:
-            if v["clip_norm"] > 0 and not self._clip:
-                raise L.B2rlError("set_agent_hps: clip_norm > 0 needs the clipped actor step, which this population's graphs "
-                                  "do not contain (no agent clipped at construction)")
-            if self.autotune and (v["log_alpha_lr"] > 0) != self._alpha_steps:
-                raise L.B2rlError("set_agent_hps: log_alpha_lr cannot move between 0 (gradient only) and positive rates")
+        self._check_graph_variant(new, "set_agent_hps")
         rows = torch.from_numpy(agent_hp_table(new, self.td3)).pin_memory()
         for i, g in enumerate(gs):
             self.agent_hp_table[g].copy_(rows[i], non_blocking=True)
@@ -540,6 +569,188 @@ class Population:
                 self._lo[dst].copy_(self._lo[src])
             self.agent_hp_table[dst].copy_(self.agent_hp_table[src])
         self._hp[dst] = dict(self._hp[src])
+
+    # ------------------------------------------------------------------ checkpoints
+    def _between_steps(self, what: str) -> None:
+        if torch.cuda.is_current_stream_capturing():
+            raise L.B2rlError(f"{what}: not legal inside a graph capture")
+        torch.cuda.current_stream(self.device).synchronize()
+
+    def _hps_dict(self) -> dict:
+        return dict(self.hps) if isinstance(self.hps, Mapping) else dict(vars(self.hps))
+
+    def save(self, path, replay: bool = True) -> Path:
+        """Write the learner state of this population's agents to the file `path` (one torch.save'd dict, written to
+        path.tmp and then renamed, so an interrupted save never leaves a truncated file under the real name). Between
+        steps only: the current stream is synchronised first (no step in flight) and a call inside a graph capture is
+        refused.
+
+        The file holds a header (format, version, hps, seed, shapes, action bounds, arena region size, row stride, replay
+        capacity, wide and the GLOBAL ids of the agents) and, per agent in the order of those ids: arena regions P, T, M
+        and V (not G: the backward kernels overwrite every gradient element), alpha_state, the counters, the log block,
+        the rows of the hyperparameter table and their host values (agent_hps); then the host counters size, cursor,
+        iterations and the predict draw, and with replay=True every agent's replay rows [:size]. The staging buffers of
+        step_async are not state and are not saved. Tensors are stored on the CPU, so that a loader can torch.load the
+        file with mmap=True and read only the rows it needs."""
+        self._between_steps("save")
+        if bool(self.counters[:, [L.CTR_TICKET, L.CTR_XTICKET]].any()):
+            raise L.B2rlError("save: counters[:, CTR_TICKET / CTR_XTICKET] are not 0: a step did not complete")
+        path = Path(path)
+        ckpt = {
+            "format": CKPT_FORMAT, "version": CKPT_VERSION, "hps": self._hps_dict(), "seed": self.seed,
+            "ob_dim": self.ob_dim, "ac_dim": self.ac_dim, "min_ac": self.min_ac.tolist(), "max_ac": self.max_ac.tolist(),
+            "region": self.layout.region, "row_stride": self.fmt.row_stride, "capacity": self.capacity, "wide": self.wide,
+            "ids": list(self.ids),
+            "arena": _to_host(self.arena.flat[:, :L.REGION_G]),
+            "alpha_state": self.alpha_state.cpu(), "counters": self.counters.cpu(), "out": self.out.cpu(),
+            "agent_hp_table": self.agent_hp_table.cpu(), "agent_hps": [dict(v) for v in self._hp],
+            "size": self.size, "cursor": self.cursor, "iterations": self.iterations, "predict_draw": self._predict_draw,
+        }
+        if replay:
+            ckpt["storage"] = _to_host(self.storage[:, :self.size])
+        tmp = path.with_name(path.name + ".tmp")
+        with open(tmp, "wb") as f:
+            torch.save(ckpt, f)
+            f.flush()
+            os.fsync(f.fileno())
+        os.replace(tmp, path)
+        return path
+
+    def _read_checkpoint(self, p) -> dict:
+        """torch.load a population checkpoint (memory-mapped) and check that its learners fit this population."""
+        try:
+            ck = torch.load(p, map_location="cpu", mmap=True, weights_only=False)
+        except Exception as e:
+            raise L.B2rlError(f"load: {p}: not a population checkpoint (format: torch.load failed: {e})") from e
+        fmt = ck.get("format") if isinstance(ck, Mapping) else type(ck).__name__
+        if fmt != CKPT_FORMAT:
+            raise L.B2rlError(f"load: {p}: not a population checkpoint (format = {fmt!r}, expected {CKPT_FORMAT!r})")
+        if ck.get("version") != CKPT_VERSION:
+            raise L.B2rlError(f"load: {p}: unknown population checkpoint version = {ck.get('version')!r} "
+                              f"(this code reads version {CKPT_VERSION})")
+        theirs = dict(ck, prefer_td3_over_sac=bool(hp_get(ck["hps"], "prefer_td3_over_sac")),
+                      layer_norm=bool(hp_get(ck["hps"], "layer_norm")))
+        mine = {"prefer_td3_over_sac": self.td3, "ob_dim": self.ob_dim, "ac_dim": self.ac_dim,
+                "layer_norm": bool(self.hps.layer_norm), "min_ac": self.min_ac.tolist(), "max_ac": self.max_ac.tolist(),
+                "region": self.layout.region, "row_stride": self.fmt.row_stride, "seed": self.seed}
+        for k, v in mine.items():
+            if theirs[k] != v:
+                raise L.B2rlError(f"load: {p}: {k} = {theirs[k]!r} in the file, {v!r} in this population")
+        if "storage" in ck and ck["capacity"] != self.capacity:
+            raise L.B2rlError(f"load: {p}: capacity = {ck['capacity']} in the file (which holds the replay), "
+                              f"{self.capacity} in this population (a file saved with replay=False carries no replay)")
+        return ck
+
+    def load(self, paths) -> None:
+        """Fill this population IN PLACE from the rows of one checkpoint file or a list of them (e.g. one per rank of an
+        earlier run: each rank passes every rank's file, or one file of the whole population) whose global ids are
+        self.ids. Every write is a copy into the existing tensors, so graphs captured before the load stay valid and the
+        next iteration() / step_async() continues from the loaded state (loading an earlier checkpoint into a running
+        population rewinds it). The w2n shadows come with the arena rows; a 3xTF32 mirror, if there is one, is
+        recomputed. Between steps only: the current stream is synchronised first, and a call inside a graph capture is
+        refused.
+
+        Everything is validated before the first write (a refused load changes nothing); B2rlError names the key when a
+        file is not a population checkpoint of a known version; the algorithm, ob_dim, ac_dim, layer_norm, min_ac / max_ac,
+        region, row_stride or seed differ; capacity differs and the file holds the replay; an id of this population is in
+        no file or in more than one; the files disagree on a host counter; or a loaded hyperparameter row needs a graph
+        variant this population does not have (the rules of set_agent_hps).
+
+        A file without the replay (save(replay=False)) leaves storage, the replay counters CTR_SIZE / CTR_CURSOR and the
+        host size / cursor as they are: training continues bitwise only if the caller refills the same data. `wide` may
+        differ between the file and this population (the state has the same layout on both paths); training continues
+        bitwise only on the path that wrote the file. Everything not in the file comes from this population: batch_size,
+        actor_update_delay, crit_targ_update_freq, use_graphs and the rest of its hps."""
+        self._between_steps("load")
+        paths = [paths] if isinstance(paths, (str, os.PathLike)) else list(paths)
+        cks = [self._read_checkpoint(p) for p in paths]
+        src: dict = {}  # global id -> (file, row)
+        for k, ck in enumerate(cks):
+            for r, aid in enumerate(ck["ids"]):
+                if self.base <= aid < self.base + self.N:
+                    if aid in src:
+                        raise L.B2rlError(f"load: ids: agent {aid} is in more than one file ({paths[src[aid][0]]}, {paths[k]})")
+                    src[aid] = (k, r)
+        missing = [aid for aid in self.ids if aid not in src]
+        if missing:
+            raise L.B2rlError(f"load: ids: agent {missing[0]} is in none of the files {[str(p) for p in paths]}")
+        used = sorted({k for k, _ in src.values()})
+        for key in ("size", "cursor", "iterations", "predict_draw"):
+            if len({cks[k][key] for k in used}) > 1:
+                raise L.B2rlError(f"load: the files disagree on {key} ({[cks[k][key] for k in used]})")
+        if len({"storage" in cks[k] for k in used}) > 1:
+            raise L.B2rlError("load: storage: some of the files hold the replay and some do not")
+        new_hp = [dict(cks[src[aid][0]]["agent_hps"][src[aid][1]]) for aid in self.ids]
+        self._check_graph_variant(new_hp, "load")
+
+        runs: list = []  # [file, first local agent, first row, count]
+        for g, aid in enumerate(self.ids):
+            k, r = src[aid]
+            if runs and runs[-1][0] == k and runs[-1][2] + runs[-1][3] == r:
+                runs[-1][3] += 1
+            else:
+                runs.append([k, g, r, 1])
+        head = cks[used[0]]
+        replay, size = "storage" in head, head["size"]
+        cols = [c for c in range(self.counters.shape[1]) if replay or c not in (L.CTR_SIZE, L.CTR_CURSOR)]
+        with torch.no_grad():
+            for k, g, r, n in runs:
+                ck, dst, rows = cks[k], slice(g, g + n), slice(r, r + n)
+                _copy_rows(self.arena.flat[dst, :L.REGION_G], ck["arena"][rows])
+                self.alpha_state[dst].copy_(ck["alpha_state"][rows])
+                self.counters[dst, cols] = ck["counters"][rows][:, cols].to(self.device)
+                self.out[dst].copy_(ck["out"][rows])
+                self.agent_hp_table[dst].copy_(ck["agent_hp_table"][rows])
+                if replay:
+                    _copy_rows(self.storage[dst, :size], ck["storage"][rows])
+                    self.storage[dst, size:].zero_()
+        self._hp = new_hp
+        if replay:
+            self.size, self.cursor = size, head["cursor"]
+        self.iterations, self._predict_draw = head["iterations"], head["predict_draw"]
+        self.refresh_lo()
+
+    def save_agent(self, g: int, path, sfx: Optional[str] = None, timesteps_so_far: int = 0) -> Path:
+        """Export local member g as an Agent checkpoint in directory `path` (ckpt_{sfx}.pth, or .ckpt_{timesteps}ts.pth):
+        Agent.save's layout (agents.agent.checkpoint_dict), which Agent.load_from_disk reads. Its hps are this
+        population's with the member's effective per-agent values (agent_hps(g)) in place of the shared ones (targ_ent
+        only when it is not -ac_dim), so an Agent built from ckpt["hps"] with seed = self.seed, agent_id = base + g and
+        the member's replay trains as the member does. Between steps only."""
+        (g,) = self._agents(g)
+        self._between_steps("save_agent")
+        hp = self._hp[g]
+        hps = self._hps_dict()
+        for k, v in hp.items():
+            absent = -float(self.ac_dim) if k == "targ_ent" else _ABSENT.get(k)
+            if k in hps or v != absent:
+                hps[k] = v
+        lay, ar, ln = self.layout, self.arena, bool(self.hps.layer_norm)
+        ob, ac = (self.ob_dim,), (self.ac_dim,)
+        if self.td3:
+            actor = Actor(ob, ac, HID_DIMS, self.min_ac, self.max_ac, exploration_noise=0.0, layer_norm=ln, device="meta")
+            actor.exploration_noise = torch.as_tensor(hp["actor_noise_std"], device=self.device)
+        else:
+            actor = TanhGaussActor(ob, ac, HID_DIMS, self.min_ac, self.max_ac, layer_norm=ln, device="meta")
+        actor.bind(ar.named(lay.actor, L.REGION_P, g), requires_grad=False)
+        q1, q2 = (Critic(ob, ac, HID_DIMS, layer_norm=ln, device="meta") for _ in range(2))
+        q1.bind(ar.named(lay.critic[0], L.REGION_P, g), requires_grad=False)
+        q2.bind(ar.named(lay.critic[1], L.REGION_P, g), requires_grad=False)
+        own = SimpleNamespace(counters=self.counters[g])  # (ArenaAdam.state_dict reads the step from counters[counter])
+        pmv = (L.REGION_P, L.REGION_M, L.REGION_V)
+        actor_opt = ArenaAdam(own, *(ar.named(lay.actor, r, g) for r in pmv), hp["actor_lr"], L.CTR_PI, [])
+        q_opt = ArenaAdam(own, *(ar.stacked(r, g) for r in pmv), hp["qnets_lr"], L.CTR_Q, [])
+        kw = {}
+        if not self.td3:
+            a = self.alpha_state[g]  # {log_alpha, grad, exp_avg, exp_avg_sq, -}
+            kw["log_alpha"] = a[0]
+            if self.autotune:
+                kw["alpha_optimizer"] = ArenaAdam(own, {"log_alpha": a[0]}, {"log_alpha": a[2]}, {"log_alpha": a[3]},
+                                                  hp["log_alpha_lr"], L.CTR_ALPHA, [])
+        ckpt = checkpoint_dict(hps, timesteps_so_far, actor, q1, q2, actor_opt, q_opt, ar.named(lay.actor, L.REGION_T, g),
+                               ar.stacked(L.REGION_T, g), **kw)
+        path = checkpoint_path(path, sfx, timesteps_so_far)
+        torch.save(ckpt, path)
+        return path
 
     # ------------------------------------------------------------------ inspection
     def agent_arena(self, g: int) -> torch.Tensor:
