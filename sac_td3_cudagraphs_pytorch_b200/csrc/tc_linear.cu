@@ -661,6 +661,9 @@ tc_linear_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
           for (int c = c0; c < c0 + CPW; ++c, ++vi) {
             mbar_wait_(&S.xfull[ew][vi % NXB], (vi / NXB) & 1);
             tile_get(S.tile[ew][vi % NXB], lane, x);
+            // every lane's reads of the slot are ordered before TMA's refill of it (generic -> async proxy): without the
+            // fence a refill could overwrite rows a lane had not read yet, and their row sums took the next chunk's x-hat
+            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
             __syncwarp();
             if (lane == 0) xissue(vi + NXB);
             tmem_ld32(tl + c * 32, v);

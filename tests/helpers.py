@@ -84,3 +84,61 @@ def check_param_after_first_adam(name, got, ref32, ref64, g_got, g_ref32, lr, fl
     assert float(excess) <= 0.0, (
         f"{name}: |cuda - oracle32| exceeds tol*max|p| + lr*|adam_ratio(g_cuda) - adam_ratio(g_oracle32)| by "
         f"{float(excess):.3e} (plain rel dev {rel_dev(got, r32):.3e}, tol {tol:.3e})")
+
+
+def kink_safe(inp, batch, margin=2e-5):
+    """Rows of the batch whose online-critic pre-activations all stay `margin` away from the ReLU kink.
+    The update is discontinuous there: a pre-activation of 1.3e-6 (fp32 path, oracle) against <= 0 (3xTF32 path,
+    1e-6 away) flips one unit of one row and moves the batch gradient by 1e-2 of its max (measured on td3_hopper,
+    critic 1, row 90) — both evaluations are correct to fp32 rounding. Parity is therefore asserted on the rows
+    where the comparison is well-posed (a ragged batch, which the wide path takes as it comes)."""
+    x = torch.cat([batch["observations"], batch["actions"]], 1).double()
+    ok = torch.ones(x.shape[0], dtype=torch.bool, device=x.device)
+    ln = bool(inp["hps"]["layer_norm"])
+    for q in (inp["q1"], inp["q2"]):
+        h = x
+        for blk in ("fc_block_1", "fc_block_2"):
+            w = lambda k: q[f"fc_stack.{blk}.{k}"].to(x.device, torch.float64)
+            z = h @ w("fc.weight").T + w("fc.bias")
+            if ln:
+                z = (z - z.mean(1, keepdim=True)) / torch.sqrt(z.var(1, unbiased=False, keepdim=True) + 1e-5)
+                z = z * w("ln.weight") + w("ln.bias")
+            ok &= z.abs().min(1).values > margin
+            h = torch.relu(z)
+    return ok
+
+
+def kink_safe_actor(inp, batch, eps, margin=2e-5):
+    """As kink_safe, for the actor step: the actor's own layers on obs and the critics' layers on (obs, a_pi)."""
+    ob = batch["observations"].double()
+    dev = ob.device
+    ok = torch.ones(ob.shape[0], dtype=torch.bool, device=dev)
+    ln = bool(inp["hps"]["layer_norm"])
+
+    def trunk(x, q):
+        nonlocal ok
+        h = x
+        for blk in ("fc_block_1", "fc_block_2"):
+            w = lambda k: q[f"fc_stack.{blk}.{k}"].to(dev, torch.float64)
+            z = h @ w("fc.weight").T + w("fc.bias")
+            if ln:
+                z = (z - z.mean(1, keepdim=True)) / torch.sqrt(z.var(1, unbiased=False, keepdim=True) + 1e-5)
+                z = z * w("ln.weight") + w("ln.bias")
+            ok &= z.abs().min(1).values > margin
+            h = torch.relu(z)
+        return h
+
+    a = inp["actor"]
+    u = trunk(ob, a) @ a["head.weight"].to(dev, torch.float64).T + a["head.bias"].to(dev, torch.float64)
+    lo, hi = torch.as_tensor(inp["min_ac"]).to(dev, torch.float64), torch.as_tensor(inp["max_ac"]).to(dev, torch.float64)
+    scale, bias = (hi - lo) / 2, (hi + lo) / 2
+    A = inp["ac"]
+    if inp["hps"]["prefer_td3_over_sac"]:
+        act = torch.tanh(u) * scale + bias
+    else:
+        ls = -5.0 + 3.5 * (torch.tanh(u[:, A:]) + 1.0)
+        act = torch.tanh(u[:, :A] + eps.to(dev, torch.float64) * torch.exp(ls)) * scale + bias
+    x = torch.cat([ob, act], 1)
+    trunk(x, inp["q1"])
+    trunk(x, inp["q2"])
+    return ok

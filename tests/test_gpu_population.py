@@ -103,16 +103,19 @@ def test_wide_population_is_invariant_to_sharding(algo, B):
     assert not torch.equal(whole.arena.flat[0], whole.arena.flat[1])
 
 
-@pytest.mark.parametrize("algo", ["sac", "td3"])
-def test_wide_population_matches_the_fp32_row_path(algo):
+@pytest.mark.parametrize("algo,B", [("sac", 256), ("td3", 256), ("sac", 1000), ("td3", 1000)],
+                         ids=["sac", "td3", "sac-1000", "td3-1000"])
+def test_wide_population_matches_the_fp32_row_path(algo, B):
     """Same agents, data, index draws and noise on the row-group fp32 kernels and on the stacked 3xTF32 tensor-core path:
     after the first iteration (critic step + two actor steps from identical state) the losses agree to 2e-5, the critics'
     gradients to 5e-5 of each agent's largest entry (stated 3xTF32 bound; a ReLU unit within ~1e-6 of its kink may flip
     between two correct evaluations — seeds are fixed, and none does here), and after 6 iterations the parameters to 2e-3
-    (Adam's first steps move every weight by lr whatever the gradient's size, which amplifies rounding-level differences)."""
+    (Adam's first steps move every weight by lr whatever the gradient's size, which amplifies rounding-level differences).
+    B = 1000 gives every agent several CTAs of each wide kernel (8 tiles of 128 rows, 4 of 256, 125 head groups of 8) and a
+    ragged last tile, with the agents' rows stacked back to back."""
     from sac_td3_cudagraphs_pytorch_b200 import _lib as L
     ids = [3, 4, 5]
-    wide, row = _wide_population(ids, algo, 256), _wide_population(ids, algo, 256, wide=None)
+    wide, row = _wide_population(ids, algo, B), _wide_population(ids, algo, B, wide=None)
     wide.iteration()
     row.iteration()
     torch.cuda.synchronize()

@@ -1,6 +1,10 @@
 """tcgen05 (TF32) large-batch hidden layer vs torch: Linear -> LayerNorm -> ReLU (agents/nets.py:66-82).
 Tolerance: TF32 products (10-bit mantissa, truncated operands) — stated bound 3e-3 of the output scale; the
-LayerNorm statistics and everything after the product are fp32."""
+LayerNorm statistics and everything after the product are fp32.
+M = 65 536 (BASELINE.json config 5) runs the forward, first-layer and backward pipelines at full grid — 148 CTAs with four
+tiles each, every ring slot and both TMEM buffers reused — with the same bounds as the small sizes: each output row (and
+each per-tile column sum) is one K = 256 (or K = O) accumulation whatever M is, so unlike the weight gradient's
+batch-long contraction there is no longer chain to allow for."""
 import ctypes as C
 
 import pytest
@@ -10,7 +14,8 @@ pytestmark = pytest.mark.gpu
 
 
 @pytest.mark.parametrize("x3", [False, True])
-@pytest.mark.parametrize("M,ln,relu", [(128, True, True), (1000, True, True), (4096, False, True), (300, True, False)])
+@pytest.mark.parametrize("M,ln,relu", [(128, True, True), (1000, True, True), (4096, False, True), (300, True, False),
+                                       (65536, True, True)])
 def test_tc_linear_matches_torch(M, ln, relu, x3):
     from sac_td3_cudagraphs_pytorch_b200 import _lib as L
     lib = L.load()
@@ -167,7 +172,7 @@ def test_tc_wgrad_stacked_agents_match_torch(n_agents, Bn, MA, lda, x3):
 
 @pytest.mark.parametrize("x3", [False, True])
 @pytest.mark.parametrize("n_agents,M,K,ldx", [(1, 256, 14, 28), (3, 200, 14, 28), (1, 1000, 11, 16), (2, 256, 393, 396), (1, 128, 32, 32),
-                                              (4, 72, 5, 8)])
+                                              (4, 72, 5, 8), (1, 65536, 14, 28)])
 def test_tc_first_layer_matches_torch(n_agents, M, K, ldx, x3):
     """The first layer on the tensor cores (MODE 1): X [M][K] K-major, w1t [K][256] MN-major (the arena's forward layout),
     K not a multiple of 32 (tails zero-filled by TMA on both operands), stacked agents with their own weights, vs float64
@@ -233,7 +238,8 @@ def _bwd_reference(DZ2, W2t, XH, rstd, gam, bet, ln):
 
 
 @pytest.mark.parametrize("x3", [False, True, "in-kernel"])  # in-kernel: W_lo == W, the weights' lo parts made in shared memory
-@pytest.mark.parametrize("n_agents,M,ln", [(1, 1000, True), (1, 4096, True), (3, 200, True), (1, 300, False), (2, 72, True)])
+@pytest.mark.parametrize("n_agents,M,ln", [(1, 1000, True), (1, 4096, True), (3, 200, True), (1, 300, False), (2, 72, True),
+                                            (1, 65536, True)])
 def test_tc_linear_bwd_matches_torch(n_agents, M, ln, x3):
     """b2rl_tc_linear_bwd against float64: dz1 and the per-tile column sums (ragged and stacked batches), and part = NULL
     (dX only, the actor step's pass through the critics) gives the same dz1 bit for bit."""
@@ -332,8 +338,10 @@ def test_wide_ln_bwd_matches_torch(M, n_out):
 def test_tc_kernels_are_reproducible_at_full_grid():
     """The 2-SM pipelines at a machine-filling size (65 536 rows: 148 CTAs, four tiles each, every ring slot and both TMEM
     buffers reused; cross-CTA mbarrier arrivals, TMA-fed and TMA-stored epilogues): 12 launches each of the 3xTF32 forward,
-    backward and weight-gradient kernels from the same inputs must give the same bits — a race in the hand-rolled
-    synchronisation would show up as a result that depends on timing."""
+    backward and weight-gradient kernels, and of the plain-TF32 backward (the multicast pipeline, one CTA per MMA, whose
+    epilogue runs ahead of it), from the same inputs must give the same bits — a race in the hand-rolled synchronisation
+    would show up as a result that depends on timing. (The plain-TF32 backward once refilled an x-hat slot by TMA without
+    ordering the lanes' reads of it first: a few rows per launch took the next chunk's x-hat into their LayerNorm sums.)"""
     from sac_td3_cudagraphs_pytorch_b200 import _lib as L
     lib = L.load()
     L.init_device(torch.device("cuda"))
@@ -359,14 +367,17 @@ def test_tc_kernels_are_reproducible_at_full_grid():
         DZ1, part = torch.empty(M, 256, device="cuda"), torch.empty(nt, 3, 256, device="cuda")
         L.check(lib.b2rl_tc_linear_bwd(DZ.data_ptr(), M, W.data_ptr(), Wlo.data_ptr(), XH.data_ptr(), stat.data_ptr(), gam.data_ptr(),
                                        bet.data_ptr(), 1, DZ1.data_ptr(), part.data_ptr(), None, st), "tc_linear_bwd")
+        DZ1t = torch.empty(M, 256, device="cuda")
+        L.check(lib.b2rl_tc_linear_bwd(DZ.data_ptr(), M, W.data_ptr(), None, XH.data_ptr(), stat.data_ptr(), gam.data_ptr(),
+                                       bet.data_ptr(), 1, DZ1t.data_ptr(), None, None, st), "tc_linear_bwd (TF32)")
         G, Gt = torch.empty(256, 256, device="cuda"), torch.empty(256, 256, device="cuda")
         L.check(lib.b2rl_tc_wgrad(H.data_ptr(), 256, 256, 256, DZ1.data_ptr(), M, G.data_ptr(), Gt.data_ptr(), scratch.data_ptr(), 1,
                                   None, None, st), "tc_wgrad")
         torch.cuda.synchronize()
-        cur = (H, XH, stat, DZ1, part, G, Gt)
+        cur = (H, XH, stat, DZ1, part, G, Gt, DZ1t)
         if first is None:
             first = cur
             assert all(torch.isfinite(t).all() for t in cur)
         else:
-            for a, c, what in zip(first, cur, ("H", "x-hat", "stat", "dz1", "column sums", "dW", "dW^T")):
+            for a, c, what in zip(first, cur, ("H", "x-hat", "stat", "dz1", "column sums", "dW", "dW^T", "dz1 (TF32)")):
                 assert torch.equal(a, c), f"launch {it}: {what} differs from the first launch"
