@@ -21,18 +21,26 @@ Members may differ in their hyperparameters (a sweep, `agent_hps`), and these ma
 A population's learner state is saved with `save` and read back in place with `load`, also by a population that holds
 a different partition of the same global ids (re-sharding); `save_agent` exports one member as an Agent checkpoint
 (tests/test_gpu_population_checkpoint.py).
+
+A population sharded over the ranks of a process group is one population for PBT: `all_gather` puts every agent's score
+in global id order on every rank, and `exploit_many` moves learner states between any global ids — device copies on a
+rank, point-to-point transfers between ranks — with the result of a single-rank population that did the same exploits
+(tests/test_gpu_population_pbt.py).
 """
 from __future__ import annotations
 
 import ctypes as C
+import hashlib
 import math
+import operator
 import os
 from pathlib import Path
 from types import SimpleNamespace
-from typing import Mapping, Optional
+from typing import Mapping, NamedTuple, Optional, Sequence
 
 import numpy as np
 import torch
+import torch.distributed as dist
 
 from . import _lib as L
 from .agents.agent import HID_DIMS, ArenaAdam, checkpoint_dict, checkpoint_path
@@ -128,6 +136,126 @@ def agent_hp_table(values: list, td3: bool) -> np.ndarray:
         r.clip_norm = v["clip_norm"] if v["clip_norm"] > 0 else math.inf
         t[g] = np.frombuffer(bytes(r), dtype=np.float32)
     return t
+
+
+def _graph_variant_problem(v: dict, clip: bool, autotune: bool, alpha_steps: bool) -> Optional[str]:
+    """Why per-agent values v need a graph variant that graphs captured with these flags do not contain (None: they fit)."""
+    if v["clip_norm"] > 0 and not clip:
+        return "clip_norm > 0 needs the clipped actor step, which this population's graphs do not contain (no agent " \
+               "clipped at construction)"
+    if autotune and (v["log_alpha_lr"] > 0) != alpha_steps:
+        return "log_alpha_lr cannot move between 0 (gradient only) and positive rates"
+    return None
+
+
+# ---------------------------------------------------------------------- population-based training over a sharded population
+def _normalize_pairs(pairs) -> list:
+    """[(dst, src)] as Python ints; B2rlError on anything that is not a sequence of integer pairs."""
+    try:
+        out = [(operator.index(d), operator.index(s)) for d, s in pairs]
+    except (TypeError, ValueError) as e:
+        raise L.B2rlError(f"exploit_many: pairs must be a sequence of (dst, src) integer global ids ({e})") from None
+    return out
+
+
+def check_pairs(pairs, n_total: int) -> list:
+    """The (dst, src) global ids of one PBT round, validated: every id in [0, n_total), no dst twice, no dst == src."""
+    pairs = _normalize_pairs(pairs)
+    seen = set()
+    for d, s in pairs:
+        for what, x in (("dst", d), ("src", s)):
+            if not 0 <= x < n_total:
+                raise L.B2rlError(f"exploit_many: {what} id {x} is outside [0, n_total = {n_total})")
+        if d == s:
+            raise L.B2rlError(f"exploit_many: pair ({d}, {s}): dst and src are the same agent")
+        if d in seen:
+            raise L.B2rlError(f"exploit_many: dst {d} appears in more than one pair")
+        seen.add(d)
+    return pairs
+
+
+class ExploitPlan(NamedTuple):
+    """What one rank does in a PBT round (global ids). copies: (dst, src) with both on this rank. snapshots: this rank's
+    srcs that are also dsts — cloned before anything is written, and read from the clone. sends / recvs: (peer, dst, src)
+    with src / dst on this rank and the other on peer, in ascending dst order — so rank r's sends to rank s, in order,
+    are rank s's receives from r."""
+    copies: list
+    snapshots: list
+    sends: list
+    recvs: list
+
+
+def plan_exploit(pairs, owner: Sequence[int], rank: int) -> ExploitPlan:
+    """The plan of `rank` for validated pairs (check_pairs); owner[id] is the rank that holds global id `id`. Every dst
+    ends with its src's state as it was before the round (chains and swaps included), whatever the order of the pairs."""
+    pairs = sorted(pairs)
+    dsts = {d for d, _ in pairs}
+    copies, sends, recvs, read = [], [], [], set()
+    for d, s in pairs:
+        rd, rs = owner[d], owner[s]
+        if rs == rank:
+            read.add(s)
+            (copies.append((d, s)) if rd == rank else sends.append((rd, d, s)))
+        elif rd == rank:
+            recvs.append((rs, d, s))
+    return ExploitPlan(copies, sorted(read & dsts), sends, recvs)
+
+
+class _Ranks:
+    """The ranks of a process group that together hold one population: the id block, configuration and graph-variant
+    flags of each, gathered once per population and group and validated (every rank reaches the same verdict)."""
+
+    def __init__(self, pop: "Population", group):
+        self.group = group
+        self.world = dist.get_world_size(group) if dist.is_initialized() else 1
+        self.rank = dist.get_rank(group) if dist.is_initialized() else 0
+        # gloo moves host tensors only: state travels through host buffers there (NCCL reads and writes the device rows)
+        self.staged = self.world > 1 and dist.get_backend(group) == dist.Backend.GLOO
+        got = self.gather((pop.base, pop.N, pop._config(), (pop._clip, pop.autotune, pop._alpha_steps)))
+        for r, (_, _, cfg, _) in enumerate(got):
+            for k, v in cfg.items():
+                if v != got[0][2][k]:
+                    raise L.B2rlError(f"sharded population: the configurations differ between ranks: {k} = {v!r} "
+                                      f"on rank {r}, {got[0][2][k]!r} on rank 0")
+        blocks = sorted((base, base + n, r) for r, (base, n, _, _) in enumerate(got))
+        end = 0
+        for lo, hi, r in blocks:
+            if lo != end:
+                raise L.B2rlError(f"sharded population: the ranks' id ranges {'overlap' if lo < end else 'leave a hole'}: "
+                                  f"rank {r} holds [{lo}, {hi}), the ranks before it end at {end}")
+            end = hi
+        self.n_total = end
+        self.ranges = [range(base, base + n) for base, n, _, _ in got]
+        self.owner = np.empty(end, dtype=np.int64)
+        for r, ids in enumerate(self.ranges):
+            self.owner[ids.start:ids.stop] = r
+        self.flags = [f for _, _, _, f in got]
+
+    def gather(self, obj) -> list:
+        if self.world == 1:
+            return [obj]
+        out = [None] * self.world
+        dist.all_gather_object(out, obj, group=self.group)
+        return out
+
+    def post(self, ops: list):
+        """Post the point-to-point transfers [(send?, peer rank in the group, device tensor)] as one batch; returns the
+        function that waits for them (stream-ordered on the current stream under NCCL)."""
+        if not ops:
+            return lambda: None
+        bufs = [t.cpu() if send else torch.empty(t.shape, dtype=t.dtype) for send, _, t in ops] if self.staged else \
+            [t for _, _, t in ops]
+        reqs = dist.batch_isend_irecv([dist.P2POp(dist.isend if send else dist.irecv, b, group=self.group, group_peer=p)
+                                       for (send, p, _), b in zip(ops, bufs)])
+
+        def wait():
+            for r in reqs:
+                r.wait()
+            if self.staged:
+                for (send, _, t), b in zip(ops, bufs):
+                    if not send:
+                        t.copy_(b)
+        return wait
 
 
 CKPT_FORMAT, CKPT_VERSION = "b2rl-population", 1
@@ -261,6 +389,7 @@ class Population:
             self.wide_pi = WideActor(own, self.B, wide)
         self._stage = StepStaging(dev, (N,), self.fmt.row_stride, self.ob_dim, self.ac_dim)
         self._predict_draw = 0
+        self._rank_layouts: dict = {}  # process group -> _Ranks (exploit_many, all_gather, n_total)
 
     # ------------------------------------------------------------------ replay
     def fill_replay(self, td: Mapping[str, torch.Tensor], agent: Optional[int] = None) -> None:
@@ -524,11 +653,9 @@ class Population:
     def _check_graph_variant(self, values: list, what: str) -> None:
         """Refuse per-agent values that would need a graph variant this population's graphs do not contain."""
         for v in values:
-            if v["clip_norm"] > 0 and not self._clip:
-                raise L.B2rlError(f"{what}: clip_norm > 0 needs the clipped actor step, which this population's graphs "
-                                  "do not contain (no agent clipped at construction)")
-            if self.autotune and (v["log_alpha_lr"] > 0) != self._alpha_steps:
-                raise L.B2rlError(f"{what}: log_alpha_lr cannot move between 0 (gradient only) and positive rates")
+            problem = _graph_variant_problem(v, self._clip, self.autotune, self._alpha_steps)
+            if problem:
+                raise L.B2rlError(f"{what}: {problem}")
 
     def set_agent_hps(self, agents, **values) -> None:
         """Change per-agent hyperparameters of the local agents `agents` (an index or a sequence) during training: the
@@ -569,6 +696,146 @@ class Population:
                 self._lo[dst].copy_(self._lo[src])
             self.agent_hp_table[dst].copy_(self.agent_hp_table[src])
         self._hp[dst] = dict(self._hp[src])
+
+    # ------------------------------------------------------------------ the whole population over the ranks of a process group
+    def _config(self) -> dict:
+        """What must be the same on every rank for learner states to move between them."""
+        return {"algorithm": "td3" if self.td3 else "sac", "ob_dim": self.ob_dim, "ac_dim": self.ac_dim,
+                "layer_norm": bool(self.hps.layer_norm), "wide": self.wide, "region": self.layout.region,
+                "row_stride": self.fmt.row_stride}
+
+    def _ranks(self, group) -> _Ranks:
+        """The id blocks of the ranks of `group` (None: the default process group if there is one, else this rank
+        alone). Collective the first time for a group: every rank of it calls."""
+        key = group if group is not None else ("default" if dist.is_initialized() else None)
+        r = self._rank_layouts.get(key)
+        if r is None:
+            r = self._rank_layouts[key] = _Ranks(self, group)
+        return r
+
+    @property
+    def n_total(self) -> int:
+        """The number of agents of the whole population over the ranks of the default process group (this population's
+        when there is none). Collective on the first use (see exploit_many)."""
+        return self._ranks(None).n_total
+
+    def local_index(self, global_id: int) -> Optional[int]:
+        """The local index of global agent id `global_id`, or None when another rank holds it."""
+        g = operator.index(global_id) - self.base
+        return g if 0 <= g < self.N else None
+
+    def all_gather(self, values, group=None) -> np.ndarray:
+        """Per-local-agent values [N, ...] (evaluation scores, say; a tensor or anything np.asarray takes) -> an array
+        [n_total, ...] in global id order, the same on every rank of `group` (shards may differ in size). Collective."""
+        ranks = self._ranks(group)
+        v = values.detach().cpu().numpy() if isinstance(values, torch.Tensor) else np.asarray(values)
+        got = ranks.gather(v)
+        for r, a in enumerate(got):
+            if a.ndim < 1 or a.shape[0] != len(ranks.ranges[r]) or a.shape[1:] != got[0].shape[1:]:
+                raise L.B2rlError(f"all_gather: rank {r} passed values of shape {a.shape}; expected [{len(ranks.ranges[r])}"
+                                  f"{''.join(', ' + str(x) for x in got[0].shape[1:])}] (one row per local agent)")
+        out = np.empty((ranks.n_total, *got[0].shape[1:]), dtype=np.result_type(*got))
+        for r, a in enumerate(got):
+            out[ranks.ranges[r].start:ranks.ranges[r].stop] = a
+        return out
+
+    def _aux(self, ids: list) -> torch.Tensor:
+        """The small state exploit moves for these local agents (global ids) as one float32 tensor [len(ids), 27]:
+        alpha_state, the optimizer step counters CTR_Q..CTR_ALPHA (int64, bit for bit) and the hyperparameter row."""
+        g = [i - self.base for i in ids]
+        ctr = self.counters[g, L.CTR_Q:L.CTR_ALPHA + 1].contiguous().view(torch.float32)
+        return torch.cat([self.alpha_state[g], ctr, self.agent_hp_table[g]], dim=1)
+
+    def _set_aux(self, ids: list, aux: torch.Tensor) -> None:
+        if not ids:
+            return
+        g = [i - self.base for i in ids]
+        a, c, h = aux.split([self.alpha_state.shape[1], 2 * (L.CTR_ALPHA + 1 - L.CTR_Q), self.agent_hp_table.shape[1]], 1)
+        self.alpha_state[g] = a
+        # the counters' bits back as int64 through a fresh buffer: a column slice of aux cannot be viewed as int64 itself
+        ctr = torch.empty(len(g), c.shape[1] // 2, dtype=torch.int64, device=aux.device)
+        ctr.view(torch.float32).copy_(c)
+        self.counters[g, L.CTR_Q:L.CTR_ALPHA + 1] = ctr
+        self.agent_hp_table[g] = h
+
+    def exploit_many(self, pairs, group=None) -> None:
+        """One exploit round of population-based training over the whole population held by the ranks of `group` (None:
+        the default process group if one is initialised, else this rank alone, with no communication). pairs: (dst, src)
+        GLOBAL ids. Collective: every rank of the group calls it with the same pairs.
+
+        The result is as if every dst took its src's learner state as it was when the call started (chains and swaps
+        included), copying what exploit copies: the arena row, alpha_state, counters[CTR_Q..CTR_ALPHA], the 3xTF32 mirror
+        row if this rank has one (recomputed from the arena row when the src is on another rank), the hyperparameter
+        row and its host values. A dst keeps its replay slice, its replay counters, its log block and its global id.
+        Pairs within a rank are device copies (a src that is also a dst is cloned first); between ranks each rank sends
+        and receives only its own agents' rows, point to point (batch_isend_irecv; from and into the device tensors under
+        NCCL, through host buffers under gloo). Follow with set_agent_hps on the dsts a rank holds (local_index) to
+        perturb.
+
+        Between steps only: a call inside a graph capture is refused and the current stream is synchronised first.
+        Everything is validated from data gathered from every rank before any write or transfer, so every rank raises
+        the same B2rlError when: an id is outside [0, n_total); a dst appears twice; dst == src; the pair lists differ
+        between ranks; the populations' configurations differ between ranks (algorithm, shapes, layer_norm, wide, region,
+        row stride); the ranks' id ranges overlap or leave a hole; or a src's hyperparameters need a graph variant the
+        dst's population does not contain (the rules of set_agent_hps)."""
+        if torch.cuda.is_current_stream_capturing():
+            raise L.B2rlError("exploit_many: not legal inside a graph capture")
+        ranks = self._ranks(group)
+        try:
+            norm, err = _normalize_pairs(pairs), None
+        except L.B2rlError as e:
+            norm, err = None, str(e)
+        digest = None if norm is None else hashlib.sha256(repr(norm).encode()).hexdigest()
+        mine = {} if norm is None else {s: self._hp[s - self.base] for _, s in norm if self.local_index(s) is not None}
+        got = ranks.gather((err, digest, mine))
+        for r, (e, _, _) in enumerate(got):
+            if e is not None:
+                raise L.B2rlError(e if ranks.world == 1 else f"{e} (on rank {r})")
+        if len({dg for _, dg, _ in got}) > 1:
+            raise L.B2rlError(f"exploit_many: the pair lists differ between ranks (digests {[dg[:12] for _, dg, _ in got]})")
+        pairs = check_pairs(norm, ranks.n_total)
+        hp = {s: v for _, _, m in got for s, v in m.items()}
+        for d, s in pairs:
+            r = int(ranks.owner[d])
+            problem = _graph_variant_problem(hp[s], *ranks.flags[r])
+            if problem:
+                raise L.B2rlError(f"exploit_many: pair ({d}, {s}): agent {s}'s hyperparameters do not fit the population "
+                                  f"of rank {r}: {problem}")
+        plan = plan_exploit(pairs, ranks.owner, ranks.rank)
+        self._between_steps("exploit_many")
+
+        base, flat, lo = self.base, self.arena.flat, self._lo
+        with torch.no_grad():
+            snap = {s: (flat[s - base].clone(), None if lo is None else lo[s - base].clone()) for s in plan.snapshots}
+            row = lambda s: snap[s][0] if s in snap else flat[s - base]
+            lo_row = lambda s: snap[s][1] if s in snap else lo[s - base]
+            copy_aux = self._aux([s for _, s in plan.copies])
+            peers = lambda items: {p: [(d, s) for q, d, s in items if q == p] for p in sorted({q for q, _, _ in items})}
+            sends, recvs = peers(plan.sends), peers(plan.recvs)
+            ops, recv_aux = [], {}
+            for p, ds in sends.items():  # per peer: the small state of every pair in one tensor, then each arena row
+                ops += [(True, p, self._aux([s for _, s in ds]))] + [(True, p, row(s)) for _, s in ds]
+            for p, ds in recvs.items():
+                recv_aux[p] = torch.empty(len(ds), copy_aux.shape[1], dtype=torch.float32, device=self.device)
+                ops += [(False, p, recv_aux[p])] + [(False, p, flat[d - base]) for d, _ in ds]
+            wait = ranks.post(ops)
+            for d, s in plan.copies:
+                flat[d - base].copy_(row(s))
+                if lo is not None:
+                    lo[d - base].copy_(lo_row(s))
+            self._set_aux([d for d, _ in plan.copies], copy_aux)
+            wait()
+            for p, ds in recvs.items():
+                self._set_aux([d for d, _ in ds], recv_aux[p])
+                if lo is not None:  # the mirror is the lo part of the arena row, element by element (tc_split_lo)
+                    for d, _ in ds:
+                        g = d - base
+                        stk = L.Stack(1, d, self.arena.agent_stride, 2 * self.layout.region, 0, 0, 0)
+                        L.check(self._lib.b2rl_tc_split_lo(flat[g].data_ptr(), lo[g].data_ptr(), 2 * self.layout.region,
+                                                           C.byref(stk), self._stream()), "tc_split_lo")
+        for d, s in pairs:
+            if self.local_index(d) is not None:
+                self._hp[d - base] = dict(hp[s])
 
     # ------------------------------------------------------------------ checkpoints
     def _between_steps(self, what: str) -> None:
