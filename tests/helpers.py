@@ -29,6 +29,16 @@ def make_oracle(inp, dtype=torch.float32, capturable=True) -> OracleAgent:
                        dtype=dtype, actor_init=cast(inp["actor"]), qnet_init=[cast(inp["q1"]), cast(inp["q2"])])
 
 
+def oracle_cuda(inp, dtype) -> OracleAgent:
+    """The reference learner on the GPU (float32 or float64) with the case's parameters. Its fp32 products must be
+    true fp32: on TF32 the fp32 oracle would be a worse yardstick than the CUDA path it judges."""
+    assert not torch.backends.cuda.matmul.allow_tf32 and torch.get_float32_matmul_precision() == "highest", \
+        "the fp32 oracle must not run its products on TF32"
+    cast = lambda d: {k: v.to(dtype) for k, v in d.items()}
+    return OracleAgent(inp["ob"], inp["ac"], inp["min_ac"], inp["max_ac"], oracle_hps(inp["hps"], True), device="cuda", dtype=dtype,
+                       actor_init=cast(inp["actor"]), qnet_init=[cast(inp["q1"]), cast(inp["q2"])])
+
+
 def make_agent(inp, device="cuda", seed=0):
     from sac_td3_cudagraphs_pytorch_b200 import Hps
     from sac_td3_cudagraphs_pytorch_b200.agents.agent import Agent

@@ -13,7 +13,7 @@ from tests.helpers import make_agent
 pytestmark = pytest.mark.gpu
 
 
-def _run(name, noise_level, iters=9, engine="row"):
+def _run(name, noise_level, iters=9, engine="row", batch=None):
     from sac_td3_cudagraphs_pytorch_b200.engine import LearnerEngine
     from sac_td3_cudagraphs_pytorch_b200.replay import ReplayBuffer
     inp = case_inputs(CASES[name])
@@ -24,7 +24,7 @@ def _run(name, noise_level, iters=9, engine="row"):
     big_a, big_b = torch.empty(48 << 20, device="cuda"), torch.empty(48 << 20, device="cuda")  # 192 MB each: larger than L2
     ma = torch.randn(2048, 2048, device="cuda")
     if engine == "row":
-        eng = LearnerEngine(ag, rb, batch_size=inp["B"], use_graphs=True)
+        eng = LearnerEngine(ag, rb, batch_size=batch or inp["B"], use_graphs=True)
         step = eng.iteration
     else:
         from sac_td3_cudagraphs_pytorch_b200.dp import DataParallelLearner, GradComm
@@ -41,12 +41,15 @@ def _run(name, noise_level, iters=9, engine="row"):
     return ag.arena.flat.clone(), ag.out.clone(), ag.counters.clone()
 
 
-@pytest.mark.parametrize("name,engine", [("td3_hopper", "row"), ("sac_hopper", "row"), ("sac_humanoid_b256", "row"),
-                                         ("sac_hopper", "wide"), ("td3_hopper", "wide")])
-def test_results_do_not_depend_on_timing(name, engine):
-    ref = _run(name, 0, engine=engine)
+@pytest.mark.parametrize("name,engine,batch", [pytest.param(n, e, None, id=f"{n}-{e}") for n, e in (
+    ("td3_hopper", "row"), ("sac_hopper", "row"), ("sac_humanoid_b256", "row"), ("sac_hopper", "wide"), ("td3_hopper", "wide"))]
+    + [pytest.param("sac_hopper", "row", 8192, id="sac_hopper-row-8192")])
+def test_results_do_not_depend_on_timing(name, engine, batch):
+    """batch 8 192 on the row path: the temperature step's last-cluster ticket (alpha_kernel) sees 1 024 arrivals, and its
+    last cluster sums 1 024 partials (32 per lane)."""
+    ref = _run(name, 0, engine=engine, batch=batch)
     assert torch.isfinite(ref[1]).all()
     for level in (1, 3, 6):
-        got = _run(name, level, engine=engine)
+        got = _run(name, level, engine=engine, batch=batch)
         for a, b, what in zip(ref, got, ("arena", "log block", "counters")):
             assert torch.equal(a, b), f"{name}/{engine}: {what} differs under background load level {level}"

@@ -72,8 +72,12 @@ def _arena_equal(a, b):
     return torch.equal(a.arena.flat, b.arena.flat) and torch.equal(a._alpha_state, b._alpha_state)
 
 
-@pytest.mark.parametrize("name", ["sac_hopper", "td3_hopper", "sac_clip_targfreq2"])
-def test_engine_graph_equals_eager_equals_api(name):
+@pytest.mark.parametrize("name,batch", [pytest.param(n, None, id=n) for n in ("sac_hopper", "td3_hopper", "sac_clip_targfreq2")]
+                         + [pytest.param("sac_hopper", 4097, id="sac_hopper-4097")])
+def test_engine_graph_equals_eager_equals_api(name, batch):
+    """batch 4 097: 513 rows per warp slice of the weight-gradient kernel (17 staged chunks), so wgrad_kernel<true> (the
+    fused optimizer) is bitwise equal to wgrad_kernel<false> followed by Adam on the long form of every batch loop as well
+    (test_gpu_row_kernels.py checks the plain kernel against float64 there)."""
     from sac_td3_cudagraphs_pytorch_b200.engine import LearnerEngine
     inp = case_inputs(name)
     td = inp["storage"]
@@ -82,8 +86,8 @@ def test_engine_graph_equals_eager_equals_api(name):
     rbs = [_rb(td["observations"].shape[0], td, seed=99) for _ in range(3)]
     # the graph engine also takes the fused-optimizer path (Adam + Polyak inside the weight-gradient kernel),
     # the eager one the three-launch path: bitwise equality below covers b2rl_*_update_opt
-    eng_graph = LearnerEngine(agents[0], rbs[0], use_graphs=True, fused_opt=True)
-    eng_eager = LearnerEngine(agents[1], rbs[1], use_graphs=False, record_noise=True)
+    eng_graph = LearnerEngine(agents[0], rbs[0], batch_size=batch, use_graphs=True, fused_opt=True)
+    eng_eager = LearnerEngine(agents[1], rbs[1], batch_size=batch, use_graphs=False, record_noise=True)
     api = agents[2]
     for i in range(n_it):
         eng_graph.iteration(i)

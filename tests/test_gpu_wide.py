@@ -147,15 +147,6 @@ def test_wide_critic_step_bound_on_the_whole_batch(name):
 
 
 # ---- the steps at the batch they exist for, and over the shape / option space ----------------------------------------------
-def _oracle_cuda(inp, dtype):
-    """The reference learner on the GPU (float32 or float64) with the case's parameters."""
-    from oracle import OracleAgent
-    from tests.helpers import oracle_hps
-    cast = lambda d: {k: v.to(dtype) for k, v in d.items()}
-    return OracleAgent(inp["ob"], inp["ac"], inp["min_ac"], inp["max_ac"], oracle_hps(inp["hps"], True), device="cuda", dtype=dtype,
-                       actor_init=cast(inp["actor"]), qnet_init=[cast(inp["q1"]), cast(inp["q2"])])
-
-
 def _wide_steps_match_the_oracle(case, tag, min_keep=0.75):
     """One wide critic step and one wide actor (+ temperature) step on 3xTF32, each from the case's initial state, against
     the fp32 oracle with the fp32 oracle's own distance to float64 as yardstick (tests/helpers.check_close), on the rows of
@@ -169,10 +160,8 @@ def _wide_steps_match_the_oracle(case, tag, min_keep=0.75):
     must leave."""
     from sac_td3_cudagraphs_pytorch_b200.replay import pack_rows
     from sac_td3_cudagraphs_pytorch_b200.wide import WideActor, WideCritic
-    from tests.helpers import alpha_loss_scale, check_close, check_param_after_first_adam
+    from tests.helpers import alpha_loss_scale, check_close, check_param_after_first_adam, oracle_cuda
     gfloor, afloor = TOLS["3xtf32"][1], 10 * TOLS["3xtf32"][0]
-    assert not torch.backends.cuda.matmul.allow_tf32 and torch.get_float32_matmul_precision() == "highest", \
-        "the fp32 oracle must not run its products on TF32"
     inp = case_inputs(case)
     full = batch_of(inp, 0, device="cuda")
     # ---- critic step
@@ -182,7 +171,7 @@ def _wide_steps_match_the_oracle(case, tag, min_keep=0.75):
     B = int(keep.sum())
     assert B >= min_keep * inp["B"], "the kink filter should only drop a few rows"
     ag = make_agent(inp)
-    o32, o64 = _oracle_cuda(inp, torch.float32), _oracle_cuda(inp, torch.float64)
+    o32, o64 = oracle_cuda(inp, torch.float32), oracle_cuda(inp, torch.float64)
     tq = torch.zeros(B, device="cuda")
     wc = WideCritic(ag, B, "3xtf32")
     out = wc.update_qnets(pack_rows(batch, ag.fmt), eps=eps, targ_out=tq)
@@ -205,7 +194,7 @@ def _wide_steps_match_the_oracle(case, tag, min_keep=0.75):
     B = int(keep.sum())
     assert B >= min_keep * inp["B"]
     ag = make_agent(inp)
-    o32, o64 = _oracle_cuda(inp, torch.float32), _oracle_cuda(inp, torch.float64)
+    o32, o64 = oracle_cuda(inp, torch.float32), oracle_cuda(inp, torch.float64)
     wa = WideActor(ag, B, "3xtf32")
     out = wa.update_actor(pack_rows(batch, ag.fmt), eps=e1, eps_alpha=e2)
     r32 = o32.update_actor(batch, e1, e2)
