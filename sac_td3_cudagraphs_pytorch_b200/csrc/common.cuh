@@ -56,8 +56,14 @@ static __device__ long long g_b2rl_timing[64];  // one copy per translation unit
   do {                                                                                     \
     if (blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0) g_b2rl_timing[slot] = clock64(); \
   } while (0)
+// the same on CTA 0 or CTA 1 (each CTA's own clock: compare its slots with its own start)
+#define B2RL_TICK2(slot)                                                                   \
+  do {                                                                                     \
+    if (blockIdx.x < 2 && blockIdx.y == 0 && threadIdx.x == 0) g_b2rl_timing[slot] = clock64(); \
+  } while (0)
 #else
 #define B2RL_TICK(slot) do {} while (0)
+#define B2RL_TICK2(slot) do {} while (0)
 #endif
 
 // ---- cluster launches ----------------------------------------------------------------------------------------

@@ -4,10 +4,15 @@
 // is wgrad.cu, the optimizer step is adam.cu.
 //
 // Cluster rank = 2k + c: the twin critics are independent except for min(Q'_1, Q'_2) in the TD target, so
-// group k (2 CTAs) takes critic k — target pass, online pass, backward — and CTA c of the group computes
-// output columns [128c, 128c+128) of every layer (mlp_cluster.cuh). Both groups recompute the (cheap,
-// identical) next-action pass; the two groups swap their 8 target Q values through distributed shared
-// memory. Critical path: 4 network passes, each layer streaming 128 KB of weights per SM; 4 * B/8 = 128 CTAs.
+// group k (2 CTAs) takes critic k — target pass, online pass, backward — and the two groups swap their 8 target Q
+// values through distributed shared memory. Both groups recompute the (identical) next-action pass.
+// Inside a group, the online critic's forward pass depends on neither the next action nor the target, so the first
+// pass runs two networks side by side, each whole on one CTA (trunk_fwd_full, no exchange): CTA 0 the next-action
+// pass and the sampling, CTA 1 the forward pass of online critic k. CTA 0 hands a' (and log pi) to CTA 1 before the
+// target pass; CTA 1 hands its activations and Q values to CTA 0 for the backward pass, in flight during the target
+// pass. The target pass and the backward pass split output columns: CTA c computes [128c, 128c+128) of every layer
+// (mlp_cluster.cuh). Every element goes through the same steps in the same order either way, so the results are
+// bit-identical to column-split passes throughout. Critical path: 3 network passes; 4 * B/8 = 128 CTAs.
 #include "mlp_cluster.cuh"
 #include "policy.cuh"
 #include "rng.cuh"
@@ -18,12 +23,15 @@ constexpr int MAX_A = MAX_OUT / 2;
 
 struct CriticSmem {
   Work s;
-  Acts a;                      // the online critic's pass (kept for its backward pass)
-  NetStage nsA, nsT, nsQ;      // staged small tensors of the actor, of target critic k and of online critic k
+  Acts a;                      // the online critic's pass (kept for its backward pass; CTA 0 receives it from CTA 1)
+  // staged small tensors of the actor, of target critic k and of online critic k. The first pass's network (CTA 0: the
+  // actor, CTA 1: online critic k) has both first-layer column slices staged, the upper one in the w1s of the stage
+  // whose network this CTA does not run forward (CTA 0: nsQ, CTA 1: nsA).
+  NetStage nsA, nsT, nsQ;
   Net nA, nT, nQ;              // their descriptors
   float lo[MAX_A], hi[MAX_A], eps[RT][MAX_A];
   float rd[RT][2];             // (reward, done) of the 8 rows
-  float logpi[RT], qn[2][RT], y[RT], dq[RT], sq[RT];  // per-row scalars
+  float logpi[RT], qn[2][RT], qv[RT], y[RT], dq[RT], sq[RT];  // per-row scalars
   // followed by two input tiles float4[RQ * (O + A)]: [next_obs | a'] and [obs | act], then CriticVals
 };
 // this agent's values (common.cuh agent_hp), behind the tiles so that the tiles keep their offset
@@ -79,11 +87,12 @@ __global__ void __launch_bounds__(NT, 1) critic_fused_kernel(const __grid_consta
     tile_noise<RT, MAX_A>(M.eps, A.eps, rank == 0 ? A.eps_out : nullptr, A.hp.seed, (int64_t)agent * B + b0, b0, nvalid, AD, step, gid,
                           STREAM_CRITIC_EPS, !td3 || A.hp.targ_smoothing, l);
   } else if (w == 1) {
-    stage_net(PA, &A.actor, &M.nsA, &M.nA, G.c * CW);
+    if (G.c == 0) stage_net(PA, &A.actor, &M.nsA, &M.nA, 0, M.nsQ.w1s);
+    else stage_net(P, &A.critic[k], &M.nsQ, &M.nQ, 0, M.nsA.w1s);
   } else if (w == 2) {
     stage_net(T, &A.critic[k], &M.nsT, &M.nT, G.c * CW);
   } else if (w == 3) {
-    stage_net(P, &A.critic[k], &M.nsQ, &M.nQ, G.c * CW);
+    if (G.c == 0) stage_net(P, &A.critic[k], &M.nsQ, &M.nQ, -1);  // (no first layer: its backward pass only)
   } else {
     // In-kernel sampling (A.storage): lane i draws the replay index of tile row i & 7 — the Philox key of
     // replay.cu::gather_kernel, so the batch is the one b2rl_replay_sample_gather would have gathered — and the tiles
@@ -139,40 +148,75 @@ __global__ void __launch_bounds__(NT, 1) critic_fused_kernel(const __grid_consta
   if (blockIdx.x == 0 && blockIdx.y == 0 && l == 0) g_b2rl_timing[52 + w] = clock64();
 #endif
   __syncthreads();
-  int gi = 0;
+  const Workspace ws = ws_carve(wsb, B, k);
+  const uint32_t peer = (uint32_t)(rank ^ 1), peer_xbar = map_peer(smem_u32(&S.xbar[1]), peer);
 
-  // ---- next action
-  gi = trunk_fwd<WIDE>(G, &act, XA, ldx, nullptr, &S, gi, nullptr, nullptr, b0, nvalid, 2);
-  rowdot(act.p[F_W3], act.p[F_B3], act.out_dim, S.h[1], S.u);
-  __syncthreads();
-  B2RL_TICK(10);
-  for (int r = w; r < RT; r += NW) {  // warp <-> batch row, lane <-> action dim
-    float lp = 0.f;
-    if (l < AD) {
-      const float lo = M.lo[l], hi = M.hi[l];
-      const float scale = (hi - lo) * 0.5f, bias = (hi + lo) * 0.5f;  // agents/nets.py:200-204
-      const float z = M.eps[r][l];
-      const float u0 = uref(S.u, r, l);
-      float act_v;
-      if (td3) {
-        float th;
-        act_v = td3_action(u0, scale, bias, th);
-        if (A.hp.targ_smoothing) {
-          float n = __fmul_rn(z, V.td3_std);
-          n = fminf(fmaxf(n, -V.td3_c), V.td3_c);
-          act_v = fminf(fmaxf(__fadd_rn(act_v, n), lo), hi);
-        }
-      } else {
-        const GaussSample g = gauss_sample(u0, uref(S.u, r, AD + l), z, scale, bias);
-        act_v = g.action;
-        lp = g.logp;
-      }
-      reinterpret_cast<float*>(&XA[(r >> 2) * ldx + O + l])[r & 3] = act_v;
+  // ---- first pass, each network whole on one CTA; the hand-offs are counted on the receiver's xbar[1]
+  if (G.c == 1) {
+    // online Q_k on (obs, act)  (agent.py:230-231); h1 / h2 go to the workspace, all 256 columns
+    B2RL_TICK2(1);
+    trunk_fwd_full<WIDE>(&qo, XB, ldx, &M.a, &S, ws.h1, ws.h2, b0, nvalid, 24);
+    rowdot(qo.p[F_W3], qo.p[F_B3], 1, S.h[1], S.u);
+    __syncthreads();
+    B2RL_TICK2(33);
+    if (t == 0) mbar_expect(&S.xbar[1], RT * (AD + 1) * sizeof(float));  // a' and log pi from CTA 0
+    exchange_init_wait();  // (first remote access of the kernel)
+    static_assert(sizeof(Acts) % sizeof(float4) == 0, "Acts is sent as float4");
+    const float4* src = reinterpret_cast<const float4*>(&M.a);
+    const uint32_t dst = map_peer(smem_u32(&M.a), peer);
+#pragma unroll 1
+    for (int i = t; i < (int)(sizeof(Acts) / sizeof(float4)); i += NT) st_async_v4(dst + i * sizeof(float4), src[i], peer_xbar);
+    if (t < RT) {
+      const float q = uref(S.u, t, 0);
+      M.qv[t] = q;
+      st_async_f32(map_peer(smem_u32(&M.qv[t]), peer), q, peer_xbar);
     }
-    lp = warp_sum(lp);
-    if (l == 0) M.logpi[r] = lp;
+    mbar_wait(&S.xbar[1], 0);
+    B2RL_TICK2(37);
+  } else {
+    // next action (agent.py:194-205)
+    trunk_fwd_full<WIDE>(&act, XA, ldx, nullptr, &S, nullptr, nullptr, b0, nvalid, 2);
+    rowdot(act.p[F_W3], act.p[F_B3], act.out_dim, S.h[1], S.u);
+    __syncthreads();
+    B2RL_TICK(10);
+    if (t == 0) mbar_expect(&S.xbar[1], sizeof(Acts) + RT * sizeof(float));  // Q_k's activations and values from CTA 1
+    exchange_init_wait();  // (first remote access of the kernel)
+    for (int r = w; r < RT; r += NW) {  // warp <-> batch row, lane <-> action dim
+      float lp = 0.f;
+      if (l < AD) {
+        const float lo = M.lo[l], hi = M.hi[l];
+        const float scale = (hi - lo) * 0.5f, bias = (hi + lo) * 0.5f;  // agents/nets.py:200-204
+        const float z = M.eps[r][l];
+        const float u0 = uref(S.u, r, l);
+        float act_v;
+        if (td3) {
+          float th;
+          act_v = td3_action(u0, scale, bias, th);
+          if (A.hp.targ_smoothing) {
+            float n = __fmul_rn(z, V.td3_std);
+            n = fminf(fmaxf(n, -V.td3_c), V.td3_c);
+            act_v = fminf(fmaxf(__fadd_rn(act_v, n), lo), hi);
+          }
+        } else {
+          const GaussSample g = gauss_sample(u0, uref(S.u, r, AD + l), z, scale, bias);
+          act_v = g.action;
+          lp = g.logp;
+        }
+        float* dst = reinterpret_cast<float*>(&XA[(r >> 2) * ldx + O + l]) + (r & 3);
+        *dst = act_v;
+        st_async_f32(map_peer(smem_u32(dst), peer), act_v, peer_xbar);
+      }
+      lp = warp_sum(lp);
+      if (l == 0) {
+        M.logpi[r] = lp;
+        st_async_f32(map_peer(smem_u32(&M.logpi[r]), peer), lp, peer_xbar);
+      }
+    }
+    __syncthreads();
   }
-  __syncthreads();
+  // The first exchange below would wait on the cluster barrier a second time: the counter starts at 4, which selects
+  // the same z buffer and mbarrier phase as 0 (reduce_gather).
+  int gi = 4;
 
   // ---- target Q_k on (next_obs, a')  (agent.py:208-210), then swap the 8 values with the peer group
   B2RL_TICK(11);
@@ -205,21 +249,16 @@ __global__ void __launch_bounds__(NT, 1) critic_fused_kernel(const __grid_consta
     M.y[r] = y;
     if (A.dbg_targ_q && rank == 0 && r < nvalid) A.dbg_targ_q[(size_t)agent * B + b0 + r] = y;
   }
-  // (M.y is read after the barriers inside trunk_fwd)
 
-  // ---- online Q_k, loss, backward (agent.py:230-235)
+  // ---- loss, backward of online Q_k (agent.py:232-235)
   {
-    const Workspace ws = ws_carve(wsb, B, k);
     float* part = ws.part + (size_t)rb * PART_LEN;
+    if (G.c == 0) mbar_wait(&S.xbar[1], 0);  // Q_k's activations and values have landed
     B2RL_TICK(23);
-    gi = trunk_fwd<WIDE>(G, &qo, XB, ldx, &M.a, &S, gi, ws.h1, ws.h2, b0, nvalid, 24);
-    rowdot(qo.p[F_W3], qo.p[F_B3], 1, S.h[1], S.u);
-    __syncthreads();
-    B2RL_TICK(33);
-    if (t < RT) {
+    if (t < RT) {  // (thread r wrote M.y[r] above)
       const int r = t;
       const bool valid = r < nvalid;
-      const float qv = uref(S.u, r, 0);
+      const float qv = M.qv[r];
       const float dlt = qv - M.y[r];
       const float dq = valid ? dlt * (2.0f / (float)B) : 0.f;  // d mean((q-y)^2) / dq
       M.dq[r] = dq;

@@ -39,6 +39,7 @@ enum { F_W1T, F_B1, F_G1, F_BE1, F_W2T, F_B2, F_G2, F_BE2, F_W3, F_B3, F_W2N, F_
 struct Net {
   const float* p[F_N];
   const float* w1s;  // this CTA's column slice of w1t staged in shared memory ([in_dim][128]), or null
+  const float* w1s_hi;  // a full-width pass (trunk_fwd_full): columns [128, 256) of w1t, staged likewise, or null
   int in_dim, out_dim, ln, pad;
 };
 
@@ -78,7 +79,10 @@ struct NetStage {
 // cycles per bulk copy: too many small pieces for the TMA engine), ~40 unrolled LDG.128 + STS.128 3 650, offsets
 // passed by shuffle + fully rolled loops 3 500-4 300. The three networks' 45 KB per CTA (5.8 MB per launch) from L2 and
 // ~90 LDGSTS per SM set the floor, not the mechanism.
-static __device__ __noinline__ void stage_net(const float* region, const b2rl_net_t* d, NetStage* st, Net* out, int j0) {
+// The first layer's slice [j0, j0 + 128) goes to st->w1s; with w1s_hi (j0 = 0, a network run at full width by one CTA)
+// columns [128, 256) go there as well; j0 < 0 stages no first-layer weights (a network this CTA never runs forward).
+static __device__ __noinline__ void stage_net(const float* region, const b2rl_net_t* d, NetStage* st, Net* out, int j0,
+                                              float* w1s_hi = nullptr) {
   const int lane = threadIdx.x & 31;
   const int64_t* offs = &d->w1t;
   int64_t o[F_N];
@@ -86,7 +90,7 @@ static __device__ __noinline__ void stage_net(const float* region, const b2rl_ne
   for (int f = 0; f < F_N; ++f) o[f] = offs[f];
   const int in_dim = d->in_dim, out_dim = d->out_dim;
   const bool ln = d->layer_norm != 0;
-  const bool w3s = out_dim <= W3_ROWS, w1s = in_dim <= W1S_ROWS;
+  const bool w3s = out_dim <= W3_ROWS, w1s = in_dim <= W1S_ROWS && j0 >= 0;
   if (lane < F_N) {
     const float* ptr = region + offs[lane];
     const int v = lane - 1 - (lane > 4);  // b1 g1 be1 -> 0 1 2, b2 g2 be2 -> 3 4 5
@@ -98,11 +102,16 @@ static __device__ __noinline__ void stage_net(const float* region, const b2rl_ne
   if (lane == F_N) {
     out->in_dim = in_dim; out->out_dim = out_dim; out->ln = d->layer_norm;
     out->w1s = w1s ? st->w1s : nullptr;
+    out->w1s_hi = w1s ? w1s_hi : nullptr;
   }
   if (w1s) {  // the first layer's column slice first (the first product needs it): 512 contiguous bytes per input feature
     const float* w1 = region + o[F_W1T] + j0 + 4 * lane;
 #pragma unroll 4
     for (int k = 0; k < in_dim; ++k) cp_async16(st->w1s + k * CW + 4 * lane, w1 + (size_t)k * HID);
+    if (w1s_hi) {
+#pragma unroll 4
+      for (int k = 0; k < in_dim; ++k) cp_async16(w1s_hi + k * CW + 4 * lane, w1 + CW + (size_t)k * HID);
+    }
   }
 #pragma unroll
   for (int v = 0; v < 6; ++v) {  // 64 float4 per vector: two per lane
@@ -145,6 +154,7 @@ struct Group {  // the CS CTAs that share 8 rows of one network
   int c;        // this CTA's column slice
   int base;     // cluster rank of slice 0
 };
+constexpr int ALL_COLS = -1;  // Group::c of a CTA that runs a network alone (trunk_fwd_full): it owns every column
 
 // ---- the products: red[w][r][j] = sum_{k in slice(w)} W[k][j0 + j] * X[r][k],  r < 8, j < 128 --------------------
 // W is [K][256] row-major (w1t / w2t for the forward pass, w2n for dX). Warp w owns a contiguous slice of K;
@@ -336,7 +346,25 @@ __device__ __forceinline__ void exchange_init_arrive(Work& S) {
 }
 __device__ __forceinline__ void exchange_init_wait() { asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory"); }
 
-// ---- split-K reduction (fixed order) + bias + exchange of this CTA's 8x128 slice with the peer ------------------
+// ---- split-K reduction (fixed order) + bias ----------------------------------------------------------------------
+// Thread t: row t >> 5, columns j0 + 4 (t & 31)..+3, summed over the k-slices in a fixed order, plus the bias.
+__device__ __forceinline__ float4 reduce_slice(const Work& S, int j0, const float* __restrict__ bias) {
+  const int t = threadIdx.x, r = t >> 5, cq = t & 31;
+  const float* rp = S.red + (size_t)r * CW + 4 * cq;
+  float4 s = *reinterpret_cast<const float4*>(rp);
+#pragma unroll
+  for (int w = 1; w < KS; ++w) {
+    const float4 v = *reinterpret_cast<const float4*>(rp + (size_t)w * RT * CW);
+    s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
+  }
+  if (bias) {
+    const float4 bv = *reinterpret_cast<const float4*>(bias + j0 + 4 * cq);
+    s.x += bv.x; s.y += bv.y; s.z += bv.z; s.w += bv.w;
+  }
+  return s;
+}
+
+// ---- split-K reduction + exchange of this CTA's 8x128 slice with the peer ----------------------------------------
 // Thread (r = t >> 5, cq = t & 31) owns row r, columns j0+4cq..+3. Its float4 goes to the local z buffer with a
 // plain store and to the peer's with st.async, which also counts 16 bytes on the PEER's mbarrier; thread 0 has
 // armed this CTA's mbarrier for the 4096 bytes the peer will send. No cluster barrier and no memory fence: each
@@ -348,17 +376,7 @@ __device__ __forceinline__ const float* reduce_gather(const Group G, Work& S, in
   const int t = threadIdx.x, r = t >> 5, cq = t & 31, j = G.c * CW + 4 * cq;
   const int b = gi & 1;
   if (t == 0) mbar_expect(&S.mbar[b], RT * CW * sizeof(float));
-  const float* rp = S.red + (size_t)r * CW + 4 * cq;
-  float4 s = *reinterpret_cast<const float4*>(rp);
-#pragma unroll
-  for (int w = 1; w < KS; ++w) {
-    const float4 v = *reinterpret_cast<const float4*>(rp + (size_t)w * RT * CW);
-    s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
-  }
-  if (bias) {
-    const float4 bv = *reinterpret_cast<const float4*>(bias + j);
-    s.x += bv.x; s.y += bv.y; s.z += bv.z; s.w += bv.w;
-  }
+  const float4 s = reduce_slice(S, G.c * CW, bias);
   float* zl = S.z[b];
   float* dst = zl + (size_t)r * HID + j;
   *reinterpret_cast<float4*>(dst) = s;
@@ -419,7 +437,7 @@ __device__ __forceinline__ void layer_fwd_rows(const float* __restrict__ z, cons
     B2RL_TICK(tk);
     if (stat_keep && t < RT) stat_keep[t] = S.stat[t];
   }
-  const bool mine = ws_h && (j >> 7) == G.c;
+  const bool mine = ws_h && (G.c == ALL_COLS || (j >> 7) == G.c);
 #pragma unroll
   for (int q = 0; q < RQ; ++q) {
     float xh[4], h[4];
@@ -608,6 +626,48 @@ static __device__ __noinline__ int trunk_fwd(const Group G, const Net* np, const
     B2RL_TICK(tk + 3 + 3 * layer);
   }
   return gi;
+}
+
+// ---- the two hidden layers, forward, all 256 columns by this CTA alone (no exchange) --------------------------------
+// For a CTA that runs a whole network pass while its peer runs another one (critic.cu, first pass). Each layer's
+// product is trunk_fwd's two column slices one after the other — the same calls with j0 = 0 and then j0 = 128, each
+// followed by the same fixed-order reduction — so every element is bit-identical to the split pass; the local
+// reduction fills the Z buffer that the exchange fills there. The next product's first weight groups are requested
+// before each reduction (and before the row-wise step). Only S.z[1] is used: the peer's first exchange after this pass
+// targets S.z[0] and may land while this pass still runs. Leaves h2 in S.h[1] (synchronised), x-hat / statistics in
+// `A` if given, and stores all 256 columns of h1 / h2 to the workspace when ws_h1 / ws_h2 are given. Touches no
+// mbarrier: the exchange counter of trunk_fwd / trunk_bwd is unaffected.
+template <bool WIDE>
+static __device__ __noinline__ void trunk_fwd_full(const Net* np, const float4* __restrict__ X, int ldx, Acts* A, Work* Sp,
+                                                   float* ws_h1, float* ws_h2, int b0, int nvalid, int tk) {
+  const Net& n = *np;
+  Work& S = *Sp;
+  float* z = S.z[1];
+  WPipe P;
+  B2RL_TICK2(tk + 0);
+#pragma unroll 1
+  for (int layer = 0; layer < 2; ++layer) {
+#pragma unroll 1
+    for (int h = 0; h < CS; ++h) {
+      const int j0 = h * CW;
+      if (layer == 0) {
+        if (!WIDE || n.w1s) first_smem(h ? n.w1s_hi : n.w1s, n.in_dim, X, ldx, S.red);
+        else first_global(n.p[F_W1T], n.in_dim, X, ldx, j0, S.red);
+        if (h == CS - 1) hidden_prefetch(n.p[F_W2T], 0, P);  // (not before: first_global is a call)
+      } else {
+        hidden_fma(n.p[F_W2T], j0, P, S.h[0], S.red);
+        if (h == 0) hidden_prefetch(n.p[F_W2T], CW, P);
+      }
+      __syncthreads();
+      const float4 v = reduce_slice(S, j0, n.p[F_B1 + 4 * layer]);
+      *reinterpret_cast<float4*>(z + (threadIdx.x >> 5) * HID + j0 + 4 * (threadIdx.x & 31)) = v;
+      __syncthreads();  // S.red is free for the next product; after the last slice, z holds the full tile
+    }
+    B2RL_TICK2(tk + 2 + 3 * layer);
+    layer_fwd_rows(z, n.p[F_G1 + 4 * layer], n.p[F_BE1 + 4 * layer], n.ln != 0, S, S.h[layer], A ? A->xh[layer] : nullptr,
+                   A ? A->st[layer] : nullptr, layer ? ws_h2 : ws_h1, b0, nvalid, Group{ALL_COLS, 0}, tk + 7);
+    B2RL_TICK2(tk + 3 + 3 * layer);
+  }
 }
 
 // ---- the two hidden layers, backward (dX path) ----------------------------------------------------------------------
