@@ -559,8 +559,10 @@ def test_fused_optimizer_stacked_high_counters_bitwise(td3):
 # ------------------------------------------------------------------------------------------------ 5. temperature Adam
 @pytest.mark.gpu
 @pytest.mark.parametrize("n", [1, 128, 129, 300])
-@pytest.mark.parametrize("grad_scale", [1.0, 0.5])
-def test_alpha_adam_matches_float64(n, grad_scale):
+@pytest.mark.parametrize("grad_scale,table", [(1.0, False), (0.5, False), (1.0, True)], ids=["1.0", "0.5", "1.0-table"])
+def test_alpha_adam_matches_float64(n, grad_scale, table):
+    """One temperature Adam step per agent (b2rl_alpha_adam); table: each agent's own lr from a per-agent hyperparameter
+    table (b2rl_alpha_adam_hp)."""
     lib = _lib()
     rng = np.random.default_rng(n)
     st = np.zeros((n, 5), dtype=np.float32)
@@ -576,7 +578,15 @@ def test_alpha_adam_matches_float64(n, grad_scale):
     out0 = np.full((n, 8), SENT, dtype=np.float32)
     d_st, d_ctr, d_out = (torch.from_numpy(x).cuda() for x in (st, ctr, out0))
     lr = f32(1e-3)
-    L.check(lib.b2rl_alpha_adam(d_st.data_ptr(), d_ctr.data_ptr(), n, lr, grad_scale, d_out.data_ptr(), _st()), "alpha_adam")
+    if table:
+        hp = np.zeros((n, C.sizeof(L.AgentHp) // 4), dtype=np.float32)
+        hp[:, L.CTR_ALPHA] = np.array([1e-4, 3e-3, 0.05], dtype=np.float32)[np.arange(n) % 3]
+        d_hp = torch.from_numpy(hp).cuda()
+        lr = hp[:, L.CTR_ALPHA].astype(np.float64)
+        L.check(lib.b2rl_alpha_adam_hp(d_st.data_ptr(), d_ctr.data_ptr(), n, d_hp.data_ptr(), grad_scale, d_out.data_ptr(), _st()),
+                "alpha_adam_hp")
+    else:
+        L.check(lib.b2rl_alpha_adam(d_st.data_ptr(), d_ctr.data_ptr(), n, lr, grad_scale, d_out.data_ptr(), _st()), "alpha_adam")
     torch.cuda.synchronize()
     got, c1, out = d_st.cpu().numpy(), d_ctr.cpu().numpy(), d_out.cpu().numpy()
     want = ctr.copy()
@@ -603,7 +613,7 @@ def test_alpha_adam_matches_float64(n, grad_scale):
     assert np.isinf(out[alpha >= 2.0 ** 128, L.OUT_ALPHA]).all()
     keep = [i for i in range(8) if i not in (L.OUT_ALPHA_LOSS, L.OUT_ALPHA)]
     assert np.array_equal(out[:, keep].view(np.uint32), out0[:, keep].view(np.uint32))
-    worst.report(f"alpha_adam n={n} grad_scale={grad_scale} worst dev/bound")
+    worst.report(f"alpha_adam n={n} grad_scale={grad_scale} table={table} worst dev/bound")
 
 
 @pytest.mark.gpu

@@ -158,11 +158,12 @@ def group_sum(a: R, g: int, k: int) -> R:
 
 
 # ---- float64 references (plain torch functions of the kernels' fp32 inputs; CPU or GPU) --------------------------------
-def policy_head_ref(h2, w3, b3, eps, lo, hi, A, td3, smoothing=False, std=0.0, c=0.0):
+def policy_head_ref(h2, w3, b3, eps, lo, hi, A, td3, smoothing=False, std=0.0, c=0.0, u=None):
     """wide_policy_head for one agent: head u = h2 . w3^T + b3, then TD3's tanh action (+ clipped, clamped smoothing
     noise) or SAC's tanh-Gaussian sample and log-prob (policy.cuh, in its operation order). Returns R-valued
-    {act, logp, eps, sigma, y, th} (SAC) / {act, th} (TD3)."""
-    u = r_dot(h2, w3, b3, 14)
+    {act, logp, eps, sigma, y, th} (SAC) / {act, th} (TD3). u: the head's output as an R, when it is computed elsewhere
+    (an h2 that carries its own bound)."""
+    u = r_dot(h2, w3, b3, 14) if u is None else u
     lo, hi = lo.double(), hi.double()
     scale, bias = (R(hi) - R(lo)) * 0.5, (R(hi) + R(lo)) * 0.5
     if td3:
@@ -188,12 +189,14 @@ def policy_head_ref(h2, w3, b3, eps, lo, hi, A, td3, smoothing=False, std=0.0, c
 
 
 def q_target_ref(q: R, qn0, qn1, logp, log_alpha, r, d, gamma, M, td3, bcq):
-    """The critic head's online mode (agents/agent.py:212-233): TD target y, dLoss/dQ = 2 (q - y) / M, (q - y)^2."""
-    qn0, qn1 = qn0.double(), qn1.double()
-    qmin, qmax = torch.minimum(qn0, qn1), torch.maximum(qn0, qn1)
-    qp = 0.75 * R(qmin) + 0.25 * R(qmax) if bcq else R(qmin)
+    """The critic head's online mode (agents/agent.py:212-233): TD target y, dLoss/dQ = 2 (q - y) / M, (q - y)^2.
+    qn0, qn1, logp: fp32 inputs, or R values that carry their own bounds (min / max move by at most the larger one)."""
+    qn0, qn1 = R.of(qn0), R.of(qn1)
+    e = torch.maximum(qn0.e, qn1.e)
+    qmin, qmax = R(torch.minimum(qn0.v, qn1.v), e), R(torch.maximum(qn0.v, qn1.v), e)
+    qp = 0.75 * qmin + 0.25 * qmax if bcq else qmin
     if not td3:
-        qp = qp - r_exp(R(log_alpha)) * R(logp)
+        qp = qp - r_exp(R(log_alpha)) * R.of(logp)
     y = R(r) + ((1.0 - R(d)) * f32(gamma)) * qp
     dlt = q - y
     return dict(y=y, dz=dlt * (R(2.0) / R(float(M))), sq=dlt * dlt)
@@ -231,16 +234,18 @@ def actor_loss_ref(q0, q1, logp, log_alpha, td3, M):
     return dict(d0=d0, d1=d1, loss=loss, lp=R(logp))
 
 
-def head_bwd_ref(dqda0, dqda1, save, lo, hi, log_alpha, td3, A, M):
+def head_bwd_ref(dqda0, dqda1, save, lo, hi, log_alpha, td3, A, M, recip=False):
     """wide_actor_head_bwd for one agent: du [M][out] from dQ/da and the saved sampling intermediates (policy.cuh
-    gauss_backward in its operation order)."""
-    ga = R(dqda0) if dqda1 is None else R(dqda0) + R(dqda1)
+    gauss_backward in its operation order). dQ/da and save may be R values: save then is the sequence (eps, sigma, y, th).
+    recip: c_pi = alpha * fl(1 / M), the fused actor's rounding, instead of alpha / M."""
+    ga = R.of(dqda0) if dqda1 is None else R.of(dqda0) + R.of(dqda1)
     scale = (R(hi.double()) - R(lo.double())) * 0.5
-    th = R(save[:, 3])
+    sv = save if isinstance(save, (list, tuple)) else [save[:, i] for i in range(4)]
+    th = R.of(sv[3])
     if td3:
         return dict(du=ga * scale * (1.0 - th * th), sat=torch.zeros_like(ga.v, dtype=torch.bool))
-    eps, sigma, y = R(save[:, 0]), R(save[:, 1]), R(save[:, 2])
-    c_pi = r_exp(R(log_alpha)) / R(float(M))
+    eps, sigma, y = R.of(sv[0]), R.of(sv[1]), R.of(sv[2])
+    c_pi = r_exp(R(log_alpha)) * (R(1.0) / R(float(M))) if recip else r_exp(R(log_alpha)) / R(float(M))
     omy = 1.0 - y * y
     dcorr = (-2.0 * y * scale) / (scale * omy + f32(1e-6))
     gx = (ga * scale - c_pi * dcorr) * omy
