@@ -363,6 +363,36 @@ typedef struct b2rl_wide_policy {  /* policy head + action sample (agents/nets.p
 } b2rl_wide_policy_t;
 int b2rl_wide_policy_head(const b2rl_wide_policy_t* p, const b2rl_stack_t* stack, void* stream);
 
+/* Behaviour policy on the wide path: b2rl_actor_predict (Agent.predict, agents/agent.py:172-181, nets.py:149-159, :222-234)
+ * for ONE learner on the h2 [n][256] of its actor — b2rl_tc_first and b2rl_tc_linear on the n observations — so that the
+ * actor's weights are read once per 128 rows instead of once per 8. mode, explore_std, draw, eps and agent_hp mean what they
+ * mean for b2rl_actor_predict, and the Philox noise is the same numbers (key ~seed, the global id `agent`, row and action
+ * dimension as there; draw = UINT64_MAX: counters[B2RL_CTR_Q] | 2^31): the two policies differ only by the forward pass's
+ * arithmetic. TD3 mode 1 adds the noise unclamped, as b2rl_actor_predict does. */
+typedef struct b2rl_wide_predict {
+  const float* h2;      /* [n][256] */
+  const float* w3;      /* [out_dim][256] */
+  const float* b3;
+  const float* min_ac;
+  const float* max_ac;
+  const float* eps;     /* [n][A] or NULL => Philox */
+  float* eps_out;       /* [n][A] or NULL: the noise used (mode 1) */
+  float* actions;       /* out [n][A] */
+  const uint64_t* counters;         /* the learner's (read when draw = UINT64_MAX) */
+  const b2rl_agent_hp_t* agent_hp;  /* NULL, or a row whose explore_std replaces explore_std */
+  int32_t n, A, out_dim, mode, td3;
+  float explore_std;    /* TD3 mode 1 (hps.actor_noise_std) */
+  uint64_t seed;        /* the learner's hp.seed */
+  uint64_t draw;
+  uint32_t agent;       /* global learner id */
+  uint32_t reserved;
+} b2rl_wide_predict_t;
+int b2rl_wide_actor_predict(const b2rl_wide_predict_t* p, void* stream);
+/* n rows of `width` floats from src (row pitch lds floats) to dst (pitch ldd): ONE memory-copy node (cudaMemcpy2DAsync),
+ * either side device or pinned host memory. Puts pinned observations [n][O] into the [n][(O + 3) & ~3] device buffer whose
+ * rows TMA can address (b2rl_tc_first). */
+int b2rl_copy_rows(float* dst, int64_t ldd, const float* src, int64_t lds, int32_t n, int32_t width, void* stream);
+
 typedef struct b2rl_wide_q {  /* critic head; mode 1 adds the TD target, dLoss/dQ and squared-error partials (agent.py:212-233) */
   const float* h2;
   const float* w3;
@@ -531,7 +561,8 @@ int b2rl_bump_counter(uint64_t* counters, int32_t which, int32_t n_agents, void*
  * Stacked agents (a->n_agents > 1; 0 or 1 = one learner): agent g reads its actor at a->arena + g * a->arena_agent_stride,
  *   its counters at a->counters + g * 8 (draw = UINT64_MAX), keys its noise on the global id a->agent_base + g, and
  *   obs / a->eps / actions_out are [n_agents][n][..], contiguous. Each agent's actions equal those of a single call for it.
- *   a->agent_hp: agent g's TD3 noise std in mode 1 is its row's explore_std (explore_std is then ignored). */
+ *   a->agent_hp: agent g's TD3 noise std in mode 1 is its row's explore_std (explore_std is then ignored).
+ *   a->eps_out [n_agents][n][A] or NULL: mode 1 records the noise it used there. */
 int b2rl_actor_predict(const b2rl_update_args_t* a, const float* obs, int32_t n, int32_t mode,
                        float explore_std, uint64_t draw, float* actions_out, void* stream);
 

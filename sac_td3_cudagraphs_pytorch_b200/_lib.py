@@ -79,6 +79,15 @@ class WidePolicy(C.Structure):
                 ("seed", C.c_uint64), ("agent", C.c_uint32), ("reserved", C.c_uint32)]
 
 
+class WidePredict(C.Structure):
+    """b2rl_wide_predict_t"""
+    _fields_ = [("h2", C.c_void_p), ("w3", C.c_void_p), ("b3", C.c_void_p), ("min_ac", C.c_void_p), ("max_ac", C.c_void_p),
+                ("eps", C.c_void_p), ("eps_out", C.c_void_p), ("actions", C.c_void_p), ("counters", C.c_void_p),
+                ("agent_hp", C.c_void_p), ("n", C.c_int32), ("A", C.c_int32), ("out_dim", C.c_int32), ("mode", C.c_int32),
+                ("td3", C.c_int32), ("explore_std", C.c_float), ("seed", C.c_uint64), ("draw", C.c_uint64),
+                ("agent", C.c_uint32), ("reserved", C.c_uint32)]
+
+
 class WideQ(C.Structure):
     _fields_ = [("h2", C.c_void_p), ("w3", C.c_void_p), ("b3", C.c_void_p), ("q_out", C.c_void_p), ("qn0", C.c_void_p),
                 ("qn1", C.c_void_p), ("logp", C.c_void_p), ("rows", C.c_void_p), ("log_alpha", C.c_void_p), ("dz3", C.c_void_p),
@@ -130,6 +139,8 @@ SYMBOLS = {
     "b2rl_tc_linear_bwd": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                     C.c_int32, C.c_void_p, C.c_void_p, _STK, C.c_void_p]),
     "b2rl_wide_policy_head": (C.c_int, [C.POINTER(WidePolicy), _STK, C.c_void_p]),
+    "b2rl_wide_actor_predict": (C.c_int, [C.POINTER(WidePredict), C.c_void_p]),
+    "b2rl_copy_rows": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p]),
     "b2rl_wide_q_head": (C.c_int, [C.POINTER(WideQ), _STK, C.c_void_p]),
     "b2rl_wide_ln_bwd": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32,
                                   C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, _STK, C.c_void_p]),

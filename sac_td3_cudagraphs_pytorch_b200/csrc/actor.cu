@@ -420,9 +420,14 @@ predict_kernel(const __grid_constant__ b2rl_update_args_t A, const float* __rest
       if (td3) {  // agents/nets.py:149-159
         float th;
         a = td3_action(u0, scale, bias, th);
-        if (mode == 1) a += noise_at(A.eps, e, ~A.hp.seed, b0 + r, l, step, agent, STREAM_ACTOR_EPS) * (scale * *xstd);
+        if (mode == 1) {
+          const float z = noise_at(A.eps, e, ~A.hp.seed, b0 + r, l, step, agent, STREAM_ACTOR_EPS);
+          if (A.eps_out) A.eps_out[e] = z;
+          a += z * (scale * *xstd);
+        }
       } else if (mode == 1) {  // sample
         const float z = noise_at(A.eps, e, ~A.hp.seed, b0 + r, l, step, agent, STREAM_ACTOR_EPS);  // key != learner's
+        if (A.eps_out) A.eps_out[e] = z;
         a = gauss_sample(u0, uref(S.u, r, AD + l), z, scale, bias).action;
       } else {  // mode = tanh(mean)*scale + bias, agents/nets.py:233
         a = __fadd_rn(__fmul_rn(tanhf(u0), scale), bias);

@@ -41,6 +41,7 @@ cudaError_t launch_tc_linear_bwd(const float*, int, const float*, const float*, 
                                  const float*, int, float*, float*, const Stk&, cudaStream_t);
 cudaError_t launch_wide_policy_head(const b2rl_wide_policy_t&, const Stk&, cudaStream_t);
 cudaError_t launch_wide_q_head(const b2rl_wide_q_t&, const Stk&, cudaStream_t);
+cudaError_t launch_wide_predict(const b2rl_wide_predict_t&, cudaStream_t);
 cudaError_t launch_wide_ln_bwd(const float*, int, const float*, const float*, const float*, const float*, const float*, int, int,
                                float*, float*, float*, const Stk&, cudaStream_t);
 cudaError_t launch_wide_actor_loss(const float*, const float*, const float*, const float*, int, int, float*, float*, float*,
@@ -318,6 +319,20 @@ int b2rl_wide_policy_head(const b2rl_wide_policy_t* p, const b2rl_stack_t* stack
       p->A < 1 || p->A > 32 || p->out_dim < p->A || p->out_dim > B2RL_MAX_OUT || p->ldn < p->O + p->A)
     return fail(B2RL_E_INVALID, "wide_policy_head: bad arguments");
   return check_launch(b2rl::launch_wide_policy_head(*p, make_stk(stack), (cudaStream_t)stream), "wide_policy_head");
+}
+int b2rl_wide_actor_predict(const b2rl_wide_predict_t* p, void* stream) {
+  if (!p || !p->h2 || !p->w3 || !p->b3 || !p->min_ac || !p->max_ac || !p->actions || p->n < 1 || p->A < 1 || p->A > 32 ||
+      p->out_dim != (p->td3 ? p->A : 2 * p->A))
+    return fail(B2RL_E_INVALID, "wide_actor_predict: bad arguments");
+  if (p->mode != 0 && p->mode != 1) return fail(B2RL_E_INVALID, "wide_actor_predict: mode must be 0 or 1");
+  if (int rc = check_hp(p->agent_hp, "wide_actor_predict")) return rc;
+  return check_launch(b2rl::launch_wide_predict(*p, (cudaStream_t)stream), "wide_actor_predict");
+}
+int b2rl_copy_rows(float* dst, int64_t ldd, const float* src, int64_t lds, int32_t n, int32_t width, void* stream) {
+  if (!dst || !src || n < 1 || width < 1 || ldd < width || lds < width) return fail(B2RL_E_INVALID, "copy_rows: bad arguments");
+  return check_launch(cudaMemcpy2DAsync(dst, (size_t)ldd * sizeof(float), src, (size_t)lds * sizeof(float), (size_t)width * sizeof(float),
+                                        (size_t)n, cudaMemcpyDefault, (cudaStream_t)stream),
+                      "copy_rows");
 }
 int b2rl_wide_q_head(const b2rl_wide_q_t* q, const b2rl_stack_t* stack, void* stream) {
   if (int rc = check_stack(stack, "wide_q_head")) return rc;

@@ -141,37 +141,27 @@ constexpr int WP_ROWS = 64;  // rows per CTA (8 per warp): the head's weights ar
 // (row, dimension) pairs instead of once per row with 3 lanes alive: the one-phase version issued 669 warp instructions
 // per row and was issue-bound (74 % issue-slot utilisation, 1.5 TB/s of its 6.5: profiles/r2_ncu_full_pop256_summary.csv).
 // (min 5 CTAs per SM: without it, the per-agent smoothing values pushed ptxas from 48 to 64 registers, 4 CTAs per SM)
-__global__ void __launch_bounds__(256, 5) wide_policy_head_kernel(const __grid_constant__ WidePolicyArgs P, const Stk K) {
-  extern __shared__ float w3s[];            // [out][256], then us [64][out] head outputs, then lps [64][A] log-prob terms
-  float* us = w3s + P.out_dim * HID;
-  float* lps = us + WP_ROWS * P.out_dim;
-  const int t = threadIdx.x, w = t >> 5, l = t & 31;
-  const size_t ag = blockIdx.y;                 // stacked agents: rows [ag * M, ag * M + M), parameters ps further
-  const float* w3g = P.w3 + ag * K.ps;
-  const float* b3g = P.b3 + ag * K.ps;
-  for (int i = t; i < P.out_dim * HID; i += 256) w3s[i] = __ldg(w3g + i);
-  __syncthreads();
-  const int row0 = blockIdx.x * WP_ROWS;        // first row of this CTA inside the agent's batch
-  const int nrows = min(WP_ROWS, P.M - row0);
+// Phase (1) of the policy heads: us[rr][o] = w3s[o] . h2[grow0 + rr] + b3[o] for the CTA's nrows rows, a warp per row (rows
+// w, w + 8, ...). per_row(grow) runs at the top of each row's turn (the training head copies the row's obs-part there).
+template <class PerRow>
+__device__ __forceinline__ void head_rows(const float* __restrict__ h2, size_t grow0, int nrows, int out_dim, const float* w3s,
+                                          const float* __restrict__ b3g, float* us, int w, int l, PerRow per_row) {
   float hn[8];  // the next row's activations are requested before this row's head is computed (one round trip hidden)
   if (w < nrows) {
 #pragma unroll
-    for (int i = 0; i < 8; ++i) hn[i] = __ldg(P.h2 + (ag * P.M + row0 + w) * HID + l + 32 * i);
+    for (int i = 0; i < 8; ++i) hn[i] = __ldg(h2 + (grow0 + w) * HID + l + 32 * i);
   }
   for (int rr = w; rr < nrows; rr += 8) {
-    const size_t grow = ag * P.M + row0 + rr;   // row of the stacked arrays
+    const size_t grow = grow0 + rr;   // row of the stacked arrays
     float h[8];
 #pragma unroll
     for (int i = 0; i < 8; ++i) h[i] = hn[i];
     if (rr + 8 < nrows) {
 #pragma unroll
-      for (int i = 0; i < 8; ++i) hn[i] = __ldg(P.h2 + (grow + 8) * HID + l + 32 * i);
+      for (int i = 0; i < 8; ++i) hn[i] = __ldg(h2 + (grow + 8) * HID + l + 32 * i);
     }
-    // the obs-part of the next network's input
-    const float* src = P.rows + grow * P.row_stride + P.src_off;
-    float* xr = P.xn + grow * P.ldn;
-    for (int k = l; k < P.O; k += 32) xr[k] = __ldg(src + k);
-    if (P.out_dim <= 8) {
+    per_row(grow);
+    if (out_dim <= 8) {
       // Heads of up to 8 outputs (every task but Humanoid's SAC head): the dot products are reduced TOGETHER — a butterfly
       // that halves the number of live sums at each of its first three steps (9 shuffles instead of 5 per output; the same
       // pairs are added in the same order as warp_sum does). The per-output loop made the kernel issue-bound (ncu: 61 %
@@ -180,7 +170,7 @@ __global__ void __launch_bounds__(256, 5) wide_policy_head_kernel(const __grid_c
 #pragma unroll
       for (int o = 0; o < 8; ++o) {
         s[o] = 0.f;
-        if (o < P.out_dim) {
+        if (o < out_dim) {
 #pragma unroll
           for (int i = 0; i < 8; ++i) s[o] = fmaf(w3s[o * HID + l + 32 * i], h[i], s[o]);
         }
@@ -195,17 +185,37 @@ __global__ void __launch_bounds__(256, 5) wide_policy_head_kernel(const __grid_c
       a1 += __shfl_xor_sync(0xffffffffu, a1, 2);
       a1 += __shfl_xor_sync(0xffffffffu, a1, 1);
       const int o = (b4 ? 4 : 0) + (b3 ? 2 : 0) + (b2 ? 1 : 0);
-      if ((l & 3) == 0 && o < P.out_dim) us[rr * P.out_dim + o] = a1 + __ldg(b3g + o);
+      if ((l & 3) == 0 && o < out_dim) us[rr * out_dim + o] = a1 + __ldg(b3g + o);
     } else {
-      for (int o = 0; o < P.out_dim; ++o) {
+      for (int o = 0; o < out_dim; ++o) {
         float s = 0.f;
 #pragma unroll
         for (int i = 0; i < 8; ++i) s = fmaf(w3s[o * HID + l + 32 * i], h[i], s);
         s = warp_sum(s);
-        if (l == 0) us[rr * P.out_dim + o] = s + __ldg(b3g + o);
+        if (l == 0) us[rr * out_dim + o] = s + __ldg(b3g + o);
       }
     }
   }
+}
+
+__global__ void __launch_bounds__(256, 5) wide_policy_head_kernel(const __grid_constant__ WidePolicyArgs P, const Stk K) {
+  extern __shared__ float w3s[];            // [out][256], then us [64][out] head outputs, then lps [64][A] log-prob terms
+  float* us = w3s + P.out_dim * HID;
+  float* lps = us + WP_ROWS * P.out_dim;
+  const int t = threadIdx.x, w = t >> 5, l = t & 31;
+  const size_t ag = blockIdx.y;                 // stacked agents: rows [ag * M, ag * M + M), parameters ps further
+  const float* w3g = P.w3 + ag * K.ps;
+  const float* b3g = P.b3 + ag * K.ps;
+  for (int i = t; i < P.out_dim * HID; i += 256) w3s[i] = __ldg(w3g + i);
+  __syncthreads();
+  const int row0 = blockIdx.x * WP_ROWS;        // first row of this CTA inside the agent's batch
+  const int nrows = min(WP_ROWS, P.M - row0);
+  head_rows(P.h2, ag * P.M + row0, nrows, P.out_dim, w3s, b3g, us, w, l, [&](size_t grow) {
+    // the obs-part of the next network's input
+    const float* src = P.rows + grow * P.row_stride + P.src_off;
+    float* xr = P.xn + grow * P.ldn;
+    for (int k = l; k < P.O; k += 32) xr[k] = __ldg(src + k);
+  });
   __syncthreads();
   const uint32_t agent = P.agent + (uint32_t)ag;
   const uint64_t step = P.counters[ag * K.cs + P.counter_idx];
@@ -254,6 +264,50 @@ __global__ void __launch_bounds__(256, 5) wide_policy_head_kernel(const __grid_c
       for (int a = 0; a < P.A; ++a) s += lps[t * P.A + a];
       P.logp[ag * P.M + row0 + t] = s;
     }
+  }
+}
+
+// ---- behaviour policy: Agent.predict (agents/agent.py:172-181, nets.py:149-159, :222-234) on h2 of n observations --------
+// Phase (1) as the training head; phase (2) thread <-> (row, action dimension) with exactly the formulas and Philox key of
+// actor.cu predict_kernel (seed ~hp.seed, stream STREAM_ACTOR_EPS, row and dimension as there): the two policies draw the
+// same noise and differ only by the arithmetic of the forward pass. TD3 mode 1 adds the noise without a clamp, as
+// predict_kernel does (the reference's clamp result is dropped, SURVEY App. C.7).
+__global__ void __launch_bounds__(256) wide_predict_kernel(const __grid_constant__ b2rl_wide_predict_t P) {
+  extern __shared__ float w3s[];  // [out][256], then us [64][out]
+  float* us = w3s + P.out_dim * HID;
+  const int t = threadIdx.x, w = t >> 5, l = t & 31;
+  for (int i = t; i < P.out_dim * HID; i += 256) w3s[i] = __ldg(P.w3 + i);
+  __syncthreads();
+  const int row0 = blockIdx.x * WP_ROWS;
+  const int nrows = min(WP_ROWS, P.n - row0);
+  head_rows(P.h2, (size_t)row0, nrows, P.out_dim, w3s, P.b3, us, w, l, [](size_t) {});
+  __syncthreads();
+  const uint64_t step = (P.draw == ~0ull && P.counters) ? (P.counters[B2RL_CTR_Q] | 0x80000000ull) : P.draw;
+  const float xstd = agent_hp(P.agent_hp, 0, HP_EXPLORE, P.explore_std);
+  for (int i = t; i < nrows * P.A; i += 256) {
+    const int rr = i / P.A, a = i - rr * P.A;
+    const int row = row0 + rr;
+    const float lo = __ldg(P.min_ac + a), hi = __ldg(P.max_ac + a);
+    const float scale = (hi - lo) * 0.5f, bias = (hi + lo) * 0.5f;
+    const int64_t e = (int64_t)row * P.A + a;
+    const float u0 = us[rr * P.out_dim + a];
+    float act;
+    if (P.td3) {
+      float th;
+      act = td3_action(u0, scale, bias, th);
+      if (P.mode == 1) {
+        const float z = noise_at(P.eps, e, ~P.seed, row, a, step, P.agent, STREAM_ACTOR_EPS);
+        if (P.eps_out) P.eps_out[e] = z;
+        act += z * (scale * xstd);
+      }
+    } else if (P.mode == 1) {
+      const float z = noise_at(P.eps, e, ~P.seed, row, a, step, P.agent, STREAM_ACTOR_EPS);
+      if (P.eps_out) P.eps_out[e] = z;
+      act = gauss_sample(u0, us[rr * P.out_dim + P.A + a], z, scale, bias).action;
+    } else {
+      act = __fadd_rn(__fmul_rn(tanhf(u0), scale), bias);
+    }
+    P.actions[e] = act;
   }
 }
 
@@ -669,6 +723,8 @@ cudaError_t init_wide() {
   cudaError_t e = cudaFuncSetAttribute(wide_policy_head_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                        (MAX_OUT * HID + WP_ROWS * (MAX_OUT + MAX_OUT / 2)) * 4);
   if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(wide_predict_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (MAX_OUT * HID + WP_ROWS * MAX_OUT) * 4);
+  if (e == cudaSuccess)
     e = cudaFuncSetAttribute(wide_ln_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (MAX_OUT + 24) * HID * 4);
   cudaFuncAttributes fa;
   if (e == cudaSuccess) e = cudaFuncGetAttributes(&fa, wide_first_kernel);
@@ -691,6 +747,11 @@ cudaError_t launch_wide_first(const float* X, int64_t ldx, int M, int K, const f
 cudaError_t launch_wide_policy_head(const WidePolicyArgs& p, const Stk& k, cudaStream_t st) {
   const size_t smem = ((size_t)p.out_dim * HID + (size_t)WP_ROWS * (p.out_dim + p.A)) * sizeof(float);
   wide_policy_head_kernel<<<dim3((p.M + WP_ROWS - 1) / WP_ROWS, k.n), 256, smem, st>>>(p, k);
+  return cudaGetLastError();
+}
+cudaError_t launch_wide_predict(const b2rl_wide_predict_t& p, cudaStream_t st) {
+  const size_t smem = ((size_t)p.out_dim * HID + (size_t)WP_ROWS * p.out_dim) * sizeof(float);
+  wide_predict_kernel<<<(p.n + WP_ROWS - 1) / WP_ROWS, 256, smem, st>>>(p);
   return cudaGetLastError();
 }
 cudaError_t launch_wide_q_head(const WideQArgs& q, const Stk& k, cudaStream_t st) {

@@ -449,3 +449,48 @@ class WideActor:
         L.check(lib.b2rl_wide_policy_head(C.byref(p), stk, st), "wide_policy_head")
         L.check(lib.b2rl_wide_alpha_grad(self.logp2.data_ptr(), M, float(ag.hyper.targ_ent), ag.alpha_state.data_ptr(), stk, st),
                 "wide_alpha_grad")
+
+
+class WidePredictor:
+    """``Agent.predict`` (agents/agent.py:172-181) for one learner on n observation rows, on the tensor cores: the
+    observations are copied into a buffer whose rows TMA can address (pitch (O + 3) & ~3 floats; one memory-copy node, so
+    they may sit in pinned host memory), then b2rl_tc_first -> b2rl_tc_linear -> b2rl_wide_actor_predict. Each actor weight
+    is read once per 128 rows, where the row-group b2rl_actor_predict re-stages half of the actor per 8 rows; below 128
+    rows most of the one tile is padding. The noise is b2rl_actor_predict's, number for number; the forward pass is 3xTF32
+    (fp32-level) or TF32. Buffers are its own, sized for n. Enqueue-only (graph-capturable)."""
+
+    def __init__(self, agent, n: int, precision: str = "3xtf32"):
+        assert precision in ("3xtf32", "tf32")
+        self.ag, self.n, self.x3 = agent, int(n), precision == "3xtf32"
+        f32 = dict(dtype=torch.float32, device=agent.device)
+        self.ldo = (agent.ob_dim + 3) & ~3
+        self.x = torch.zeros(self.n, self.ldo, **f32)
+        self.h1, self.h2 = torch.empty(self.n, 256, **f32), torch.empty(self.n, 256, **f32)
+        # 3xTF32: the hidden layer's weight lo parts come from the learner's mirror, which its optimizer launches keep current
+        self.wlo = agent.lo_mirror() if self.x3 else None
+
+    def enqueue(self, obs_ptr: int, explore: bool, actions_ptr: int, eps: Optional[torch.Tensor] = None,
+                eps_out: Optional[torch.Tensor] = None, draw: int = 2 ** 64 - 1, agent_hp: Optional[torch.Tensor] = None) -> None:
+        """obs_ptr: [n][ob_dim] contiguous (device or pinned host); actions_ptr: [n][ac_dim] (device). draw as in
+        b2rl_actor_predict: UINT64_MAX keys the noise on the critic step counter (inside a step graph)."""
+        ag, lib, n = self.ag, self.ag._lib, self.n
+        lay, st = ag.layout, ag._stream()
+        act, o, RP = lay.actor, lay.actor.off, L.REGION_P
+        ln = int(bool(ag.hps.layer_norm))
+        p = lambda off: ag.arena.flat.data_ptr() + 4 * (RP * lay.region + off)
+        L.check(lib.b2rl_copy_rows(self.x.data_ptr(), self.ldo, obs_ptr, ag.ob_dim, n, ag.ob_dim, st), "copy_rows")
+        L.check(lib.b2rl_tc_first(self.x.data_ptr(), self.ldo, n, ag.ob_dim, p(o["w1t"]), p(o["b1"]), p(o["g1"]) if ln else None,
+                                  p(o["be1"]) if ln else None, ln, self.h1.data_ptr(), None, None, int(self.x3), None, st), "tc_first")
+        w = p(o["w2n"])
+        wl = self.wlo.data_ptr() + (w - p(0)) if self.x3 else None
+        L.check(lib.b2rl_tc_linear(self.h1.data_ptr(), 256, n, w, wl, p(o["b2"]), p(o["g2"]) if ln else None,
+                                   p(o["be2"]) if ln else None, ln, 1, self.h2.data_ptr(), None, None, None, st), "tc_linear")
+        q = L.WidePredict()
+        q.h2, q.w3, q.b3 = self.h2.data_ptr(), p(o["w3"]), p(o["b3"])
+        q.min_ac, q.max_ac = ag.min_ac.data_ptr(), ag.max_ac.data_ptr()
+        q.eps, q.eps_out, q.actions = L.ptr(eps), L.ptr(eps_out), actions_ptr
+        q.counters, q.agent_hp = ag.counters.data_ptr(), L.ptr(agent_hp)
+        q.n, q.A, q.out_dim, q.mode, q.td3 = n, ag.ac_dim, act.out_dim, int(explore), int(ag.td3)
+        q.explore_std = float(ag.hps.actor_noise_std) if ag.td3 else 0.0
+        q.seed, q.draw, q.agent = ag.seed, int(draw), ag.agent_id
+        L.check(lib.b2rl_wide_actor_predict(C.byref(q), st), "wide_actor_predict")
