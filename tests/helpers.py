@@ -1,11 +1,92 @@
 """Shared helpers for the parity tests (test infrastructure)."""
 from __future__ import annotations
 
+import math
+
 import numpy as np
 import torch
 
 from oracle import OracleAgent, OracleHps
 from tests.golden.cases import case_inputs
+
+# ---- running error analysis of fp32 kernels against float64 (test_gpu_wide_kernels.py, test_gpu_tc_kernels.py) ----------
+U = 2.0 ** -24       # unit roundoff of fp32
+WIDEN = 1.01         # (second-order terms of the running bounds)
+FLOOR = 2.0 ** -120
+GUARD = 64           # NaN guard band around every output buffer, in elements
+
+
+def gam(k: int) -> float:
+    return k * U / (1 - k * U)
+
+
+class R:
+    """A float64 value v (tensor) with a first-order bound e on the error of the same expression evaluated in fp32, one
+    rounding per operation. Inputs that are fp32 values are exact (e = 0)."""
+    __slots__ = ("v", "e")
+
+    def __init__(self, v, e=None):
+        self.v = v.double() if torch.is_tensor(v) else torch.tensor(float(v), dtype=torch.float64)
+        self.e = torch.zeros_like(self.v) if e is None else e
+
+    @staticmethod
+    def of(x):
+        return x if isinstance(x, R) else R(x)
+
+    def __getitem__(self, i):
+        return R(self.v[i], self.e[i])
+
+    def __add__(a, b):
+        b = R.of(b)
+        v = a.v + b.v
+        return R(v, a.e + b.e + U * v.abs())
+
+    __radd__ = __add__
+
+    def __sub__(a, b):
+        b = R.of(b)
+        v = a.v - b.v
+        return R(v, a.e + b.e + U * v.abs())
+
+    def __rsub__(a, b):
+        return R.of(b) - a
+
+    def __neg__(a):
+        return R(-a.v, a.e)
+
+    def __mul__(a, b):
+        b = R.of(b)
+        v = a.v * b.v
+        return R(v, a.v.abs() * b.e + b.v.abs() * a.e + a.e * b.e + U * v.abs())
+
+    __rmul__ = __mul__
+
+    def __truediv__(a, b):
+        b = R.of(b)
+        v = a.v / b.v
+        return R(v, (a.e + v.abs() * b.e) / (b.v.abs() - b.e) + U * v.abs())
+
+    def __rtruediv__(a, b):
+        return R.of(b) / a
+
+
+def r_sum(a: R, dim, k) -> R:
+    """Sum of rounded terms along dim: their own bounds plus gamma_k of sum|terms|."""
+    return R(a.v.sum(dim), a.e.sum(dim) + gam(k) * a.v.abs().sum(dim))
+
+
+def guarded(*shape, dtype=torch.float32):
+    """A NaN-filled buffer with a NaN guard band of GUARD elements on both sides: (whole, view of the middle)."""
+    n = math.prod(shape)
+    full = torch.full((n + 2 * GUARD,), float("nan"), dtype=dtype, device="cuda")
+    return full, full[GUARD:GUARD + n].view(*shape)
+
+
+def untouched(full, view=None, mask=None, what=""):
+    """The guard band is still NaN, and so is every element of the view where mask is True."""
+    assert torch.isnan(full[:GUARD]).all() and torch.isnan(full[-GUARD:]).all(), f"{what}: written outside the buffer"
+    if mask is not None:
+        assert torch.isnan(view[mask]).all(), f"{what}: an element the kernel does not own was written"
 
 
 def rel_dev(a, b, scale=None) -> float:

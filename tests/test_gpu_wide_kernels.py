@@ -19,7 +19,7 @@ values. Each output gets its own bound (u = 2^-24, the unit roundoff of fp32; ga
       wide_alpha_grad                                     one rounding per term (-logpi - targ_ent), ceil(M / 256) per
                                                           thread, then min(M, 256) in sequence                 k = ceil(M/256) + min(M, 256)
     A product of a sum with a scalar, or a sum of rounded terms, adds the terms' own bounds first (running error
-    analysis, class R below: every fp32 operation rounds once, |d fl(x)| <= u |x|; an FMA rounds less, so the bound
+    analysis, class R of tests/helpers.py: every fp32 operation rounds once, |d fl(x)| <= u |x|; an FMA rounds less, so the bound
     holds whether or not the compiler contracts).
   - Transcendentals (policy.cuh: tanhf, expf, logf): the CUDA C++ Programming Guide's maximum ulp errors of the
     single-precision functions — tanhf 2, expf 2, logf 1 — with 1 ulp <= 2u |result|, plus the input's bound times the
@@ -49,11 +49,9 @@ import numpy as np
 import pytest
 import torch
 
-U = 2.0 ** -24
+from tests.helpers import FLOOR, GUARD, WIDEN, R, U, gam, guarded, r_sum, untouched  # noqa: F401
+
 ULP_TANH, ULP_EXP, ULP_LOG = 2, 2, 1  # CUDA C++ Programming Guide, single-precision mathematical functions
-WIDEN = 1.01                          # (second-order terms of the running bounds)
-FLOOR = 2.0 ** -120
-GUARD = 64
 MAX_OUT, HID = 64, 256
 LOG_STD_MIN, LOG_STD_MAX = -5.0, 2.0
 f32 = lambda x: float(np.float32(x))
@@ -61,61 +59,7 @@ LOG_SQRT_2PI = f32(0.9189385332046727)
 SAT = 1e-3  # |1 - y^2| below this: a saturated sample
 
 
-def gam(k: int) -> float:
-    return k * U / (1 - k * U)
-
-
-# ---- running error analysis ---------------------------------------------------------------------------------------------
-class R:
-    """A float64 value v (tensor) with a first-order bound e on the error of the same expression evaluated in fp32, one
-    rounding per operation. Inputs that are fp32 values are exact (e = 0)."""
-    __slots__ = ("v", "e")
-
-    def __init__(self, v, e=None):
-        self.v = v.double() if torch.is_tensor(v) else torch.tensor(float(v), dtype=torch.float64)
-        self.e = torch.zeros_like(self.v) if e is None else e
-
-    @staticmethod
-    def of(x):
-        return x if isinstance(x, R) else R(x)
-
-    def __getitem__(self, i):
-        return R(self.v[i], self.e[i])
-
-    def __add__(a, b):
-        b = R.of(b)
-        v = a.v + b.v
-        return R(v, a.e + b.e + U * v.abs())
-
-    __radd__ = __add__
-
-    def __sub__(a, b):
-        b = R.of(b)
-        v = a.v - b.v
-        return R(v, a.e + b.e + U * v.abs())
-
-    def __rsub__(a, b):
-        return R.of(b) - a
-
-    def __neg__(a):
-        return R(-a.v, a.e)
-
-    def __mul__(a, b):
-        b = R.of(b)
-        v = a.v * b.v
-        return R(v, a.v.abs() * b.e + b.v.abs() * a.e + a.e * b.e + U * v.abs())
-
-    __rmul__ = __mul__
-
-    def __truediv__(a, b):
-        b = R.of(b)
-        v = a.v / b.v
-        return R(v, (a.e + v.abs() * b.e) / (b.v.abs() - b.e) + U * v.abs())
-
-    def __rtruediv__(a, b):
-        return R.of(b) / a
-
-
+# ---- running error analysis (gam, R, r_sum: tests/helpers.py) ---------------------------------------------------------
 def r_tanh(a: R) -> R:
     v = torch.tanh(a.v)
     return R(v, (1 - v * v) * a.e + 2 * ULP_TANH * U * v.abs())
@@ -141,11 +85,6 @@ def r_dot(x, w, b, k):
     """x [M][K] . w [O][K]^T + b [O]: a sum whose longest chain is k roundings."""
     x, w, b = x.double(), w.double(), b.double()
     return R(x @ w.T + b, gam(k) * (x.abs() @ w.abs().T + b.abs()))
-
-
-def r_sum(a: R, dim, k) -> R:
-    """Sum of rounded terms along dim: their own bounds plus gamma_k of sum|terms|."""
-    return R(a.v.sum(dim), a.e.sum(dim) + gam(k) * a.v.abs().sum(dim))
 
 
 def group_sum(a: R, g: int, k: int) -> R:
@@ -281,20 +220,6 @@ def check(kernel, what, got, ref: R, sat=None):
         msg += f"; {int(sat.sum())} saturated samples, worst {r_sat:.3f}"
     print(msg)
     assert r_ok <= 1.0 and r_sat <= 1.0, msg
-
-
-def guarded(*shape, dtype=torch.float32):
-    """A NaN-filled buffer with a NaN guard band of GUARD elements on both sides: (whole, view of the middle)."""
-    n = math.prod(shape)
-    full = torch.full((n + 2 * GUARD,), float("nan"), dtype=dtype, device="cuda")
-    return full, full[GUARD:GUARD + n].view(*shape)
-
-
-def untouched(full, view=None, mask=None, what=""):
-    """The guard band is still NaN, and so is every element of the view where mask is True."""
-    assert torch.isnan(full[:GUARD]).all() and torch.isnan(full[-GUARD:]).all(), f"{what}: written outside the buffer"
-    if mask is not None:
-        assert torch.isnan(view[mask]).all(), f"{what}: an element the kernel does not own was written"
 
 
 def _lib():
